@@ -1,12 +1,14 @@
 #!/usr/bin/env python
 """MDViT training-throughput benchmark (BASELINE.json metric: MDViT train images/sec at 1/2/4/8 B200).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch-per-domain B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch-per-domain B] [--impl reference] [--dump-outputs DIR]
 
 One *step* = the reference's optimizer step (multi_train_MDViT.py:121-213): 4 single-domain mini-batches forward,
 BCE+Dice / MKD losses, the two-pass backward, AdamW — on synthetic 256x256 data, random-init weights, dropout 0.1 /
 DropPath 0.1 as in the trainer (multi_train_MDViT.py:59).  N>1 is launched by torchrun (one rank per GPU, NCCL).
 Prints ONE JSON line on rank 0.  `--impl reference` times the CPU restatement of the reference (oracle/) instead.
+`--dump-outputs DIR` writes what the last timed training step returned (losses, logits, updated weights) as DIR/<name>.npy, so
+that two builds can be compared output for output on identical seeded inputs.
 """
 import argparse
 import json
@@ -25,12 +27,13 @@ UNIT = "images/s"
 IMG = 256
 F_TRAIN_GFLOP_PER_IMG = 62.3     # SURVEY.md §8(d): 3 x 20.77 GFLOP algorithmic fwd+bwd per image
 LINEAR_FUSE_DRAM_BYTES = 557116416 + 236415744   # ncu --set full, profiles/r2_ncu_gemm_linear_fuse_fwd.txt (dram read + write, one launch)
+DUMP_SAMPLE = 1 << 20      # --dump-outputs keeps this many elements (a fixed, seeded sample) of a larger output: 4 MB in float32
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--batch-per-domain", type=int, default=32)
     ap.add_argument("--impl", default="mdvit_b200")
@@ -43,7 +46,38 @@ def parse():
     ap.add_argument("--model", default="MDViT", choices=["MDViT", "BASE", "TransFuse"],
                     help="MDViT (default, the headline metric); BASE = BASELINE.json config 2: no DA, no MKD; TransFuse = config 4: "
                          "TransFuse_S_adapt train step (extras, not the headline)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed training step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.mode == "infer"):
+        ap.error("--dump-outputs writes the outputs of the training step of this repository's kernels")
+    return args
+
+
+def dump_outputs(path, trainer, losses):
+    """What a caller of the timed training step receives after its last step: the step's losses, the logits of its forward
+    (MKDTrainer: main and auxiliary per domain; TransFuseTrainer: map_2 per dataset) and the updated weights (the flat fp32
+    parameter buffer), as float32 .npy files.  An output larger than DUMP_SAMPLE elements is written as the same seeded sample
+    of its elements on every run."""
+    import numpy as np
+    import torch
+    outs = {"losses": losses}
+    logits = trainer.last_logits
+    if isinstance(logits[0], tuple):
+        outs["logits_out"] = torch.cat([o for o, _ in logits])
+        if logits[0][1] is not None:
+            outs["logits_aux"] = torch.cat([a for _, a in logits])
+    else:
+        outs["logits"] = torch.cat(logits)
+    outs["params"] = trainer.flat
+    os.makedirs(path, exist_ok=True)
+    for name, t in outs.items():
+        a = t.detach().float().reshape(-1)
+        if a.numel() > DUMP_SAMPLE:
+            idx = np.random.Generator(np.random.PCG64(0)).integers(0, a.numel(), DUMP_SAMPLE)
+            a = a[torch.from_numpy(np.sort(idx)).to(a.device)]
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy().astype(np.float32))
 
 
 def load_peaks():
@@ -141,7 +175,7 @@ def run_reference(args):
         return
     os.environ.pop("OMP_NUM_THREADS", None)
     bpd = args.cpu_batch_per_domain
-    steps = max(1, min(args.steps, 12))          # ~2 s of CPU work per 4-image step: keep the whole arm within ~2 minutes
+    steps = args.steps          # ~2 s of CPU work per 4-image step
     sec, cores = cpu_oracle_step_time(bpd, steps, min(args.warmup, 1))
     val = 4 * bpd / sec
     sample = f"{4 * bpd} images/step ({bpd}/domain x 4 domains) at {IMG}x{IMG}, fp32, dropout on, {steps} timed steps"
@@ -310,7 +344,7 @@ def run_infer(args):
     sampler = ClockSampler(0)
     sampler.start()
     sweep, launches = [], 0
-    steps = max(args.steps, 5)
+    steps = args.steps
     for kind in ("single", "mixed"):
         for B in (1, 2, 4, 8, 16, 32, 64, 128, 256):
             g = torch.Generator().manual_seed(B)
@@ -442,6 +476,8 @@ def run_transfuse(args):
     n1 = lib.mdv_launch_count()
     ms_e2e, loss_host = timed(step_e2e, args.steps, True)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer, loss_host)
     launches = trainer.launches_per_step if use_graph else (n1 - n0) // max(args.steps, 1)
     imgs = 4 * B * world
     if rank == 0:
@@ -564,6 +600,8 @@ def main():
     n1 = lib.mdv_launch_count()
     ms_e2e, loss_host = timed(step_e2e, args.steps, True)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer, loss_host)
     launches_per_step = trainer.launches_per_step if use_graph else (n1 - n0) // max(args.steps, 1)
 
     imgs_per_step = 4 * B * world

@@ -13,7 +13,11 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from mdvit_b200 import synth  # noqa: E402
 from oracle import ref_shim  # noqa: E402
+from oracle.golden_sample import keep_samples  # noqa: E402
 from oracle.make_golden import fingerprint  # noqa: E402
+
+# the 256x256 DeepLabV3 logits kept as a seeded sample of 1/8 of their elements (oracle/golden_sample.py)
+SAMPLED = {"dl_eval_out": 16384, "dl_eval_aux": 16384, "dl_train_aux": 16384}
 
 
 def aux_state(model, prefix="debranch"):
@@ -112,6 +116,7 @@ def main():
                     img, _ = synth.synth_batch(13, d, 2, 64, 64)
                     dl = torch.nn.functional.one_hot(torch.full((2,), d), 4).float() if am else None
                     out[f"base_dsn_{tag}_{mode}_{d}"] = m(img, dl, str(d)).numpy()
+    keep_samples(out, SAMPLED)
     path = os.path.join(ROOT, "tests", "golden", "mdvit_dsn_golden.npz")
     np.savez_compressed(path, **out)
     print("wrote", path, os.path.getsize(path) // 1024, "KiB")

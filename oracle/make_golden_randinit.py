@@ -26,9 +26,14 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from mdvit_b200 import synth  # noqa: E402
 from oracle import ref_shim  # noqa: E402
+from oracle.golden_sample import keep_samples  # noqa: E402
 from oracle.make_golden import fingerprint  # noqa: E402
 
 SEED, IMG, B, STEPS = 0, 256, 4, 5
+
+
+# train-mode logits kept as a seeded sample of 1/8 of their elements (oracle/golden_sample.py)
+SAMPLED = {f"logits256_{k}_{d}": 32768 for k in ("out", "aux") for d in range(4)}
 
 
 def hard_dice(logits, label):
@@ -88,6 +93,7 @@ def main():
     bn_keys = [k for k in sd if k.endswith("running_mean") or k.endswith("running_var")]
     out["traj_bn_names"] = np.asarray(bn_keys)
     out["traj_bn_fp"] = fingerprint([(k, sd[k]) for k in bn_keys])
+    keep_samples(out, SAMPLED)
     path = os.path.join(ROOT, "tests", "golden", "mdvit_randinit_golden.npz")
     np.savez_compressed(path, **out)
     print("wrote", path, os.path.getsize(path) // 1024, "KiB;", len(out), "arrays")

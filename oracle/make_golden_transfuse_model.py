@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY.  Golden vectors for the whole TransFuse_S_adapt (Models/Hybrid_models/TransFuseFolder/TransFuse.py:
 182-283) and structure_loss (multi_train_TransFuse.py:29-38): runs the UNMODIFIED reference from /root/reference in the build
 container at ITS OWN random init (torch.manual_seed(0), stock constructor, drop_rate=0 so that the forward is deterministic)
-and writes tests/golden/transfuse_model_golden.npz.
+and writes tests/golden/transfuse_model_golden.npz and tests/golden/transfuse_structure_loss_golden.npz.
 
     python oracle/make_golden_transfuse_model.py
 
@@ -47,12 +47,43 @@ def structure_loss_ref(pred, mask):
     return (wbce + wiou).mean()
 
 
+def structure_loss_golden(maps, mask):
+    """structure_loss_ref and its gradient, with the 0.5/0.3/0.2 weights of multi_train_TransFuse.py:169-172, on the reference's
+    maps rounded to fp16: the loss reads every pixel, so its input is stored whole, and in fp16 to keep the file small."""
+    from oracle.golden_sample import keep_samples
+    preds = [torch.from_numpy(np.asarray(p, np.float16).astype(np.float32)).requires_grad_(True) for p in maps]
+    losses = [structure_loss_ref(p, mask) for p in preds]
+    loss = 0.5 * losses[2] + 0.3 * losses[1] + 0.2 * losses[0]
+    loss.backward()
+    out = {"losses": np.asarray([l.item() for l in losses] + [loss.item()], np.float64)}
+    for n, p in zip(("x", "1", "2"), preds):
+        out["pred_" + n] = p.detach().numpy().astype(np.float16)
+        out["dpred_" + n] = p.grad.numpy().astype(np.float32)
+    keep_samples(out, {"dpred_" + n: 16384 for n in ("x", "1", "2")})
+    return out
+
+
 KEEP_FULL = ("resnet.conv1.weight", "resnet.bn1.weight", "resnet.layer1.0.conv1.weight", "resnet.layer2.0.downsample.0.weight",
              "resnet.layer3.5.bn2.bias", "up1.conv.identity.0.weight", "up_c.fc1.weight", "up_c.fc2.bias", "up_c.spatial.conv.weight",
              "up_c.spatial.bn.weight", "up_c.W_g.conv.bias", "up_c.residual.bn1.weight", "up_c.residual.conv3.conv.weight",
              "up_c_1_2.attn_block.psi.0.weight", "up_c_1_2.attn_block.psi.1.weight", "up_c_2_2.attn_block.W_x.0.weight",
              "final_x.2.conv.weight", "final_1.1.conv.bias", "final_2.0.bn.weight", "transformer.norm.weight",
              "transformer.blocks.0.attn.domain_layer.2.bias", "transformer.patch_embed.proj.bias")
+# the maps and the larger of the gradients above kept as seeded samples of their elements (oracle/golden_sample.py)
+SAMPLED = {**{n: 16384 for n in ("map_x", "map_1", "map_2", "eval_map_x", "eval_map_1", "eval_map_2")},
+           **{"grad." + n: 8192 for n in ("resnet.conv1.weight", "resnet.layer1.0.conv1.weight", "up1.conv.identity.0.weight",
+                                          "up_c.fc1.weight", "up_c.residual.conv3.conv.weight")}}
+
+
+def save(out, mask):
+    """Writes both golden files from the reference's outputs (`out` holds full tensors; it is sampled in place)."""
+    from oracle.golden_sample import keep_samples
+    sl = structure_loss_golden([out[n] for n in ("map_x", "map_1", "map_2")], mask)
+    keep_samples(out, SAMPLED)
+    for name, d in (("transfuse_model_golden.npz", out), ("transfuse_structure_loss_golden.npz", sl)):
+        path = os.path.join(ROOT, "tests", "golden", name)
+        np.savez_compressed(path, **d)
+        print("wrote", path, os.path.getsize(path) // 1024, "KiB")
 
 
 def main():
@@ -73,9 +104,6 @@ def main():
     for n, p in zip(("map_x", "map_1", "map_2"), maps):
         out[n] = p.detach().numpy().astype(np.float32)
     out["losses"] = np.asarray([l.item() for l in losses] + [loss.item()], np.float64)
-    gmaps = torch.autograd.grad(loss, maps, retain_graph=True)
-    for n, g in zip(("dmap_x", "dmap_1", "dmap_2"), gmaps):
-        out[n] = g.numpy().astype(np.float32)
     loss.backward()
     named = [(n, p.grad) for n, p in m.named_parameters() if p.grad is not None]
     out["grad_names"] = np.asarray([n for n, _ in named])
@@ -94,9 +122,8 @@ def main():
     for n, p in zip(("eval_map_x", "eval_map_1", "eval_map_2"), emaps):
         out[n] = p.numpy().astype(np.float16)
     out["eval_absmax"] = np.asarray([p.abs().max().item() for p in emaps])
-    path = os.path.join(ROOT, "tests", "golden", "transfuse_model_golden.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path) // 1024, "KiB; losses", out["losses"], "map absmax", [float(np.abs(out[n]).max()) for n in ("map_x", "map_1", "map_2")])
+    print("losses", out["losses"], "map absmax", [float(np.abs(out[n]).max()) for n in ("map_x", "map_1", "map_2")])
+    save(out, mask)
 
 
 if __name__ == "__main__":

@@ -17,6 +17,7 @@ import torch.nn.functional as F
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from mdvit_b200 import ops, transfuse as T      # noqa: E402
+from oracle import golden_sample as GS      # noqa: E402
 from oracle.make_golden_randinit import hard_dice      # noqa: E402
 from oracle.make_golden_transfuse_model import case, structure_loss_ref      # noqa: E402
 from tests import test_transfuse_wiring as W      # noqa: E402
@@ -89,12 +90,11 @@ g = np.load(os.path.join(ROOT, "tests", "golden", "transfuse_model_golden.npz"))
 img, mask, dlab = case()
 maps = m(img, dlab)
 for n, p in zip(("map_x", "map_1", "map_2"), maps):
-    ref = torch.from_numpy(g[n])
-    print(n, "max-abs / abs-max", ((p - ref).abs().max() / ref.abs().max()).item())
+    print(n, "max-abs / abs-max", GS.rel_max(p, g, n))
 ls = [structure_loss_ref(p, mask) for p in maps]
 (0.5 * ls[2] + 0.3 * ls[1] + 0.2 * ls[0]).backward()
 named = dict((n, p.grad) for n, p in m.named_parameters() if p.grad is not None)
 for k in g.files:
     if k.startswith("grad."):
-        ref, got = torch.from_numpy(g[k]), named[k[5:]]
-        print(f"  {k}: max-abs {((got - ref).abs().max() / (ref.abs().max() + 1e-30)).item():.3e}  rel-L2 {((got - ref).norm() / (ref.norm() + 1e-30)).item():.3e}")
+        got = named[k[5:]]
+        print(f"  {k}: max-abs {GS.rel_max(got, g, k):.3e}  rel-L2 {GS.rel_l2(got, g, k):.3e}")

@@ -11,6 +11,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from mdvit_b200 import _lib as L, ops, transfuse as T      # noqa: E402
+from oracle import golden_sample as GS      # noqa: E402
 from oracle.make_golden_transfuse_model import case      # noqa: E402
 from tests import test_transfuse_wiring as W      # noqa: E402
 from tests.helpers import fingerprint      # noqa: E402
@@ -54,8 +55,7 @@ def main():
     maps, losses, loss = step(m, img, mask, dlab, True)
     torch.cuda.synchronize()
     for n, p in zip(("map_x", "map_1", "map_2"), maps):
-        ref = torch.from_numpy(g[n]).to(dev)
-        print(f"{n}: rel err {((p - ref).abs().max() / ref.abs().max()).item():.3e}")
+        print(f"{n}: rel err {GS.rel_max(p, g, n):.3e}")
     print("losses", [round(l.item(), 6) for l in losses], loss.item(), "golden", g["losses"])
     named = [(n, p.grad) for n, p in m.named_parameters() if p.grad is not None]
     fp, ref_fp = fingerprint(named), g["grad_fp"]

@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from mdvit_b200 import synth
+from oracle.golden_sample import rel_max
 from tests.helpers import fingerprint
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -160,17 +161,13 @@ def test_deeplab_aux_decoder_logits_and_gradients_match_reference_golden(dgold):
     img, _ = synth.synth_batch(15, 1, 2, 256, 256)
     dl = torch.nn.functional.one_hot(torch.full((2,), 1), 4).float().to(dev)
 
-    def rel(a, b):
-        b = torch.as_tensor(b).float()
-        return ((a.detach().float().cpu() - b).abs().max() / b.abs().max()).item()
-
     m.eval()
     with torch.no_grad():
         o, a = m(img.to(dev), dl, "1")
-    assert rel(o, dgold["dl_eval_out"]) < 2e-2 and rel(a, dgold["dl_eval_aux"]) < 3e-2
+    assert rel_max(o, dgold, "dl_eval_out") < 2e-2 and rel_max(a, dgold, "dl_eval_aux") < 3e-2
     m.train()
     o, a = m(img.to(dev), dl, "1")
-    assert rel(a, dgold["dl_train_aux"]) < 3e-2
+    assert rel_max(a, dgold, "dl_train_aux") < 3e-2
     R = synth.synth_tensor("dl_probe", tuple(a.shape)).to(dev)
     (a * R).sum().backward()
     names = [str(n) for n in dgold["dl_grad_names"]]

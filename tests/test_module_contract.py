@@ -108,7 +108,7 @@ def test_random_init_is_bit_identical_to_the_reference_constructor():
     """BASELINE.json north_star: parity "on identical random-init weights".  torch.manual_seed(0) + MDViT(...) must give the
     weights the reference's stock constructor gives from the same seed (mdvit.py:484-504,648-664), including the dead
     construction-time draws of its conv containers — checked against fingerprints of the UNMODIFIED reference's parameters
-    (oracle/make_golden_randinit.py), and directly against the reference when /root/reference is present."""
+    (oracle/make_golden_randinit.py)."""
     import os
     import numpy as np
     from mdvit_b200.model import MDViT
@@ -121,10 +121,3 @@ def test_random_init_is_bit_identical_to_the_reference_constructor():
     assert names == [n for n, _ in m.named_parameters()]
     fp = fingerprint(list(m.named_parameters()))
     assert np.abs(fp - rg["init_fp"]).max() <= 1e-9 * np.abs(rg["init_fp"]).max()
-    from oracle import ref_shim
-    if ref_shim.available():
-        ref = ref_shim.load_reference()
-        torch.manual_seed(0)
-        r = ref.MDViT(img_size=256, drop_rate=0.0, drop_path_rate=0.0, adapt_method="Sup", num_domains=4, decoder_name="MLPFM")
-        a, b = r.state_dict(), m.state_dict()
-        assert list(a) == list(b) and all(torch.equal(a[k], b[k]) for k in a)

@@ -10,11 +10,13 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from oracle import golden_sample as GS
 from oracle.make_golden_transfuse_model import case, structure_loss_ref
 from tests.helpers import fingerprint
 from tests.test_transfuse_wiring import _EmuConv
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "transfuse_model_golden.npz")
+LOSS_GOLD = os.path.join(os.path.dirname(__file__), "golden", "transfuse_structure_loss_golden.npz")
 pytestmark = pytest.mark.gpu
 FWD_TOL, BWD_TOL = 2e-3, 2e-2
 
@@ -184,19 +186,19 @@ def test_resize_align_corners_fwd_bwd(shape):
 def test_structure_loss_vs_reference_formula_and_golden():
     from mdvit_b200 import ops
     dev = _dev()
-    g = np.load(GOLD)
+    g = np.load(LOSS_GOLD)          # the reference's three maps (fp16) with the loss and its gradient on them
     _, mask, _ = case()
     mask = mask.to(dev)
     weit = ops.structure_weit(mask)
     ref_weit = 1 + 5 * torch.abs(F.avg_pool2d(mask, kernel_size=31, stride=1, padding=15) - mask)
     assert rel(weit, ref_weit) < 1e-5
-    for i, n in enumerate(("map_x", "map_1", "map_2")):
-        pred = torch.from_numpy(g[n]).to(dev).requires_grad_(True)
+    for i, n in enumerate(("x", "1", "2")):
+        pred = torch.from_numpy(g["pred_" + n].astype(np.float32)).to(dev).requires_grad_(True)
         loss = ops.structure_loss(pred, mask, weit)
         assert abs(loss.item() - g["losses"][i]) < 2e-5 * abs(g["losses"][i])
         coef = (0.2, 0.3, 0.5)[i]
         (coef * loss).backward()
-        assert rel(pred.grad, g["d" + n]) < 1e-4
+        assert GS.rel_max(pred.grad, g, "dpred_" + n) < 1e-4
     # a saturated / random case against the formula itself
     pred = (8 * torch.randn(3, 1, 64, 64, device=dev)).requires_grad_(True)
     m2 = (torch.rand(3, 1, 64, 64, device=dev) > 0.6).float()
@@ -272,8 +274,8 @@ def test_model_maps_and_losses_match_reference_golden(trained_once):
     g = np.load(GOLD)
     (maps, losses, _), (smaps, _, _), sd_after, _ = trained_once
     for n, p, sp in zip(("map_x", "map_1", "map_2"), maps, smaps):
-        assert tuple(p.shape) == g[n].shape
-        e, es = rel(p, g[n]), rel(sp, g[n])
+        assert tuple(p.shape) == GS.shape(g, n)
+        e, es = GS.rel_max(p, g, n), GS.rel_max(sp, g, n)
         print(f"{n}: ours {e:.3e}, stock PyTorch TF32 {es:.3e}")
         assert e < max(1e-2, 2.0 * es) and e < 3e-2, (n, e, es)
     np.testing.assert_allclose(losses, g["losses"], rtol=2e-3)
@@ -309,9 +311,9 @@ def test_model_gradients_match_reference_golden(trained_once):
     for k in g.files:
         if k.startswith("grad."):
             n = k[5:]
-            if np.abs(g[k]).max() < 1e-3 * med or ".psi.1." in n or ".spatial.bn." in n:
+            if GS.absmax(g, k) < 1e-3 * med or ".psi.1." in n or ".spatial.bn." in n:
                 continue
-            e, es = rel(grads[n], g[k]), rel(sgrads[n], g[k])
+            e, es = GS.rel_max(grads[n], g, k), GS.rel_max(sgrads[n], g, k)
             print(f"{k}: ours {e:.3e}, stock PyTorch TF32 {es:.3e}")
             assert e < max(5e-2, 2.5 * es) and e < 0.5, (k, e, es)
 
@@ -320,7 +322,7 @@ def test_model_eval_maps_match_reference_golden(trained_once):
     g = np.load(GOLD)
     emaps = trained_once[3]
     for n, p in zip(("eval_map_x", "eval_map_1", "eval_map_2"), emaps):
-        assert rel(p, g[n].astype(np.float32)) < 3e-2, (n, rel(p, g[n].astype(np.float32)))
+        assert GS.rel_max(p, g, n) < 3e-2, (n, GS.rel_max(p, g, n))
 
 
 def test_transfuse_trainer_eager_and_graph_steps_agree():

@@ -10,6 +10,7 @@ import torch
 import torch.nn.functional as F
 
 from mdvit_b200 import ops, transfuse as T
+from oracle import golden_sample as GS
 from oracle.make_golden_transfuse_model import case, structure_loss_ref
 from tests.helpers import fingerprint
 
@@ -36,7 +37,10 @@ def test_constructor_reproduces_reference_keys_and_init():
     torch.manual_seed(0)
     m = T.TransFuse_S_adapt(drop_rate=0.0)
     assert list(m.state_dict().keys()) == list(g["keys"])
-    np.testing.assert_array_equal(fingerprint(list(m.named_parameters())), g["init_fp"])      # bit-identical weights
+    # bit-identical weights: the fingerprints are float64 sums whose last bits depend on the host CPU's summation order, so they
+    # must agree to 1e-12 of each tensor's norm (a zero tensor's fingerprint is exactly zero)
+    fp, ref = fingerprint(list(m.named_parameters())), g["init_fp"]
+    assert (np.abs(fp - ref).max(axis=1) <= 1e-12 * ref[:, 0]).all()
 
 
 def test_wiring_matches_reference_forward_backward_on_cpu(emulated):
@@ -46,9 +50,8 @@ def test_wiring_matches_reference_forward_backward_on_cpu(emulated):
     img, mask, dlab = case()
     maps = m(img, dlab)
     for n, p in zip(("map_x", "map_1", "map_2"), maps):
-        ref = torch.from_numpy(g[n])
-        assert p.shape == ref.shape
-        assert (p - ref).abs().max().item() <= 2e-4 * ref.abs().max().item(), n
+        assert tuple(p.shape) == GS.shape(g, n)
+        assert GS.rel_max(p, g, n) <= 2e-4, n
     losses = [structure_loss_ref(p, mask) for p in maps]
     loss = 0.5 * losses[2] + 0.3 * losses[1] + 0.2 * losses[0]
     np.testing.assert_allclose([l.item() for l in losses] + [loss.item()], g["losses"], rtol=2e-5)
