@@ -184,6 +184,11 @@ int mdv_col2im3_dil(const float* dcol, float* dx, int B, int H, int W, int C, in
 /* bilinear resize, align_corners=False (mdvit.py:699; Decoders.py:196,319-336) and its exact transpose */
 int mdv_upsample_fwd(const void* in, int in_bf16, int ld_in, void* out, int out_bf16, int ld_out, int B, int Hi, int Wi, int Ho,
                      int Wo, int C, void* stream);
+/* out[b,y,x,c] += sum_k resize(in_k)[b,y,x,c] (align_corners=False) for up to three fp32 maps in_k [B,Hk,Wk,C] (NULL: skipped),
+ * one pass over out [B,Ho,Wo] with pixel pitch ld_out: the upsampled stage-2..4 terms of the collapsed MLPDecoderFM
+ * (Decoders.py:317-333, see ops.AuxFn).  C, ld_out % 4 == 0, pointers 16-byte aligned. */
+int mdv_upsample_add(float* out, int ld_out, int B, int Ho, int Wo, int C, const float* in0, int H0, int W0, const float* in1, int H1,
+                     int W1, const float* in2, int H2, int W2, void* stream);
 /* ws: optional scratch of B*Ho*Wi*C floats; with it, integer factors 4 and 8 use the separable two-pass form */
 int mdv_upsample_bwd(const void* dout, int dout_bf16, int ld_out, float* din, int ld_in, int B, int Hi, int Wi, int Ho, int Wo,
                      int C, float* ws, void* stream);
@@ -285,6 +290,19 @@ int mdv_colsum(const void* x, int x_bf16, int ld, float* out, int M, int C, void
 int mdv_cast_bf16(const float* in, int ld_in, void* out_bf16, int ld_out, long long M, int C, const float* rowscale,
                   int rows_per_scale, float drop_p, const void* rng, uint32_t drop_stream, float* colsum, void* stream);
 int mdv_add_f32(const void* in, int in_bf16, int ld_in, float* out, int ld_out, long long M, int C, int accumulate, void* stream);
+/* Up to 16 independent fp32 FFMA products in one launch (`descs`: HOST array of n descriptors, distinct C):
+ *   C[M,N] = (accumulate ? C : 0) + op(A)[M,K] . op(B)[K,N] (+ u[m] v[n] when u, v are not NULL),
+ * op(A)[m,k] = trans_a ? A[k*lda + m] : A[m*lda + k], op(B) likewise.  The weight-sized products of the collapsed MLPDecoderFM
+ * (ops.AuxFn): Wf_i W_i and Wf_i b_i in the forward; E_i W_i^T + s b_i^T, Wf_i^T E_i and Wf_i^T s for the weight gradients. */
+typedef struct MdvMatmulDesc {
+    const float* A;
+    const float* B;
+    float* C;
+    const float* u;
+    const float* v;
+    int lda, ldb, ldc, M, N, K, trans_a, trans_b, accumulate, pad_;
+} MdvMatmulDesc;
+int mdv_matmul_f32_grouped(const MdvMatmulDesc* descs, int n, void* stream);
 /* fp32 master weight -> GEMM operand.  mode 0 copy, 1 transpose, 2 conv3x3 -> im2col order, 3 = transpose of 2, 4 = conv3x3 ->
  * [Cin, tap*Cout + co] (input-gradient operand of mdv_conv3_gemm); dst is bf16, or
  * fp32 (TF32 GEMM operand) when 8 is added to the mode */

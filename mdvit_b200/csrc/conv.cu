@@ -651,6 +651,77 @@ __global__ void __launch_bounds__(256) upsample_fwd_walk8_kernel(const bf16* __r
     }
 }
 
+// out[b, y, x, :] += sum_k resize(in_k)[b, y, x, :] for up to three fp32 maps of different sizes, one read-modify-write of
+// `out`: the stage-2..4 terms of the collapsed aux decoder (ops.AuxFn).  Same column walk as upsample_fwd_walk_kernel, with
+// the two horizontally interpolated source rows of every input kept in registers.
+struct UpIn3 {
+    const float* p[3];
+    int H[3], W[3];
+};
+
+__global__ void __launch_bounds__(256) upsample_add_kernel(UpIn3 in, int n_in, float* __restrict__ out, int ld_out, int Ho, int Wo, int C,
+                                                           int seg) {
+    MDV_PDL_SYNC();
+    const int c4n = C >> 2;
+    const int t = blockIdx.x * 256 + threadIdx.x;
+    if (t >= Wo * c4n) return;
+    const int x = t / c4n, c = (t % c4n) * 4;
+    const float* base[3];
+    int x0[3], x1[3], i0[3], i1[3];
+    float lx[3];
+    float4 h0[3], h1[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        if (k < n_in) {
+            bil_src(x, (float)in.W[k] / Wo, in.W[k], x0[k], x1[k], lx[k]);
+            base[k] = in.p[k] + (size_t)blockIdx.z * in.H[k] * in.W[k] * C + c;
+        }
+        i0[k] = i1[k] = -1;
+        h0[k] = h1[k] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+    float* obase = out + ((size_t)blockIdx.z * Ho * Wo + x) * ld_out + c;
+    const int y0 = blockIdx.y * seg, y1 = min(Ho, y0 + seg);
+    // four rows of `out` in flight per thread: the pass is HBM-bound, one outstanding 16-byte load per thread is not enough
+    for (int yb = y0; yb < y1; yb += 4) {
+        float4 o[4];
+#pragma unroll
+        for (int r = 0; r < 4; ++r)
+            if (yb + r < y1) o[r] = ld4(obase + (size_t)(yb + r) * Wo * ld_out);
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+            const int y = yb + r;
+            if (y >= y1) break;
+#pragma unroll
+            for (int k = 0; k < 3; ++k) {
+                if (k >= n_in) break;
+                const int Wi = in.W[k];
+                auto hload = [&](int ys) {
+                    const float4 a = ld4(base[k] + ((size_t)ys * Wi + x0[k]) * C), b = ld4(base[k] + ((size_t)ys * Wi + x1[k]) * C);
+                    return make_float4(a.x + lx[k] * (b.x - a.x), a.y + lx[k] * (b.y - a.y), a.z + lx[k] * (b.z - a.z), a.w + lx[k] * (b.w - a.w));
+                };
+                int ys0, ys1;
+                float ly;
+                bil_src(y, (float)in.H[k] / Ho, in.H[k], ys0, ys1, ly);
+                if (ys0 != i0[k]) {
+                    h0[k] = ys0 == i1[k] ? h1[k] : hload(ys0);
+                    i0[k] = ys0;
+                }
+                if (ys1 != i1[k]) {
+                    h1[k] = ys1 == i0[k] ? h0[k] : hload(ys1);
+                    i1[k] = ys1;
+                }
+                o[r].x += h0[k].x + ly * (h1[k].x - h0[k].x);
+                o[r].y += h0[k].y + ly * (h1[k].y - h0[k].y);
+                o[r].z += h0[k].z + ly * (h1[k].z - h0[k].z);
+                o[r].w += h0[k].w + ly * (h1[k].w - h0[k].w);
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < 4; ++r)
+            if (yb + r < y1) st4(obase + (size_t)(yb + r) * Wo * ld_out, o[r]);
+    }
+}
+
 // single-channel variant (the commuted segmentation heads): in [B,Hi,Wi] fp32 -> out [B,Ho,Wo] fp32
 __global__ void __launch_bounds__(256) upsample1_fwd_kernel(const float* __restrict__ in, float* __restrict__ out, int B, int Hi,
                                                              int Wi, int Ho, int Wo) {
@@ -1167,6 +1238,29 @@ extern "C" int mdv_upsample_fwd(const void* in, int in_bf16, int ld_in, void* ou
         mdv_launch((upsample_fwd_walk_kernel<float, float>), grid, dim3(256), 0, st, (const float*)in, ld_in, (float*)out, ld_out, Hi, Wi, Ho, Wo, C, seg);
     else
         return MDV_ERR_UNSUPPORTED;
+    MDV_CHECK_LAUNCH();
+    return MDV_OK;
+}
+
+extern "C" int mdv_upsample_add(float* out, int ld_out, int B, int Ho, int Wo, int C, const float* in0, int H0, int W0, const float* in1,
+                                int H1, int W1, const float* in2, int H2, int W2, void* stream) {
+    if (!out || B <= 0 || Ho <= 0 || Wo <= 0 || C <= 0 || (C & 3) || (ld_out & 3) || ld_out < C || (reinterpret_cast<uintptr_t>(out) & 15))
+        return MDV_ERR_ARG;
+    UpIn3 in = {};
+    int n = 0;
+    const float* ps[3] = {in0, in1, in2};
+    const int hs[3] = {H0, H1, H2}, ws[3] = {W0, W1, W2};
+    for (int k = 0; k < 3; ++k) {
+        if (!ps[k]) continue;
+        if (hs[k] <= 0 || ws[k] <= 0 || (reinterpret_cast<uintptr_t>(ps[k]) & 15)) return MDV_ERR_ARG;
+        if (!fits_i32((long long)B * hs[k] * ws[k] * C)) return MDV_ERR_UNSUPPORTED;
+        in.p[n] = ps[k]; in.H[n] = hs[k]; in.W[n] = ws[k];
+        ++n;
+    }
+    if (!n) return MDV_OK;
+    const int seg = Ho >= 64 ? 32 : Ho;
+    mdv_launch(upsample_add_kernel, dim3(mdv_cdiv(Wo * (C / 4), 256), mdv_cdiv(Ho, seg), B), dim3(256), 0, (cudaStream_t)stream, in, n, out,
+               ld_out, Ho, Wo, C, seg);
     MDV_CHECK_LAUNCH();
     return MDV_OK;
 }

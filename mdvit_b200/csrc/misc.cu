@@ -370,6 +370,69 @@ __global__ void __launch_bounds__(256) add_f32_kernel(const TI* __restrict__ in,
     }
 }
 
+// Grouped fp32 FFMA products C[M,N] (=|+=) op(A)[M,K] . op(B)[K,N] (+ u[m] v[n]): the weight-sized products of the collapsed aux
+// decoder.  Every problem of a group is independent (distinct C), so one grid covers them all: each is only 16-256 tiles and K <= 512,
+// i.e. latency-bound, and launched one by one they ran back to back.  32 x 32 output tile per block, 2 x 2 per thread, k-steps of
+// 32 staged in shared memory; the staging loads walk whichever index is contiguous in memory, so both orientations are coalesced.
+constexpr int MM_T = 32;
+constexpr int MM_MAX = 16;
+
+struct MatmulGroup {
+    MdvMatmulDesc d[MM_MAX];
+    int tile0[MM_MAX + 1];      // first block of each problem
+    int n;
+};
+
+__global__ void __launch_bounds__(256) matmul_f32_kernel(const __grid_constant__ MatmulGroup g) {
+    MDV_PDL_SYNC();
+    __shared__ float As[MM_T][MM_T + 1], Bs[MM_T][MM_T + 1];    // [k][m], [k][n]
+    int p = 0;
+    while (p + 1 < g.n && (int)blockIdx.x >= g.tile0[p + 1]) ++p;
+    const MdvMatmulDesc& d = g.d[p];
+    const int t = blockIdx.x - g.tile0[p], ntn = (d.N + MM_T - 1) / MM_T;
+    const int m0 = (t / ntn) * MM_T, n0 = (t % ntn) * MM_T;
+    const int M = d.M, N = d.N, K = d.K, ta = d.trans_a, tb = d.trans_b, lda = d.lda, ldb = d.ldb;
+    const float* __restrict__ A = d.A;
+    const float* __restrict__ B = d.B;
+    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+    float acc[2][2] = {};
+    for (int k0 = 0; k0 < K; k0 += MM_T) {
+        for (int e = threadIdx.x; e < MM_T * MM_T; e += 256) {
+            const int r = e / MM_T, q = e % MM_T;       // q: the index contiguous in memory
+            {
+                const int m = ta ? q : r, k = ta ? r : q, gm = m0 + m, gk = k0 + k;
+                As[k][m] = (gm < M && gk < K) ? A[ta ? (size_t)gk * lda + gm : (size_t)gm * lda + gk] : 0.f;
+            }
+            {
+                const int n = tb ? r : q, k = tb ? q : r, gn = n0 + n, gk = k0 + k;
+                Bs[k][n] = (gn < N && gk < K) ? B[tb ? (size_t)gn * ldb + gk : (size_t)gk * ldb + gn] : 0.f;
+            }
+        }
+        __syncthreads();
+#pragma unroll 8
+        for (int k = 0; k < MM_T; ++k) {
+            const float a0 = As[k][ty], a1 = As[k][ty + 16], b0 = Bs[k][tx], b1 = Bs[k][tx + 16];
+            acc[0][0] = fmaf(a0, b0, acc[0][0]);
+            acc[0][1] = fmaf(a0, b1, acc[0][1]);
+            acc[1][0] = fmaf(a1, b0, acc[1][0]);
+            acc[1][1] = fmaf(a1, b1, acc[1][1]);
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int i = 0; i < 2; ++i)
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+            const int m = m0 + ty + 16 * i, n = n0 + tx + 16 * j;
+            if (m < M && n < N) {
+                float v = acc[i][j];
+                if (d.u) v = fmaf(d.u[m], d.v[n], v);
+                float* c = d.C + (size_t)m * d.ldc + n;
+                *c = d.accumulate ? *c + v : v;
+            }
+        }
+}
+
 // Weight preparation: dst[r, c] = bf16(src[...]) with optional transpose / 3x3-conv permutation.
 //  mode 0: src [R, Cc] row-major                       -> dst [R, ld]        (Linear / 1x1 conv weight)
 //  mode 1: src [R, Cc] row-major                       -> dst [Cc, ld] = src^T (for input gradients)
@@ -742,6 +805,23 @@ extern "C" int mdv_add_f32(const void* in, int in_bf16, int ld_in, float* out, i
     if (!in || !out) return MDV_ERR_ARG;
     if (in_bf16) mdv_launch(add_f32_kernel<bf16>, dim3(grid_for(M * C)), dim3(256), 0, (cudaStream_t)stream, (const bf16*)in, ld_in, out, ld_out, M, C, accumulate);
     else mdv_launch(add_f32_kernel<float>, dim3(grid_for(M * C)), dim3(256), 0, (cudaStream_t)stream, (const float*)in, ld_in, out, ld_out, M, C, accumulate);
+    MDV_CHECK_LAUNCH();
+    return MDV_OK;
+}
+
+extern "C" int mdv_matmul_f32_grouped(const MdvMatmulDesc* descs, int n, void* stream) {
+    if (!descs || n <= 0 || n > MM_MAX) return MDV_ERR_ARG;
+    MatmulGroup g = {};
+    g.n = n;
+    for (int i = 0; i < n; ++i) {
+        const MdvMatmulDesc& d = descs[i];
+        if (!d.A || !d.B || !d.C || d.M <= 0 || d.N <= 0 || d.K <= 0 || d.lda < (d.trans_a ? d.M : d.K) || d.ldb < (d.trans_b ? d.K : d.N) ||
+            d.ldc < d.N || (!d.u != !d.v))
+            return MDV_ERR_ARG;
+        g.d[i] = d;
+        g.tile0[i + 1] = g.tile0[i] + mdv_cdiv(d.M, MM_T) * mdv_cdiv(d.N, MM_T);
+    }
+    mdv_launch(matmul_f32_kernel, dim3(g.tile0[n]), dim3(256), 0, (cudaStream_t)stream, g);
     MDV_CHECK_LAUNCH();
     return MDV_OK;
 }

@@ -323,6 +323,39 @@ def upsample_bwd(dout, B, Hi, Wi, Ho, Wo, C, ld_out=None):
     return din
 
 
+def upsample_add(out, ins, B, Ho, Wo, C, ld_out=None):
+    """out [B*Ho*Wo, C] fp32 += sum of the bilinear resizes of the fp32 maps `ins` = [(x [B*Hi*Wi, C], Hi, Wi)] (at most 3)."""
+    args = []
+    for x, Hi, Wi in list(ins) + [(None, 0, 0)] * (3 - len(ins)):
+        args += [ptr(x), Hi, Wi]
+    check(L.lib().mdv_upsample_add(ptr(out), ld_out or C, B, Ho, Wo, C, *args, L.stream()), "mdv_upsample_add")
+    return out
+
+
+class _MatmulDesc(ctypes.Structure):
+    _fields_ = [("A", ctypes.c_void_p), ("B", ctypes.c_void_p), ("C", ctypes.c_void_p), ("u", ctypes.c_void_p), ("v", ctypes.c_void_p)] + \
+               [(n, ctypes.c_int) for n in ("lda", "ldb", "ldc", "M", "N", "K", "trans_a", "trans_b", "accumulate", "pad_")]
+
+
+def mm(A, B, C, M, N, K, *, lda=None, ldb=None, ldc=None, trans_a=False, trans_b=False, accumulate=False, u=None, v=None):
+    """One problem of matmul_f32: C[M,N] (+)= op(A)[M,K] . op(B)[K,N] (+ u v^T), op = transpose when trans_*.  None when C is None
+    (the gradient it would produce is off in this backward mode).  The descriptor holds references to its tensors until the
+    launch: it carries raw device pointers, and a tensor freed before then could have its memory handed to the next one."""
+    if C is None:
+        return None
+    d = _MatmulDesc(ptr(A), ptr(B), ptr(C), ptr(u), ptr(v), lda or (M if trans_a else K), ldb or (K if trans_b else N), ldc or N, M, N, K,
+                    int(trans_a), int(trans_b), int(accumulate), 0)
+    d.tensors = (A, B, C, u, v)
+    return d
+
+
+def matmul_f32(problems):
+    """Independent fp32 products (mm(...) descriptors with distinct outputs; None entries skipped) in one launch."""
+    ds = [d for d in problems if d is not None]
+    if ds:
+        check(L.lib().mdv_matmul_f32_grouped((_MatmulDesc * len(ds))(*ds), len(ds), L.stream()), "mdv_matmul_f32_grouped")
+
+
 def _contig(t):
     return t if t.is_contiguous() else t.contiguous()
 
@@ -1238,8 +1271,26 @@ class HeadFn(torch.autograd.Function):
         return dx, rw, rb, None, None, None, None
 
 
+def _bf16_t(w, R, Cc):
+    """bf16 [Cc, R] = w^T of a contiguous fp32 [R, Cc] that is not a parameter (no operand cache: recomputed every forward)."""
+    dst = torch.empty((Cc, R), dtype=BF16, device=w.device)
+    check(L.lib().mdv_prep_weight(ptr(w), ptr(dst), R, Cc, R, 1, 0, L.stream()), "mdv_prep_weight")
+    return dst
+
+
 class AuxFn(torch.autograd.Function):
-    """MLPDecoderFM.forward (Decoders.py:315-339): the MKD auxiliary 'peer' decoder."""
+    """MLPDecoderFM.forward (Decoders.py:315-339): the MKD auxiliary 'peer' decoder, with linear_fuse folded into linear1-4.
+
+    A bilinear resize (align_corners=False) is linear per channel with weights summing to 1, and a 1x1 conv is linear per
+    pixel, so with Wf_i the column block of linear_fuse's weight that multiplies input i (order x1..x4, x5):
+        z = Wf . cat(up(W_i x_i + b_i), x5) + bf = [W'_1 | Wf_5] . [x1 | x5] + bf + c_1 + sum_{i=2..4} up(W'_i x_i + c_i),
+        W'_i = Wf_i W_i,   c_i = Wf_i b_i.
+    The [M0, 2112] concat and its K = 2112 GEMMs never exist: z is one K = C1 + C5 GEMM at full resolution, three GEMMs at
+    the stage resolutions (outputs y_i kept in fp32) and one upsample-accumulate pass.  W'_i and c_i are computed in fp32
+    from the master weights in every forward (so a captured step graph sees each optimizer update).  Backward, with dz the
+    gradient of z, dz_i = up^T(dz) and s = colsum(dz) (= colsum(dz_i)):
+        dx1 | dx5 = dz [W'_1 | Wf_5],  dx_i = dz_i W'_i,  E_i = dz_i^T x_i,
+        dWf_i += E_i W_i^T + s b_i^T,  dWf_5 += E_5,  dW_i += Wf_i^T E_i,  db_i += Wf_i^T s,  dbf += s."""
 
     @staticmethod
     def forward(ctx, x1, x2, x3, x4, x5, l1w, l1b, l2w, l2b, l3w, l3b, l4w, l4b, fw, fb, g, b, ow, ob, bufs, sizes, Ho, Wo, drop2d,
@@ -1253,44 +1304,53 @@ class AuxFn(torch.autograd.Function):
         hc = fw.shape[0]               # 512
         K = fw.shape[1]                # 2112 (MLPDecoderFM) / 2048 (MLPDecoder)
         C5 = x5.shape[2] if x5 is not None else 0
+        Cs = [t.shape[2] for t in xs]
+        C1 = Cs[0]
+        Kx = C1 + C5
         rm, rv, nb = bufs
         lib = L.lib()
         lw, lb = (l1w, l2w, l3w, l4w), (l1b, l2b, l3b, l4b)
         with _dev_ctx(x1):
-            cat = torch.empty((M0, K), dtype=BF16, device=dev)
-            acts = []
-            for i in range(4):
+            # collapsed weights: w1x = [W'_1 | Wf_5] (fp32 [hc, Kx]) and W'_2..4; bias c_i = Wf_i b_i (c_1 also takes bf), added to
+            # the stage-i product before the resize (a resize keeps constants)
+            w1x = torch.empty((hc, Kx), dtype=F32, device=dev)
+            if C5:
+                check(lib.mdv_add_f32(ptr(fw[:, 4 * hc:]), 0, K, ptr(w1x[:, C1:]), Kx, hc, C5, 0, L.stream()), "mdv_add_f32")
+            wps = [torch.empty((hc, Cs[i]), dtype=F32, device=dev) for i in range(1, 4)]
+            cb = torch.empty((4, hc), dtype=F32, device=dev)
+            check(lib.mdv_add_f32(ptr(fb), 0, hc, ptr(cb), hc, 1, hc, 0, L.stream()), "mdv_add_f32")
+            matmul_f32([mm(fw, lw[0], w1x, hc, C1, hc, lda=K, ldc=Kx)] +
+                       [mm(fw[:, i * hc:], lw[i], wps[i - 1], hc, Cs[i], hc, lda=K) for i in range(1, 4)] +
+                       [mm(fw[:, i * hc:], lb[i], cb[i], hc, 1, hc, lda=K, accumulate=i == 0) for i in range(4)])
+            # z = [x1 | x5] . w1x^T + c_1 + sum_i up(x_i . W'_i^T + c_i)
+            xa = torch.empty((M0, Kx), dtype=BF16, device=dev)
+            cast_bf16(xs[0], M0, C1, out=xa, ld_out=Kx)
+            if C5:
+                cast_bf16(x5, M0, C5, out=xa[:, C1:], ld_out=Kx)
+            z = torch.empty((M0, hc), dtype=F32, device=dev)
+            gemm_nt(xa, cast_bf16(w1x, hc, Kx), M0, hc, Kx, z, bias=cb[0])
+            acts, ys = [xa], []
+            for i in range(1, 4):
                 Hi, Wi = sizes[i]
-                Mi, Ci = B * Hi * Wi, xs[i].shape[2]
+                Mi, Ci = B * Hi * Wi, Cs[i]
                 a = cast_bf16(xs[i], Mi, Ci)
                 acts.append(a)
-                wb = prep_weight(lw[i], 0, hc, Ci)
-                if i == 0:
-                    gemm_nt(a, wb, Mi, hc, Ci, cat, ldc=K, bias=lb[i])
-                else:
-                    t = torch.empty((Mi, hc), dtype=BF16, device=dev)
-                    gemm_nt(a, wb, Mi, hc, Ci, t, bias=lb[i])
-                    upsample_fwd(t, cat[:, i * hc:], B, Hi, Wi, H, W, hc, ld_out=K)
-            if x5 is not None:
-                cast_bf16(x5, M0, C5, out=cat[:, 4 * hc:], ld_out=K)
-            if not training:      # eval: conv bias + BatchNorm + ReLU folded into the linear_fuse GEMM epilogue
-                a5 = torch.empty((M0, hc), dtype=BF16, device=dev)
-                sc, sh = bn_fold(g, b, rm, rv, fb)
-                gemm_nt(cat, prep_weight(fw, 0, hc, K), M0, hc, K, a5, colscale=sc, bias=sh, act=ACT_RELU)
-                z = mean = rstd = None
-            else:
-                z = torch.empty((M0, hc), dtype=F32, device=dev)
-                gemm_nt(cat, prep_weight(fw, 0, hc, K), M0, hc, K, z, bias=fb)
-                a5, mean, rstd = bn_forward(z, M0, hc, g, b, rm, rv, nb, training, ACT_RELU, True)
+                ys.append((gemm_nt(a, cast_bf16(wps[i - 1], hc, Ci), Mi, hc, Ci, torch.empty((Mi, hc), dtype=F32, device=dev), bias=cb[i]), Hi, Wi))
+            upsample_add(z, ys, B, H, W, hc)
+            a5, mean, rstd = bn_forward(z, M0, hc, g, b, rm, rv, nb, training, ACT_RELU, True)
             p2 = drop2d if training else 0.0
             sid = new_stream_id() if p2 > 0 else 0
             lo = torch.empty(M0, dtype=F32, device=dev)
             check(lib.mdv_rowdot_fwd(ptr(a5), 1, ptr(ow), ptr(ob), ptr(lo), M0, hc, H * W, ctypes.c_float(p2),
                                      ptr(rng_tensor(dev)) if p2 > 0 else None, sid, L.stream()), "mdv_rowdot_fwd")
             out = upsample_fwd(lo, torch.empty((B, 1, Ho, Wo), dtype=F32, device=dev), B, H, W, Ho, Wo, 1)
-        ctx.save_for_backward(cat, z, mean, rstd, a5, *acts)
+            if training:     # input-gradient operands: bf16 transposes of the collapsed weights
+                wts = [_bf16_t(w1x, hc, Kx)] + [_bf16_t(wps[i - 1], hc, Cs[i]) for i in range(1, 4)]
+            else:
+                wts, z = [], None
+        ctx.save_for_backward(z, mean, rstd, a5, *acts, *wts)
         ctx.params = (l1w, l1b, l2w, l2b, l3w, l3b, l4w, l4b, fw, fb, g, b, ow, ob)
-        ctx.meta = (B, sizes, Ho, Wo, hc, K, C5, p2, sid, training, [t.shape[2] for t in xs])
+        ctx.meta = (B, sizes, Ho, Wo, hc, K, C5, p2, sid, training, Cs)
         _fwd_mark(ctx)
         return out
 
@@ -1299,10 +1359,13 @@ class AuxFn(torch.autograd.Function):
         B, sizes, Ho, Wo, hc, K, C5, p2, sid, training, Cs = ctx.meta
         if not training:
             raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
-        cat, z, mean, rstd, a5, *acts = ctx.saved_tensors
+        z, mean, rstd, a5, *rest = ctx.saved_tensors
+        acts, wts = rest[:4], rest[4:]
         l1w, l1b, l2w, l2b, l3w, l3b, l4w, l4b, fw, fb, g, b, ow, ob = ctx.params
         (H, W) = sizes[0]
         M0, dev = B * H * W, dout.device
+        C1 = Cs[0]
+        Kx = C1 + C5
         lib = L.lib()
         dout = _contig(dout.float())
         lw, lb = (l1w, l2w, l3w, l4w), (l1b, l2b, l3b, l4b)
@@ -1322,38 +1385,39 @@ class AuxFn(torch.autograd.Function):
                                            ptr(z), ptr(mean), ptr(rstd), ptr(g), ptr(b), ACT_RELU, ptr(dz), 1, ptr(g_g), ptr(g_b), M0, hc,
                                            ptr(ws_bn), L.stream()), "mdv_bn_act_bwd_rank1")
             g_fw, r_fw = gtarget(fw, (hc, K))
-            gemm_tn(dz, cat, M0, hc, K, g_fw)
             g_fb, r_fb = gtarget(fb)
-            colsum(dz, M0, hc, g_fb)
-            dcat = torch.empty((M0, K), dtype=BF16, device=dev)
-            gemm_nt(dz, prep_weight(fw, 1, hc, K), M0, K, hc, dcat)
-            gx, rw, rbs = [], [], []
-            for i in range(4):
+            tw = [gtarget(lw[i], (hc, Cs[i])) for i in range(4)]
+            tb = [gtarget(lb[i]) for i in range(4)]
+            wgrad = any(t is not None for t in [g_fw, g_fb] + [t[0] for t in tw + tb])
+            gx = [gemm_nt(dz, wts[0], M0, C1, hc, torch.empty((B, H * W, C1), dtype=F32, device=dev))]
+            dx5 = gemm_nt(dz, wts[0][C1:], M0, C5, hc, torch.empty((B, H * W, C5), dtype=F32, device=dev)) if C5 else None
+            if wgrad:
+                s = colsum(dz, M0, hc, torch.zeros(hc, dtype=F32, device=dev))
+                Es = [gemm_tn(dz, acts[0], M0, hc, Kx, torch.zeros((hc, Kx), dtype=F32, device=dev))]
+            for i in range(1, 4):
                 Hi, Wi = sizes[i]
                 Mi, Ci = B * Hi * Wi, Cs[i]
-                sl = dcat[:, i * hc:]
-                g_b, r_b = gtarget(lb[i])
-                if i == 0:
-                    dtb, lda = sl, K
-                    colsum(sl, Mi, hc, g_b, ld=K)
-                else:
-                    dt = upsample_bwd(sl, B, Hi, Wi, H, W, hc, ld_out=K)
-                    dtb, lda = cast_bf16(dt, Mi, hc), hc
-                    colsum(dt, Mi, hc, g_b)
-                g_w, r_w = gtarget(lw[i], (hc, Ci))
-                gemm_tn(dtb, acts[i], Mi, hc, Ci, g_w, lda=lda)
-                dxi = torch.empty((B, Hi * Wi, Ci), dtype=F32, device=dev)
-                gemm_nt(dtb, prep_weight(lw[i], 1, hc, Ci), Mi, Ci, hc, dxi, lda=lda)
-                gx.append(dxi)
-                rw.append(r_w)
-                rbs.append(r_b)
-            dx5 = None
-            if C5:
-                dx5 = torch.empty((B, H * W, C5), dtype=F32, device=dev)
-                check(lib.mdv_add_f32(ptr(dcat[:, 4 * hc:]), 1, K, ptr(dx5), C5, M0, C5, 0, L.stream()), "mdv_add_f32")
+                dzi = cast_bf16(upsample_bwd(dz, B, Hi, Wi, H, W, hc), Mi, hc)
+                gx.append(gemm_nt(dzi, wts[i], Mi, Ci, hc, torch.empty((B, Hi * Wi, Ci), dtype=F32, device=dev)))
+                if wgrad:
+                    Es.append(gemm_tn(dzi, acts[i], Mi, hc, Ci, torch.zeros((hc, Ci), dtype=F32, device=dev)))
+            if wgrad:
+                probs = []
+                for i in range(4):
+                    Ci, ldE = Cs[i], (Kx if i == 0 else Cs[i])
+                    wf = fw[:, i * hc:]
+                    gwf = g_fw[:, i * hc:] if g_fw is not None else None
+                    probs += [mm(Es[i], lw[i], gwf, hc, hc, Ci, lda=ldE, ldc=K, trans_b=True, accumulate=True, u=s, v=lb[i]),
+                              mm(wf, Es[i], tw[i][0], hc, Ci, hc, lda=K, ldb=ldE, trans_a=True, accumulate=True),
+                              mm(wf, s, tb[i][0], hc, 1, hc, lda=K, trans_a=True, accumulate=True)]
+                matmul_f32(probs)
+                if g_fw is not None and C5:
+                    check(lib.mdv_add_f32(ptr(Es[0][:, C1:]), 0, Kx, ptr(g_fw[:, 4 * hc:]), K, hc, C5, 1, L.stream()), "mdv_add_f32")
+                if g_fb is not None:
+                    check(lib.mdv_add_f32(ptr(s), 0, hc, ptr(g_fb), hc, 1, hc, 1, L.stream()), "mdv_add_f32")
         _grads_done(ctx)
-        return (gx[0], gx[1], gx[2], gx[3], dx5, rw[0], rbs[0], rw[1], rbs[1], rw[2], rbs[2], rw[3], rbs[3], r_fw, r_fb, rg, rb, r_ow,
-                r_ob, None, None, None, None, None, None)
+        return (gx[0], gx[1], gx[2], gx[3], dx5, tw[0][1], tb[0][1], tw[1][1], tb[1][1], tw[2][1], tb[2][1], tw[3][1], tb[3][1], r_fw,
+                r_fb, rg, rb, r_ow, r_ob, None, None, None, None, None, None)
 
 
 # ------------------------------------------------------------------------------------------------- domain split
