@@ -126,6 +126,36 @@ int mdv_layernorm_bwd(const float* dy, const float* x, const float* mean, const 
                       float drop_p, const void* rng, uint32_t drop_stream, float* dgamma, float* dbeta,
                       float* dbias_masked /* [C] += column sums of dx_masked, or NULL */, int M, int C, void* stream);
 
+/* ------------------------------------------------------------------ per-group norm parameter sets (MDViT_DSN / BASE_DSN) */
+/* The stacked multi-domain pass of the domain-specific-norm models runs G single-domain mini-batches as one [G*Mg, C]
+ * tensor; row group g = rows [g*Mg, (g+1)*Mg) uses norm parameter set g.  A table names one tensor per group (p[g], g < G);
+ * it is passed by value, so a captured CUDA graph holds the addresses and no host-to-device copy is needed.  1 <= G <= 8.
+ * Two groups naming the same running buffer or the same gradient target would race: those calls return MDV_ERR_ARG
+ * before any CUDA call. */
+#define MDV_MAX_GROUPS 8
+typedef struct MdvPtrTable {
+    void* p[MDV_MAX_GROUPS];
+} MdvPtrTable;
+
+/* mdv_layernorm_fwd / mdv_layernorm_bwd with gamma[g], beta[g] for row group g.  dgamma[g] / dbeta[g] accumulate (+=) the
+ * sums over group g only and may each be NULL; dbias_masked (a shared bias) is one [C] sum over all rows. */
+int mdv_layernorm_fwd_gp(const float* x, MdvPtrTable gamma, MdvPtrTable beta, float eps, void* y_bf16, float* mean, float* rstd,
+                         int G, int Mg, int C, void* stream);
+int mdv_layernorm_bwd_gp(const float* dy, const float* x, const float* mean, const float* rstd, MdvPtrTable gamma,
+                         const float* dres, float* dx, void* dx_masked_bf16, const float* rowscale, int rows_per_scale,
+                         float drop_p, const void* rng, uint32_t drop_stream, MdvPtrTable dgamma, MdvPtrTable dbeta,
+                         float* dbias_masked, int G, int Mg, int C, void* stream);
+/* mdv_bn_train_fwd_grouped / mdv_bn_act_bwd_grouped with one parameter set per group: group g normalises with gamma[g],
+ * beta[g] and updates only running_mean[g], running_var[g] (momentum, unbiased variance) and *num_batches_tracked[g] += 1,
+ * exactly as nn.BatchNorm2d set g would on its own mini-batch; dgamma[g] / dbeta[g] accumulate group g's sums.  Buffer and
+ * gradient entries may be NULL.  Workspaces as for the grouped forms. */
+int mdv_bn_train_fwd_gp(const float* z, int G, int Mg, int C, float eps, float momentum, MdvPtrTable running_mean,
+                        MdvPtrTable running_var, MdvPtrTable num_batches_tracked, MdvPtrTable gamma, MdvPtrTable beta, int act,
+                        float* mean, float* rstd, void* y, int y_bf16, void* ws, void* stream);
+int mdv_bn_act_bwd_gp(const float* dy, const float* z, const float* mean, const float* rstd, MdvPtrTable gamma, MdvPtrTable beta,
+                      int act, void* dz, int dz_bf16, MdvPtrTable dgamma, MdvPtrTable dbeta, int G, int Mg, int C, void* ws,
+                      void* stream);
+
 /* ------------------------------------------------------------------ BatchNorm2d (+act) on [M=B*H*W, C] (mpvit.py:119-122 ...) */
 /* training: batch mean / biased var -> mean,rstd; running stats updated with momentum (unbiased var) and
  * *num_batches_tracked += 1.  eval: mean,rstd from the running buffers.  ws >= 2*C doubles. */

@@ -24,6 +24,24 @@ class GemmEpi(ctypes.Structure):
     ]
 
 
+MAX_GROUPS = 8      # MDV_MAX_GROUPS
+
+
+class PtrTable(ctypes.Structure):
+    """MdvPtrTable: one device pointer per row group (G <= MAX_GROUPS), passed by value."""
+    _fields_ = [("p", c_void_p * MAX_GROUPS)]
+
+
+def ptr_table(tensors):
+    """PtrTable of the tensors' device pointers (None entries -> NULL)."""
+    if len(tensors) > MAX_GROUPS:
+        raise ValueError(f"at most {MAX_GROUPS} groups")
+    t = PtrTable()
+    for i, x in enumerate(tensors):
+        t.p[i] = None if x is None else x.data_ptr()
+    return t
+
+
 _lib = None
 
 
@@ -100,7 +118,7 @@ def profile_report(top=80, clear=True):
 
 HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "mdvit_b200.h")
 _CTYPES = {"int": c_int, "float": c_float, "double": ctypes.c_double, "long long": ctypes.c_longlong,
-           "uint32_t": c_uint32, "void": None}
+           "uint32_t": c_uint32, "void": None, "MdvPtrTable": PtrTable}
 
 
 def header_signatures(path=HEADER_PATH):

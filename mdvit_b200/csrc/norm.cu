@@ -4,6 +4,8 @@
 #include "../../include/mdvit_b200.h"
 #include "common.cuh"
 
+#include <initializer_list>
+
 namespace {
 
 constexpr int LN_MAXV = 8;  // float2 per lane -> C <= 512
@@ -11,19 +13,26 @@ constexpr int LN_MAXV = 8;  // float2 per lane -> C <= 512
 // ---------------------------------------------------------------------------------- LayerNorm forward
 // one warp owns R rows per iteration (all loads issued before any arithmetic: at C = 64 a row is only 256 B, and one
 // row per warp leaves HBM latency exposed); a row lives in registers, NV float2 per lane.
-template <int NV, int R>
+// GP: per-group parameter sets — blockIdx.y is the row group, M its row count, and gamma/beta come from the tables.
+template <int NV, int R, bool GP>
 __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x, const float* __restrict__ gamma,
                                                       const float* __restrict__ beta, float eps, bf16* __restrict__ y,
-                                                      float* __restrict__ mean_out, float* __restrict__ rstd_out, int M) {
+                                                      float* __restrict__ mean_out, float* __restrict__ rstd_out, int M,
+                                                      const __grid_constant__ MdvPtrTable gtab, const __grid_constant__ MdvPtrTable btab) {
     MDV_PDL_SYNC();
     constexpr int C = NV * 64;
     const int lane = threadIdx.x & 31;
-    const int row0 = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * R;
-    if (row0 >= M) return;
+    const int lo = GP ? blockIdx.y * M : 0, hi = lo + M;
+    if (GP) {
+        gamma = (const float*)gtab.p[blockIdx.y];
+        beta = (const float*)btab.p[blockIdx.y];
+    }
+    const int row0 = lo + (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * R;
+    if (row0 >= hi) return;
     float2 v[R][NV];
 #pragma unroll
     for (int r = 0; r < R; ++r) {
-        const bool ok = row0 + r < M;
+        const bool ok = row0 + r < hi;
         const float* xr = x + (size_t)(ok ? row0 + r : row0) * C;
 #pragma unroll
         for (int i = 0; i < NV; ++i) v[r][i] = *reinterpret_cast<const float2*>(xr + i * 64 + lane * 2);
@@ -37,7 +46,7 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x
 #pragma unroll
     for (int r = 0; r < R; ++r) {
         const int row = row0 + r;
-        if (row >= M) break;
+        if (row >= hi) break;
         float s = 0.f;
 #pragma unroll
         for (int i = 0; i < NV; ++i) s += v[r][i].x + v[r][i].y;
@@ -67,7 +76,9 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x
 // and its column sums (that Linear's bias gradient) are accumulated into dbias_masked.
 // One warp owns R rows per iteration (all of their loads are issued before any arithmetic: with C = 64 a row is only
 // 256 B, so a single row per warp leaves HBM latency exposed); a row lives in registers, NV float2 per lane.
-template <int NV, int R>
+// GP: blockIdx.y is the row group (M rows) and gamma, dgamma, dbeta come from the tables — a block never crosses a group boundary,
+// so its column partials belong to one group's dgamma / dbeta.
+template <int NV, int R, bool GP>
 __global__ void __launch_bounds__(256) ln_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ x,
                                                       const float* __restrict__ mean_in, const float* __restrict__ rstd_in,
                                                       const float* __restrict__ gamma, const float* __restrict__ dres,
@@ -75,11 +86,18 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const float* __restrict__ d
                                                       const float* __restrict__ rowscale, int rows_per_scale, float drop_p,
                                                       const unsigned long long* __restrict__ rng, uint32_t drop_stream,
                                                       float* __restrict__ dgamma, float* __restrict__ dbeta,
-                                                      float* __restrict__ dbias_masked, int M) {
+                                                      float* __restrict__ dbias_masked, int M, const __grid_constant__ MdvPtrTable gtab,
+                                                      const __grid_constant__ MdvPtrTable dgtab, const __grid_constant__ MdvPtrTable dbtab) {
     MDV_PDL_SYNC();
     constexpr int C = NV * 64;
     __shared__ float red[8][64];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
+    const int lo = GP ? blockIdx.y * M : 0, hi = lo + M;
+    if (GP) {
+        gamma = (const float*)gtab.p[blockIdx.y];
+        dgamma = (float*)dgtab.p[blockIdx.y];
+        dbeta = (float*)dbtab.p[blockIdx.y];
+    }
     float2 ag[NV], ab[NV], am[NV], gm[NV];
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
@@ -95,13 +113,13 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const float* __restrict__ d
         dinv = 1.f / (1.f - drop_p);
         dkey = rng_key(rng, drop_stream);
     }
-    for (int row0 = (blockIdx.x * nwarp + warp) * R; row0 < M; row0 += gridDim.x * nwarp * R) {
+    for (int row0 = lo + (blockIdx.x * nwarp + warp) * R; row0 < hi; row0 += gridDim.x * nwarp * R) {
         float2 d[R][NV], xh[R][NV], rr[R][NV];
         float mean[R], rstd[R];
 #pragma unroll
         for (int r = 0; r < R; ++r) {
             const int row = row0 + r;
-            const bool ok = row < M;
+            const bool ok = row < hi;
             const size_t off = (size_t)(ok ? row : 0) * C;
             mean[r] = ok ? mean_in[row] : 0.f;
             rstd[r] = ok ? rstd_in[row] : 0.f;
@@ -116,7 +134,7 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const float* __restrict__ d
 #pragma unroll
         for (int r = 0; r < R; ++r) {
             const int row = row0 + r;
-            if (row >= M) break;
+            if (row >= hi) break;
             const size_t off = (size_t)row * C;
             float s1 = 0.f, s2 = 0.f;
 #pragma unroll
@@ -412,18 +430,23 @@ __global__ void rank1_table_kernel(Rank1Dy r1, float* __restrict__ wtab, int sam
     *reinterpret_cast<float4*>(wtab + i) = rank1_w4(r1, i / C, i % C, C);
 }
 
-template <bool BWD, bool RANK1 = false>
+// GP (all grouped kernels below): group g's gamma / beta are gt.p[g] / bt.p[g] (domain-specific norm sets) instead of one shared pair
+template <bool BWD, bool RANK1 = false, bool GP = false>
 __global__ void __launch_bounds__(256) bn_reduce_g_kernel(const float* __restrict__ a, const float* __restrict__ z,
                                                            const float* __restrict__ mean, const float* __restrict__ rstd,
                                                            const float* __restrict__ gamma, const float* __restrict__ beta, int act,
                                                            double* __restrict__ sums, int Mg, int C, int rows_per_block,
-                                                           Rank1Dy rk = Rank1Dy()) {
+                                                           Rank1Dy rk, const __grid_constant__ MdvPtrTable gt, const __grid_constant__ MdvPtrTable bt) {
     MDV_PDL_SYNC();
     __shared__ float4 sh[2][256];
     const int tpr = C >> 2;                       // threads per row
     const int rpi = 256 / tpr;                    // rows per block iteration
     const int cl = threadIdx.x % tpr, rl = threadIdx.x / tpr;
     const int g = blockIdx.z;
+    if (GP) {
+        gamma = (const float*)gt.p[g];
+        beta = (const float*)bt.p[g];
+    }
     const int r0 = blockIdx.x * rows_per_block, r1 = min(Mg, r0 + rows_per_block);
     const size_t base = (size_t)g * Mg * C;
     float4 s = make_float4(0.f, 0.f, 0.f, 0.f), q = s;
@@ -523,16 +546,20 @@ __global__ void bn_finalize_g_kernel(const double* __restrict__ sums, int G, int
 }
 
 // y = act(gamma (z - mean) rstd + beta): row-walking like the backward apply kernel (parameters once per thread, 4 rows in flight)
-template <typename TO>
+template <typename TO, bool GP = false>
 __global__ void __launch_bounds__(256) bn_act_fwd_g_kernel(const float* __restrict__ z, const float* __restrict__ mean,
                                                             const float* __restrict__ rstd, const float* __restrict__ gamma,
                                                             const float* __restrict__ beta, int act, TO* __restrict__ y, int Mg,
-                                                            int C, int rows_per_block) {
+                                                            int C, int rows_per_block, const __grid_constant__ MdvPtrTable gt, const __grid_constant__ MdvPtrTable bt) {
     MDV_PDL_SYNC();
     const int tpr = C >> 2, rpi = 256 / tpr;
     const int cl = threadIdx.x % tpr, rl = threadIdx.x / tpr;
     if (rl >= rpi) return;
     const int g = blockIdx.z, c = 4 * cl;
+    if (GP) {
+        gamma = (const float*)gt.p[g];
+        beta = (const float*)bt.p[g];
+    }
     const int r0 = blockIdx.x * rows_per_block, r1e = min(Mg, r0 + rows_per_block);
     const size_t base = (size_t)g * Mg * C;
     const float4 mu = *reinterpret_cast<const float4*>(mean + (size_t)g * C + c), rs = *reinterpret_cast<const float4*>(rstd + (size_t)g * C + c);
@@ -578,21 +605,65 @@ __global__ void bn_bwd_finalize_g_kernel(const double* __restrict__ sums, int G,
     if (dgamma) atomicAdd(dgamma + c, (float)sq);
 }
 
+// per-group parameter sets: group g's statistics update only its own running buffers (one nn.BatchNorm2d step each)
+__global__ void bn_finalize_gp_kernel(const double* __restrict__ sums, int G, int Mg, int C, float eps, float momentum, const __grid_constant__ MdvPtrTable rmt,
+                                      const __grid_constant__ MdvPtrTable rvt, const __grid_constant__ MdvPtrTable nbt, float* __restrict__ mean, float* __restrict__ rstd) {
+    MDV_PDL_SYNC();
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c == 0)
+        for (int g = 0; g < G; ++g)
+            if (nbt.p[g]) *(long long*)nbt.p[g] += 1;
+    if (c >= C) return;
+    for (int g = 0; g < G; ++g) {
+        const double mu = sums[(size_t)g * 2 * C + c] / Mg;
+        double var = sums[(size_t)g * 2 * C + C + c] / Mg - mu * mu;
+        if (var < 0) var = 0;
+        mean[(size_t)g * C + c] = (float)mu;
+        rstd[(size_t)g * C + c] = (float)(1.0 / sqrt(var + (double)eps));
+        float* rm = (float*)rmt.p[g];
+        float* rv = (float*)rvt.p[g];
+        if (rm) rm[c] = (1.f - momentum) * rm[c] + momentum * (float)mu;
+        if (rv) {
+            const double unb = Mg > 1 ? var * Mg / (Mg - 1) : var;
+            rv[c] = (1.f - momentum) * rv[c] + momentum * (float)unb;
+        }
+    }
+}
+
+// coef as above; dgamma[g] += group g's sum_gxhat, dbeta[g] += its sum_g
+__global__ void bn_bwd_finalize_gp_kernel(const double* __restrict__ sums, int G, int Mg, int C, float* __restrict__ coef, const __grid_constant__ MdvPtrTable dgt,
+                                          const __grid_constant__ MdvPtrTable dbt) {
+    MDV_PDL_SYNC();
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    for (int g = 0; g < G; ++g) {
+        const double a = sums[(size_t)g * 2 * C + c], b = sums[(size_t)g * 2 * C + C + c];
+        coef[(size_t)g * 2 * C + c] = (float)(a / Mg);
+        coef[(size_t)g * 2 * C + C + c] = (float)(b / Mg);
+        if (dbt.p[g]) atomicAdd((float*)dbt.p[g] + c, (float)a);
+        if (dgt.p[g]) atomicAdd((float*)dgt.p[g] + c, (float)b);
+    }
+}
+
 // dz = gamma rstd (g - c0 - xhat c1), g = dy act'(.).  Same thread mapping as bn_reduce_g_kernel: a thread owns 4 channels and walks
 // the rows of its block's band, 4 rows in flight — the per-channel parameters (7 float4) are loaded once instead of once per 16
 // bytes of z, and there is no index arithmetic per element.
-template <typename TO, bool RANK1 = false>
+template <typename TO, bool RANK1 = false, bool GP = false>
 __global__ void __launch_bounds__(256) bn_bwd_apply_g_kernel(const float* __restrict__ dy, const float* __restrict__ z,
                                                               const float* __restrict__ mean, const float* __restrict__ rstd,
                                                               const float* __restrict__ gamma, const float* __restrict__ beta, int act,
                                                               const float* __restrict__ coef, TO* __restrict__ dz, int Mg, int C,
-                                                              int rows_per_block, Rank1Dy r1 = Rank1Dy()) {
+                                                              int rows_per_block, Rank1Dy r1, const __grid_constant__ MdvPtrTable gt, const __grid_constant__ MdvPtrTable bt) {
     MDV_PDL_SYNC();
     const int tpr = C >> 2;                       // threads per row
     const int rpi = 256 / tpr;                    // rows per block iteration
     const int cl = threadIdx.x % tpr, rl = threadIdx.x / tpr;
     if (rl >= rpi) return;
     const int g = blockIdx.z;
+    if (GP) {
+        gamma = (const float*)gt.p[g];
+        beta = (const float*)bt.p[g];
+    }
     const int r0 = blockIdx.x * rows_per_block, r1e = min(Mg, r0 + rows_per_block);
     const size_t base = (size_t)g * Mg * C;
     const int c = 4 * cl;
@@ -679,56 +750,117 @@ int stats_rows_per_block(int M, int C) {
 
 }  // namespace
 
-extern "C" int mdv_layernorm_fwd(const float* x, const float* gamma, const float* beta, float eps, void* y_bf16, float* mean,
-                                 float* rstd, int M, int C, void* stream) {
-    if (!x || !y_bf16 || !gamma || !beta || M <= 0 || (C & 63) || C > 64 * LN_MAXV) return MDV_ERR_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-#define MDV_LN_FWD(NV, R) mdv_launch((ln_fwd_kernel<NV, R>), dim3(mdv_cdiv(M, 8 * R)), dim3(256), 0, st, x, gamma, beta, eps, (bf16*)y_bf16, mean, rstd, M); break;
-    switch (C >> 6) {
-        case 1: MDV_LN_FWD(1, 4)
-        case 2: MDV_LN_FWD(2, 4)
-        case 3: MDV_LN_FWD(3, 2)
-        case 4: MDV_LN_FWD(4, 2)
-        case 5: MDV_LN_FWD(5, 2)
-        case 6: MDV_LN_FWD(6, 1)
-        case 7: MDV_LN_FWD(7, 1)
-        default: MDV_LN_FWD(8, 1)
+// Rows per warp iteration by width: C = 64 * NV.
+#define MDV_LN_DISPATCH(X)      \
+    switch (C >> 6) {           \
+        case 1: X(1, 4)         \
+        case 2: X(2, 4)         \
+        case 3: X(3, 2)         \
+        case 4: X(4, 2)         \
+        case 5: X(5, 2)         \
+        case 6: X(6, 1)         \
+        case 7: X(7, 1)         \
+        default: X(8, 1)        \
     }
+
+static int ln_fwd_launch(bool gp, const float* x, const float* gamma, const float* beta, MdvPtrTable gt, MdvPtrTable bt, float eps,
+                         void* y_bf16, float* mean, float* rstd, int G, int Mg, int C, cudaStream_t st) {
+#define MDV_LN_FWD(NV, R)                                                                                                        \
+    if (gp)                                                                                                                      \
+        mdv_launch((ln_fwd_kernel<NV, R, true>), dim3(mdv_cdiv(Mg, 8 * R), G), dim3(256), 0, st, x, gamma, beta, eps,           \
+                   (bf16*)y_bf16, mean, rstd, Mg, gt, bt);                                                                       \
+    else                                                                                                                         \
+        mdv_launch((ln_fwd_kernel<NV, R, false>), dim3(mdv_cdiv(Mg, 8 * R)), dim3(256), 0, st, x, gamma, beta, eps,             \
+                   (bf16*)y_bf16, mean, rstd, Mg, gt, bt);                                                                       \
+    break;
+    MDV_LN_DISPATCH(MDV_LN_FWD)
 #undef MDV_LN_FWD
     MDV_CHECK_LAUNCH();
     return MDV_OK;
+}
+
+static int ln_bwd_launch(bool gp, const float* dy, const float* x, const float* mean, const float* rstd, const float* gamma, MdvPtrTable gt,
+                         const float* dres, float* dx, void* dx_masked_bf16, const float* rowscale, int rows_per_scale, float drop_p,
+                         const void* rng, uint32_t drop_stream, float* dgamma, float* dbeta, MdvPtrTable dgt, MdvPtrTable dbt,
+                         float* dbias_masked, int G, int Mg, int C, cudaStream_t st) {
+    const int rps = rows_per_scale > 0 ? rows_per_scale : 1;
+    const int max_blocks = (4 * MDV_NUM_SMS + G - 1) / G;      // ~4 blocks per SM over all groups
+#define MDV_LN_BWD(NV, R)                                                                                                        \
+    {                                                                                                                            \
+        int blocks = mdv_cdiv(Mg, 8 * R);                                                                                        \
+        if (blocks > max_blocks) blocks = max_blocks;                                                                            \
+        if (gp)                                                                                                                  \
+            mdv_launch((ln_bwd_kernel<NV, R, true>), dim3(blocks, G), dim3(256), 0, st, dy, x, mean, rstd, gamma, dres, dx,     \
+                       (bf16*)dx_masked_bf16, rowscale, rps, drop_p, (const unsigned long long*)rng, drop_stream, dgamma, dbeta, \
+                       dbias_masked, Mg, gt, dgt, dbt);                                                                          \
+        else                                                                                                                     \
+            mdv_launch((ln_bwd_kernel<NV, R, false>), dim3(blocks), dim3(256), 0, st, dy, x, mean, rstd, gamma, dres, dx,       \
+                       (bf16*)dx_masked_bf16, rowscale, rps, drop_p, (const unsigned long long*)rng, drop_stream, dgamma, dbeta, \
+                       dbias_masked, Mg, gt, dgt, dbt);                                                                          \
+    }                                                                                                                            \
+    break;
+    MDV_LN_DISPATCH(MDV_LN_BWD)
+#undef MDV_LN_BWD
+    MDV_CHECK_LAUNCH();
+    return MDV_OK;
+}
+
+// Non-NULL entries p[0..G) of the given tables must be pairwise distinct (two groups writing one buffer would race).
+static bool tables_distinct(int G, std::initializer_list<const MdvPtrTable*> tabs) {
+    const void* seen[5 * MDV_MAX_GROUPS];
+    int n = 0;
+    for (const MdvPtrTable* t : tabs)
+        for (int g = 0; g < G; ++g) {
+            const void* q = t->p[g];
+            if (!q) continue;
+            for (int i = 0; i < n; ++i)
+                if (seen[i] == q) return false;
+            seen[n++] = q;
+        }
+    return true;
+}
+
+static bool tables_set(int G, std::initializer_list<const MdvPtrTable*> tabs) {
+    for (const MdvPtrTable* t : tabs)
+        for (int g = 0; g < G; ++g)
+            if (!t->p[g]) return false;
+    return true;
+}
+
+static bool ln_shape_ok(int M, int C) { return M > 0 && !(C & 63) && C <= 64 * LN_MAXV; }
+
+extern "C" int mdv_layernorm_fwd(const float* x, const float* gamma, const float* beta, float eps, void* y_bf16, float* mean,
+                                 float* rstd, int M, int C, void* stream) {
+    if (!x || !y_bf16 || !gamma || !beta || !ln_shape_ok(M, C)) return MDV_ERR_ARG;
+    return ln_fwd_launch(false, x, gamma, beta, MdvPtrTable(), MdvPtrTable(), eps, y_bf16, mean, rstd, 1, M, C, (cudaStream_t)stream);
+}
+
+extern "C" int mdv_layernorm_fwd_gp(const float* x, MdvPtrTable gamma, MdvPtrTable beta, float eps, void* y_bf16, float* mean, float* rstd,
+                                    int G, int Mg, int C, void* stream) {
+    if (G < 1 || G > MDV_MAX_GROUPS || !x || !y_bf16 || !mean || !rstd || !ln_shape_ok(Mg, C)) return MDV_ERR_ARG;
+    if (!tables_set(G, {&gamma, &beta}) || (long long)G * Mg >= 0x7fffffffLL) return MDV_ERR_ARG;
+    return ln_fwd_launch(true, x, nullptr, nullptr, gamma, beta, eps, y_bf16, mean, rstd, G, Mg, C, (cudaStream_t)stream);
 }
 
 extern "C" int mdv_layernorm_bwd(const float* dy, const float* x, const float* mean, const float* rstd, const float* gamma,
                                  const float* dres, float* dx, void* dx_masked_bf16, const float* rowscale,
                                  int rows_per_scale, float drop_p, const void* rng, uint32_t drop_stream, float* dgamma,
                                  float* dbeta, float* dbias_masked, int M, int C, void* stream) {
-    if (!dy || !x || !dx || !gamma || M <= 0 || (C & 63) || C > 64 * LN_MAXV) return MDV_ERR_ARG;
+    if (!dy || !x || !dx || !gamma || !ln_shape_ok(M, C)) return MDV_ERR_ARG;
     if (dbias_masked && !dx_masked_bf16) return MDV_ERR_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int rps = rows_per_scale > 0 ? rows_per_scale : 1;
-#define MDV_LN_BWD(NV, R)                                                                                                        \
-    {                                                                                                                            \
-        int blocks = mdv_cdiv(M, 8 * R);                                                                                         \
-        if (blocks > 4 * MDV_NUM_SMS) blocks = 4 * MDV_NUM_SMS;                                                                  \
-        mdv_launch((ln_bwd_kernel<NV, R>), dim3(blocks), dim3(256), 0, st, dy, x, mean, rstd, gamma, dres, dx, (bf16*)dx_masked_bf16, rowscale, rps,   \
-                                                     drop_p, (const unsigned long long*)rng, drop_stream, dgamma, dbeta,         \
-                                                     dbias_masked, M);                                                           \
-    }                                                                                                                            \
-    break;
-    switch (C >> 6) {
-        case 1: MDV_LN_BWD(1, 4)
-        case 2: MDV_LN_BWD(2, 4)
-        case 3: MDV_LN_BWD(3, 2)
-        case 4: MDV_LN_BWD(4, 2)
-        case 5: MDV_LN_BWD(5, 2)
-        case 6: MDV_LN_BWD(6, 1)
-        case 7: MDV_LN_BWD(7, 1)
-        default: MDV_LN_BWD(8, 1)
-    }
-#undef MDV_LN_BWD
-    MDV_CHECK_LAUNCH();
-    return MDV_OK;
+    return ln_bwd_launch(false, dy, x, mean, rstd, gamma, MdvPtrTable(), dres, dx, dx_masked_bf16, rowscale, rows_per_scale, drop_p, rng,
+                         drop_stream, dgamma, dbeta, MdvPtrTable(), MdvPtrTable(), dbias_masked, 1, M, C, (cudaStream_t)stream);
+}
+
+extern "C" int mdv_layernorm_bwd_gp(const float* dy, const float* x, const float* mean, const float* rstd, MdvPtrTable gamma,
+                                    const float* dres, float* dx, void* dx_masked_bf16, const float* rowscale, int rows_per_scale,
+                                    float drop_p, const void* rng, uint32_t drop_stream, MdvPtrTable dgamma, MdvPtrTable dbeta,
+                                    float* dbias_masked, int G, int Mg, int C, void* stream) {
+    if (G < 1 || G > MDV_MAX_GROUPS || !dy || !x || !mean || !rstd || !dx || !ln_shape_ok(Mg, C)) return MDV_ERR_ARG;
+    if (dbias_masked && !dx_masked_bf16) return MDV_ERR_ARG;
+    if (!tables_set(G, {&gamma}) || !tables_distinct(G, {&dgamma, &dbeta}) || (long long)G * Mg >= 0x7fffffffLL) return MDV_ERR_ARG;
+    return ln_bwd_launch(true, dy, x, mean, rstd, nullptr, gamma, dres, dx, dx_masked_bf16, rowscale, rows_per_scale, drop_p, rng,
+                         drop_stream, nullptr, nullptr, dgamma, dbeta, dbias_masked, G, Mg, C, (cudaStream_t)stream);
 }
 
 // ws: >= 2*C doubles (zeroed here).  Writes mean[C], rstd[C]; in training also updates the running buffers.
@@ -832,17 +964,17 @@ static int bn_act_bwd_impl(const float* dy, const Rank1Dy& r1, const float* z, c
         MDV_CHECK_LAUNCH();
         const int rpb = grouped_rows_per_block(M, C, 1);
         mdv_launch((bn_reduce_g_kernel<true, true>), dim3(mdv_cdiv(M, rpb), 1, 1), dim3(256), 0, st, (const float*)nullptr, z, mean, rstd, gamma, beta, act,
-                   sums, M, C, rpb, rt);
+                   sums, M, C, rpb, rt, MdvPtrTable(), MdvPtrTable());
         MDV_CHECK_LAUNCH();
         mdv_launch(bn_bwd_finalize_g_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)sums, 1, M, C, coef, dgamma, dbeta);
         MDV_CHECK_LAUNCH();
         const int rpa = apply_rows_per_block(M, C, 1);
         if (dz_bf16)
             mdv_launch((bn_bwd_apply_g_kernel<bf16, true>), dim3(mdv_cdiv(M, rpa), 1, 1), dim3(256), 0, st, (const float*)nullptr, z, mean, rstd, gamma, beta,
-                       act, (const float*)coef, (bf16*)dz, M, C, rpa, rt);
+                       act, (const float*)coef, (bf16*)dz, M, C, rpa, rt, MdvPtrTable(), MdvPtrTable());
         else
             mdv_launch((bn_bwd_apply_g_kernel<float, true>), dim3(mdv_cdiv(M, rpa), 1, 1), dim3(256), 0, st, (const float*)nullptr, z, mean, rstd, gamma, beta,
-                       act, (const float*)coef, (float*)dz, M, C, rpa, rt);
+                       act, (const float*)coef, (float*)dz, M, C, rpa, rt, MdvPtrTable(), MdvPtrTable());
         MDV_CHECK_LAUNCH();
         return MDV_OK;
     }
@@ -870,30 +1002,97 @@ static int bn_act_bwd_impl(const float* dy, const Rank1Dy& r1, const float* z, c
 // ---- grouped train-mode BatchNorm (+activation): one call = G consecutive nn.BatchNorm2d forwards on [G*Mg, C]
 static bool bn_grouped_ok(int G, int Mg, int C) { return G >= 1 && Mg >= 1 && C >= 32 && C <= 1024 && (C & 3) == 0 && (long long)G * Mg * C < 0x7fffffffLL; }
 
+// gp: per-group parameter sets (gamma/beta and the running buffers come from the tables, finalize updates group g's own buffers)
+static int bn_train_fwd_g_impl(bool gp, const float* z, int G, int Mg, int C, float eps, float momentum, float* running_mean,
+                               float* running_var, long long* num_batches_tracked, const float* gamma, const float* beta, MdvPtrTable rmt,
+                               MdvPtrTable rvt, MdvPtrTable nbt, MdvPtrTable gt, MdvPtrTable bt, int act, float* mean, float* rstd, void* y,
+                               int y_bf16, void* ws, cudaStream_t st) {
+    cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C * G, st);
+    if (e != cudaSuccess) return (int)e;
+    const int rpb = grouped_rows_per_block(Mg, C, G);
+    mdv_launch(bn_reduce_g_kernel<false>, dim3(mdv_cdiv(Mg, rpb), 1, G), dim3(256), 0, st, (const float*)nullptr, z, (const float*)nullptr,
+               (const float*)nullptr, (const float*)nullptr, (const float*)nullptr, 0, (double*)ws, Mg, C, rpb, Rank1Dy(), MdvPtrTable(),
+               MdvPtrTable());
+    MDV_CHECK_LAUNCH();
+    if (gp)
+        mdv_launch(bn_finalize_gp_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)ws, G, Mg, C, eps, momentum, rmt, rvt, nbt,
+                   mean, rstd);
+    else
+        mdv_launch(bn_finalize_g_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)ws, G, Mg, C, eps, momentum, running_mean,
+                   running_var, num_batches_tracked, mean, rstd);
+    MDV_CHECK_LAUNCH();
+    const int rpa = apply_rows_per_block(Mg, C, G);
+    const dim3 grid(mdv_cdiv(Mg, rpa), 1, G);
+    if (y_bf16 && gp)
+        mdv_launch(bn_act_fwd_g_kernel<bf16, true>, grid, dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, gamma, beta, act, (bf16*)y, Mg, C,
+                   rpa, gt, bt);
+    else if (y_bf16)
+        mdv_launch(bn_act_fwd_g_kernel<bf16>, grid, dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, gamma, beta, act, (bf16*)y, Mg, C, rpa,
+                   gt, bt);
+    else if (gp)
+        mdv_launch(bn_act_fwd_g_kernel<float, true>, grid, dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, gamma, beta, act, (float*)y, Mg,
+                   C, rpa, gt, bt);
+    else
+        mdv_launch(bn_act_fwd_g_kernel<float>, grid, dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, gamma, beta, act, (float*)y, Mg, C,
+                   rpa, gt, bt);
+    MDV_CHECK_LAUNCH();
+    return MDV_OK;
+}
+
 extern "C" int mdv_bn_train_fwd_grouped(const float* z, int G, int Mg, int C, float eps, float momentum, float* running_mean,
                                         float* running_var, long long* num_batches_tracked, const float* gamma, const float* beta, int act,
                                         float* mean, float* rstd, void* y, int y_bf16, void* ws, void* stream) {
     if (!z || !gamma || !beta || !mean || !rstd || !y || !ws) return MDV_ERR_ARG;
     if (!bn_grouped_ok(G, Mg, C)) return MDV_ERR_UNSUPPORTED;
-    cudaStream_t st = (cudaStream_t)stream;
+    const MdvPtrTable none = MdvPtrTable();
+    return bn_train_fwd_g_impl(false, z, G, Mg, C, eps, momentum, running_mean, running_var, num_batches_tracked, gamma, beta, none, none, none,
+                               none, none, act, mean, rstd, y, y_bf16, ws, (cudaStream_t)stream);
+}
+
+extern "C" int mdv_bn_train_fwd_gp(const float* z, int G, int Mg, int C, float eps, float momentum, MdvPtrTable running_mean,
+                                   MdvPtrTable running_var, MdvPtrTable num_batches_tracked, MdvPtrTable gamma, MdvPtrTable beta, int act,
+                                   float* mean, float* rstd, void* y, int y_bf16, void* ws, void* stream) {
+    if (G < 1 || G > MDV_MAX_GROUPS || !z || !mean || !rstd || !y || !ws || !tables_set(G, {&gamma, &beta})) return MDV_ERR_ARG;
+    if (!tables_distinct(G, {&running_mean, &running_var, &num_batches_tracked})) return MDV_ERR_ARG;
+    if (!bn_grouped_ok(G, Mg, C)) return MDV_ERR_UNSUPPORTED;
+    return bn_train_fwd_g_impl(true, z, G, Mg, C, eps, momentum, nullptr, nullptr, nullptr, nullptr, nullptr, running_mean, running_var,
+                               num_batches_tracked, gamma, beta, act, mean, rstd, y, y_bf16, ws, (cudaStream_t)stream);
+}
+
+static int bn_act_bwd_g_impl(bool gp, const float* dy, const float* z, const float* mean, const float* rstd, const float* gamma, const float* beta,
+                             MdvPtrTable gt, MdvPtrTable bt, int act, void* dz, int dz_bf16, float* dgamma, float* dbeta, MdvPtrTable dgt,
+                             MdvPtrTable dbt, int G, int Mg, int C, void* ws, cudaStream_t st) {
+    double* sums = (double*)ws;
+    float* coef = (float*)(sums + (size_t)2 * C * G);
     cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C * G, st);
     if (e != cudaSuccess) return (int)e;
     const int rpb = grouped_rows_per_block(Mg, C, G);
-    mdv_launch(bn_reduce_g_kernel<false>, dim3(mdv_cdiv(Mg, rpb), 1, G), dim3(256), 0, st, (const float*)nullptr, z, (const float*)nullptr,
-               (const float*)nullptr, (const float*)nullptr, (const float*)nullptr, 0, (double*)ws, Mg, C, rpb, Rank1Dy());
-    MDV_CHECK_LAUNCH();
-    mdv_launch(bn_finalize_g_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)ws, G, Mg, C, eps, momentum, running_mean, running_var,
-               num_batches_tracked, mean, rstd);
-    MDV_CHECK_LAUNCH();
-    const int total = G * Mg * C;
-    const int blocks = mdv_cdiv(total / 4, 256);
-    const int rpa = apply_rows_per_block(Mg, C, G);
-    if (y_bf16)
-        mdv_launch(bn_act_fwd_g_kernel<bf16>, dim3(mdv_cdiv(Mg, rpa), 1, G), dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, gamma, beta, act,
-                   (bf16*)y, Mg, C, rpa);
+    const dim3 rgrid(mdv_cdiv(Mg, rpb), 1, G);
+    if (gp)
+        mdv_launch(bn_reduce_g_kernel<true, false, true>, rgrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, sums, Mg, C, rpb, Rank1Dy(),
+                   gt, bt);
     else
-        mdv_launch(bn_act_fwd_g_kernel<float>, dim3(mdv_cdiv(Mg, rpa), 1, G), dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, gamma, beta, act,
-                   (float*)y, Mg, C, rpa);
+        mdv_launch(bn_reduce_g_kernel<true>, rgrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, sums, Mg, C, rpb, Rank1Dy(), gt, bt);
+    MDV_CHECK_LAUNCH();
+    if (gp)
+        mdv_launch(bn_bwd_finalize_gp_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)sums, G, Mg, C, coef, dgt, dbt);
+    else
+        mdv_launch(bn_bwd_finalize_g_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)sums, G, Mg, C, coef, dgamma, dbeta);
+    MDV_CHECK_LAUNCH();
+    const int rpa = apply_rows_per_block(Mg, C, G);
+    const dim3 agrid(mdv_cdiv(Mg, rpa), 1, G);
+    if (dz_bf16 && gp)
+        mdv_launch(bn_bwd_apply_g_kernel<bf16, false, true>, agrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, (const float*)coef,
+                   (bf16*)dz, Mg, C, rpa, Rank1Dy(), gt, bt);
+    else if (dz_bf16)
+        mdv_launch(bn_bwd_apply_g_kernel<bf16>, agrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, (const float*)coef, (bf16*)dz, Mg, C,
+                   rpa, Rank1Dy(), gt, bt);
+    else if (gp)
+        mdv_launch(bn_bwd_apply_g_kernel<float, false, true>, agrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, (const float*)coef,
+                   (float*)dz, Mg, C, rpa, Rank1Dy(), gt, bt);
+    else
+        mdv_launch(bn_bwd_apply_g_kernel<float>, agrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, (const float*)coef, (float*)dz, Mg, C,
+                   rpa, Rank1Dy(), gt, bt);
     MDV_CHECK_LAUNCH();
     return MDV_OK;
 }
@@ -903,23 +1102,17 @@ extern "C" int mdv_bn_act_bwd_grouped(const float* dy, const float* z, const flo
                                       void* ws, void* stream) {
     if (!dy || !z || !mean || !rstd || !gamma || !beta || !dz || !ws) return MDV_ERR_ARG;
     if (!bn_grouped_ok(G, Mg, C)) return MDV_ERR_UNSUPPORTED;
-    cudaStream_t st = (cudaStream_t)stream;
-    double* sums = (double*)ws;
-    float* coef = (float*)(sums + (size_t)2 * C * G);
-    cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C * G, st);
-    if (e != cudaSuccess) return (int)e;
-    const int rpb = grouped_rows_per_block(Mg, C, G);
-    mdv_launch(bn_reduce_g_kernel<true>, dim3(mdv_cdiv(Mg, rpb), 1, G), dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, sums, Mg, C, rpb, Rank1Dy());
-    MDV_CHECK_LAUNCH();
-    mdv_launch(bn_bwd_finalize_g_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)sums, G, Mg, C, coef, dgamma, dbeta);
-    MDV_CHECK_LAUNCH();
-    const int rpa = apply_rows_per_block(Mg, C, G);
-    if (dz_bf16)
-        mdv_launch(bn_bwd_apply_g_kernel<bf16>, dim3(mdv_cdiv(Mg, rpa), 1, G), dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, (const float*)coef,
-                   (bf16*)dz, Mg, C, rpa, Rank1Dy());
-    else
-        mdv_launch(bn_bwd_apply_g_kernel<float>, dim3(mdv_cdiv(Mg, rpa), 1, G), dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, (const float*)coef,
-                   (float*)dz, Mg, C, rpa, Rank1Dy());
-    MDV_CHECK_LAUNCH();
-    return MDV_OK;
+    const MdvPtrTable none = MdvPtrTable();
+    return bn_act_bwd_g_impl(false, dy, z, mean, rstd, gamma, beta, none, none, act, dz, dz_bf16, dgamma, dbeta, none, none, G, Mg, C, ws,
+                             (cudaStream_t)stream);
+}
+
+extern "C" int mdv_bn_act_bwd_gp(const float* dy, const float* z, const float* mean, const float* rstd, MdvPtrTable gamma, MdvPtrTable beta,
+                                 int act, void* dz, int dz_bf16, MdvPtrTable dgamma, MdvPtrTable dbeta, int G, int Mg, int C, void* ws,
+                                 void* stream) {
+    if (G < 1 || G > MDV_MAX_GROUPS || !dy || !z || !mean || !rstd || !dz || !ws || !tables_set(G, {&gamma, &beta})) return MDV_ERR_ARG;
+    if (!tables_distinct(G, {&dgamma, &dbeta})) return MDV_ERR_ARG;
+    if (!bn_grouped_ok(G, Mg, C)) return MDV_ERR_UNSUPPORTED;
+    return bn_act_bwd_g_impl(true, dy, z, mean, rstd, nullptr, nullptr, gamma, beta, act, dz, dz_bf16, nullptr, nullptr, dgamma, dbeta, G, Mg, C,
+                             ws, (cudaStream_t)stream);
 }

@@ -26,6 +26,21 @@ def _ctor_draw(*convs):
         c.weight.data.normal_(0, math.sqrt(2.0 / fan_out))
 
 
+def _pick(mods, d):
+    """The norm of domain d; for the stacked multi-domain pass (d = the G domain keys) the list of the G domains' norms."""
+    return [mods[int(k)] for k in d] if isinstance(d, (list, tuple)) else mods[int(d)]
+
+
+def _norm_args(*norms):
+    """The norm arguments of an ops Function (see ops._bn_set).  Each of `norms` is one BatchNorm2d, or the list of the G sets the
+    row groups of a stacked pass use.  Returns group 0's (weight, bias) pairs, every group's running buffers group by group, and
+    groups 1..G-1's (weight, bias) pairs group by group (the Function's trailing arguments)."""
+    sets = [n if isinstance(n, list) else [n] for n in norms]
+    gb = [[t for s in sets for t in (s[g].weight, s[g].bias)] for g in range(len(sets[0]))]
+    bufs = tuple(t for g in range(len(gb)) for s in sets for t in (s[g].running_mean, s[g].running_var, s[g].num_batches_tracked))
+    return gb[0], bufs, tuple(t for pairs in gb[1:] for t in pairs)
+
+
 # ----------------------------------------------------------------------------------------------- parameter containers
 class Conv2d_BN(nn.Module):
     """mpvit.py:81-124 (conv no bias + BN + act)."""
@@ -52,7 +67,7 @@ class Conv2d_BN_M(nn.Module):
         self.act_layer = act_layer() if act_layer is not None else nn.Identity()
 
     def norm(self, d=None):
-        return self.bns[int(d)]
+        return _pick(self.bns, d)
 
 
 class DWConv2d_BN(nn.Module):
@@ -71,7 +86,7 @@ class DWConv2d_BN(nn.Module):
         _ctor_draw(self.dwconv, self.pwconv)
 
     def norm(self, d=None):
-        return self.bn if hasattr(self, "bn") else self.bns[int(d)]
+        return self.bn if hasattr(self, "bn") else _pick(self.bns, d)
 
 
 class DWCPatchEmbed(nn.Module):
@@ -83,10 +98,8 @@ class DWCPatchEmbed(nn.Module):
 
     def forward(self, x, H, W, after_stem=False, d=None):
         pc = self.patch_conv
-        bn = pc.norm(d)
-        y = ops.PatchEmbedFn.apply(x, pc.dwconv.weight, pc.pwconv.weight, bn.weight, bn.bias,
-                                   (bn.running_mean, bn.running_var, bn.num_batches_tracked), H, W, pc.stride,
-                                   self.training, after_stem)
+        (g, b), bufs, gp = _norm_args(pc.norm(d))
+        y = ops.PatchEmbedFn.apply(x, pc.dwconv.weight, pc.pwconv.weight, g, b, bufs, H, W, pc.stride, self.training, after_stem, *gp)
         s = pc.stride
         return y, (H + 2 - 3) // s + 1, (W + 2 - 3) // s + 1
 
@@ -106,7 +119,7 @@ class DecoderDWConv2d_BN(nn.Module):
         _ctor_draw(self.dwconv, self.pwconv)
 
     def norm(self, d=None):
-        return self.bn if hasattr(self, "bn") else self.bns[int(d)]
+        return self.bn if hasattr(self, "bn") else _pick(self.bns, d)
 
 
 class ConvPosEnc(nn.Module):
@@ -202,8 +215,12 @@ class SerialBlock_adapt(nn.Module):
 
     def forward(self, x, size, domain_label=None, d=None):
         H, W = size
-        norm1 = self.norm1s[int(d)] if self.dsn else self.norm1
-        norm2 = self.norm2s[int(d)] if self.dsn else self.norm2
+        norm1 = _pick(self.norm1s, d) if self.dsn else self.norm1
+        norm2 = _pick(self.norm2s, d) if self.dsn else self.norm2
+        # one LayerNorm pair, or (stacked pass) the G per-domain pairs: groups 1..G-1 go to BlockFn as trailing arguments
+        n1, n2 = (norm1, norm2) if isinstance(norm1, list) else ([norm1], [norm2])
+        gp = tuple(t for a, b in zip(n1[1:], n2[1:]) for t in (a.weight, a.bias, b.weight, b.bias))
+        norm1, norm2 = n1[0], n2[0]
         att = self.factoratt_crpe
         # dispatch quirks of mdvit.py:350-353 preserved: Sup attention needs a label, plain attention rejects one
         use_label = domain_label is not None and (self.label_only_guard or self.adapt_method is not None)
@@ -222,7 +239,7 @@ class SerialBlock_adapt(nn.Module):
             norm1.weight, norm1.bias, att.qkv.weight, att.qkv.bias, att.proj.weight, att.proj.bias,
             da[0], da[1], da[2], da[3], norm2.weight, norm2.bias,
             self.mlp.fc1.weight, self.mlp.fc1.bias, self.mlp.fc2.weight, self.mlp.fc2.bias,
-            H, W, self.drop_rate, self.drop_path_rate, self.training)
+            H, W, self.drop_rate, self.drop_path_rate, self.training, *gp)
 
 
 class MHSA_stage_adapt(nn.Module):
@@ -254,10 +271,9 @@ class UnetDecodingBlockTransformer(nn.Module):
 
     def forward(self, x, h, w, skip, H, W, domain_label=None, d=None):
         ca = self.conv_after
-        bn = ca.norm(d)
+        (g, b), bufs, gp = _norm_args(ca.norm(d))
         out = ops.DecoderConvFn.apply(x, skip, self.conv_before.weight, self.conv_before.bias, ca.dwconv.weight, ca.pwconv.weight,
-                                      bn.weight, bn.bias, (bn.running_mean, bn.running_var, bn.num_batches_tracked),
-                                      h, w, H, W, self.training)
+                                      g, b, bufs, h, w, H, W, self.training, *gp)
         return self.mhsa_block(out, H, W, domain_label, d)
 
 
@@ -428,9 +444,8 @@ class _Trunk(nn.Module):
             raise RuntimeError("mdvit_b200 runs on CUDA (sm_100a) only; there is no CPU path")
         c0, n0, c1, n1 = self._stem_parts(d)
         H, W = x.shape[2] // 4, x.shape[3] // 4
-        t = ops.StemFn.apply(x, c0.weight, n0.weight, n0.bias, c1.weight, n1.weight, n1.bias,
-                             (n0.running_mean, n0.running_var, n0.num_batches_tracked,
-                              n1.running_mean, n1.running_var, n1.num_batches_tracked), self.training)
+        (g0, b0, g1, b1), bufs, gp = _norm_args(n0, n1)
+        t = ops.StemFn.apply(x, c0.weight, g0, b0, c1.weight, g1, b1, bufs, self.training, *gp)
         enc = []
         for idx in range(self.num_stages):
             t, H, W = self.patch_embed_stages[idx](t, H, W, after_stem=(idx == 0), d=d)
@@ -441,9 +456,8 @@ class _Trunk(nn.Module):
     def _bridge(self, enc, d=None):
         t3, H3, W3 = enc[3]
         c0, n0, c1, n1 = self._bridge_parts(d)
-        return ops.BridgeFn.apply(t3, c0.weight, c0.bias, n0.weight, n0.bias, c1.weight, c1.bias, n1.weight, n1.bias,
-                                  (n0.running_mean, n0.running_var, n0.num_batches_tracked,
-                                   n1.running_mean, n1.running_var, n1.num_batches_tracked), H3, W3, self.training)
+        (g0, b0, g1, b1), bufs, gp = _norm_args(n0, n1)
+        return ops.BridgeFn.apply(t3, c0.weight, c0.bias, g0, b0, c1.weight, c1.bias, g1, b1, bufs, H3, W3, self.training, *gp)
 
     def _decode_from(self, out, enc, decoders, domain_label, d=None):
         h, w = enc[3][1], enc[3][2]
@@ -569,8 +583,11 @@ class MDViT_DSN(_Trunk):
     """Drop-in for Models.Transformer.mdvit.MDViT_DSN (mdvit.py:735-960): MDViT with DOMAIN-SPECIFIC NORMS — every
     BatchNorm (stem, patch embeddings, bridge, decoder convs) and every LayerNorm (norm1s / norm2s of each block) exists
     once per domain and forward(x, domain_label, d) uses the set `int(d)`.  The kernels are the same: the autograd
-    Functions take the norm parameters as arguments, so domain selection is a pointer choice on the host.
+    Functions take the norm parameters as arguments, so domain selection is a pointer choice on the host.  In the stacked
+    training pass (forward_multi) the choice moves to the device: the norm kernels take one parameter set per row group.
     decoder_name='MLPFM' is the implemented auxiliary decoder (the reference class defaults to 'MLP')."""
+
+    domain_specific_norms = True      # forward needs the domain key d even without auxiliary branches (MKDTrainer passes it)
 
     def __init__(self, img_size=512, in_chans=3, num_stages=4, num_layers=[2, 2, 2, 2], embed_dims=[64, 128, 320, 512],
                  mlp_ratios=[8, 8, 4, 4], num_heads=[8, 8, 8, 8], qkv_bias=True, qk_scale=None, drop_rate=0., attn_drop_rate=0.,
@@ -617,8 +634,47 @@ class MDViT_DSN(_Trunk):
     def _stem_parts(self, d=None):
         return self.stem_1.conv, self.stem_1.norm(d), self.stem_2.conv, self.stem_2.norm(d)
 
+    def forward_multi(self, x, domain_label, domains):
+        """The G single-domain forwards of one training step as ONE pass over the stacked batch (see MDViT.forward_multi):
+        x = cat of G equal mini-batches, domain_label the matching rows (or None), domains the G distinct domain keys in stacking
+        order.  Row group g is normalised with norm set int(domains[g]) in every BatchNorm (stem, patch embeddings, bridge,
+        decoder convs) and LayerNorm (norm1s / norm2s): one kernel launch serves all groups, each group's statistics and
+        running buffers are its own, and each set's gradients come from its group only.  The auxiliary decoders run per slice.
+        Returns [(out_d, aux_d)] per domain (aux_d None for BASE_DSN); equivalent to the G separate forwards up to dropout masks.
+        In eval mode it returns the G separate forwards: folding one BatchNorm set per row group into the GEMM epilogues (the
+        single-domain eval path) is not implemented."""
+        G = len(domains)
+        domains = [str(d) for d in domains]
+        if len(set(domains)) != G:
+            raise ValueError(f"forward_multi needs distinct domains (each group updates its own norm set), got {domains}")
+        if x.shape[0] % G:
+            raise ValueError("forward_multi needs G equal mini-batches stacked along dim 0")
+        B = x.shape[0] // G
+        if not self.training:
+            res = []
+            for g, d in enumerate(domains):
+                o = self(x[g * B:(g + 1) * B], None if domain_label is None else domain_label[g * B:(g + 1) * B], d)
+                res.append(tuple(o) if isinstance(o, list) else (o, None))
+            return res
+        img_size = x.shape[2:]
+        with ops.bn_groups(G):
+            enc = self._trunk_forward(x, domain_label, domains)
+            dec4, h, w = self._decode(enc, domain_label, domains)
+        out = self._head(dec4, h, w, img_size)
+        if self.decoder_name is None:
+            return [(o, None) for o in ops.SplitDomainsFn.apply(out, G)]
+        split = [ops.SplitDomainsFn.apply(t, G) for t in [e[0] for e in enc] + [dec4, out]]
+        res = []
+        for g, d in enumerate(domains):
+            aux_out = None
+            if d in ('0', '1', '2', '3'):
+                branch = getattr(self, f'debranch{int(d) + 1}')
+                aux_out = branch([split[i][g] for i in range(5)], [(e[1], e[2]) for e in enc], img_size)
+            res.append((split[5][g], aux_out))
+        return res
+
     def _bridge_parts(self, d=None):
-        return self.bridge_conv1, self.bridge_norms1[int(d)], self.bridge_conv2, self.bridge_norms2[int(d)]
+        return self.bridge_conv1, _pick(self.bridge_norms1, d), self.bridge_conv2, _pick(self.bridge_norms2, d)
 
     def forward(self, x, domain_label=None, d=None, out_feat=False, out_seg=True):
         img_size = x.shape[2:]

@@ -15,7 +15,7 @@ import weakref
 import torch
 
 from . import _lib as L
-from ._lib import ACT_GELU, ACT_HSWISH, ACT_NONE, ACT_RELU, GemmEpi, check, ptr
+from ._lib import ACT_GELU, ACT_HSWISH, ACT_NONE, ACT_RELU, GemmEpi, check, ptr, ptr_table
 
 BF16, F32 = torch.bfloat16, torch.float32
 HEADS = 8
@@ -197,9 +197,15 @@ def cast_bf16(x, M, C, out=None, ld_in=None, ld_out=None, rowscale=None, rows_pe
 
 
 def layernorm_fwd(x, w, b, M, C, eps=1e-6):
+    """w, b: one parameter pair, or lists of G pairs (domain-specific norms: rows [g M/G, (g+1) M/G) use pair g)."""
     y = torch.empty((M, C), dtype=BF16, device=x.device)
     mean = torch.empty(M, dtype=F32, device=x.device)
     rstd = torch.empty(M, dtype=F32, device=x.device)
+    if isinstance(w, list):
+        G = len(w)
+        check(L.lib().mdv_layernorm_fwd_gp(ptr(x), ptr_table(w), ptr_table(b), ctypes.c_float(eps), ptr(y), ptr(mean), ptr(rstd), G, M // G, C,
+                                           L.stream()), "mdv_layernorm_fwd_gp")
+        return y, mean, rstd
     check(L.lib().mdv_layernorm_fwd(ptr(x), ptr(w), ptr(b), ctypes.c_float(eps), ptr(y), ptr(mean), ptr(rstd), M, C, L.stream()),
           "mdv_layernorm_fwd")
     return y, mean, rstd
@@ -207,11 +213,19 @@ def layernorm_fwd(x, w, b, M, C, eps=1e-6):
 
 def layernorm_bwd(dy, x, mean, rstd, w, dres, M, C, dg, db, *, masked=False, rowscale=None, rows_per_scale=1, drop_p=0.0,
                   drop_stream=0, dbias_masked=None):
+    """w, dg, db: tensors, or lists of G (per-group parameter sets, as in layernorm_fwd; dg / db entries may be None)."""
     dx = torch.empty((M, C), dtype=F32, device=x.device)
     dxm = torch.empty((M, C), dtype=BF16, device=x.device) if masked else None
+    rng = ptr(rng_tensor(x.device)) if drop_p > 0 else None
+    if isinstance(w, list):
+        G = len(w)
+        check(L.lib().mdv_layernorm_bwd_gp(ptr(dy), ptr(x), ptr(mean), ptr(rstd), ptr_table(w), ptr(dres), ptr(dx), ptr(dxm), ptr(rowscale),
+                                           rows_per_scale, ctypes.c_float(drop_p), rng, drop_stream, ptr_table(dg), ptr_table(db),
+                                           ptr(dbias_masked), G, M // G, C, L.stream()), "mdv_layernorm_bwd_gp")
+        return dx, dxm
     check(L.lib().mdv_layernorm_bwd(ptr(dy), ptr(x), ptr(mean), ptr(rstd), ptr(w), ptr(dres), ptr(dx), ptr(dxm), ptr(rowscale),
-                                    rows_per_scale, ctypes.c_float(drop_p), ptr(rng_tensor(x.device)) if drop_p > 0 else None,
-                                    drop_stream, ptr(dg), ptr(db), ptr(dbias_masked), M, C, L.stream()), "mdv_layernorm_bwd")
+                                    rows_per_scale, ctypes.c_float(drop_p), rng, drop_stream, ptr(dg), ptr(db), ptr(dbias_masked), M, C,
+                                    L.stream()), "mdv_layernorm_bwd")
     return dx, dxm
 
 
@@ -271,6 +285,8 @@ def bn_fold(weight, bias, running_mean, running_var, conv_bias=None, eps=1e-5):
 
 
 def bn_forward(z, M, C, weight, bias, running_mean, running_var, nbt, training, act, out_bf16, eps=1e-5, momentum=0.1):
+    """weight, bias and the three buffers are tensors, or lists of one per BatchNorm group (domain-specific norm sets: group g
+    normalises with set g and updates only its buffers)."""
     dev = z.device
     G = _BN_GROUPS if training else 1
     if M % G:
@@ -280,6 +296,14 @@ def bn_forward(z, M, C, weight, bias, running_mean, running_var, nbt, training, 
     mean = torch.empty((G, C), dtype=F32, device=dev)
     rstd = torch.empty((G, C), dtype=F32, device=dev)
     y = torch.empty((M, C), dtype=BF16 if out_bf16 else F32, device=dev)
+    if isinstance(weight, list):
+        if not training or len(weight) != G:
+            raise ValueError("per-group BatchNorm parameter sets need train mode and one set per bn_groups() group")
+        ws = torch.empty(2 * C * G, dtype=torch.float64, device=dev)
+        check(L.lib().mdv_bn_train_fwd_gp(ptr(z), G, Mg, C, ctypes.c_float(eps), ctypes.c_float(momentum), ptr_table(running_mean),
+                                          ptr_table(running_var), ptr_table(nbt), ptr_table(weight), ptr_table(bias), act, ptr(mean), ptr(rstd),
+                                          ptr(y), int(out_bf16), ptr(ws), L.stream()), "mdv_bn_train_fwd_gp")
+        return y, mean, rstd
     if training:
         ws = torch.empty(2 * C * G, dtype=torch.float64, device=dev)
         check(L.lib().mdv_bn_train_fwd_grouped(ptr(z), G, Mg, C, ctypes.c_float(eps), ctypes.c_float(momentum), ptr(running_mean),
@@ -300,9 +324,15 @@ def bn_backward(dy, z, mean, rstd, weight, bias, act, M, C, dz_bf16=True):
     Mg = M // G
     dy, z = dy.view(M, C), z.view(M, C)
     dz = torch.empty((M, C), dtype=BF16 if dz_bf16 else F32, device=dev)
+    ws = torch.empty(3 * C * G, dtype=torch.float64, device=dev)
+    if isinstance(weight, list):      # per-group parameter sets (see bn_forward): lists of gradient targets and return values
+        tg, tb = [gtarget(w) for w in weight], [gtarget(b) for b in bias]
+        check(L.lib().mdv_bn_act_bwd_gp(ptr(dy), ptr(z), ptr(mean), ptr(rstd), ptr_table(weight), ptr_table(bias), act, ptr(dz), int(dz_bf16),
+                                        ptr_table([t[0] for t in tg]), ptr_table([t[0] for t in tb]), G, Mg, C, ptr(ws), L.stream()),
+              "mdv_bn_act_bwd_gp")
+        return dz, [t[1] for t in tg], [t[1] for t in tb]
     dg, rg = gtarget(weight)
     db, rb = gtarget(bias)
-    ws = torch.empty(3 * C * G, dtype=torch.float64, device=dev)
     check(L.lib().mdv_bn_act_bwd_grouped(ptr(dy), ptr(z), ptr(mean), ptr(rstd), ptr(weight), ptr(bias), act, ptr(dz), int(dz_bf16), ptr(dg),
                                          ptr(db), G, Mg, C, ptr(ws), L.stream()), "mdv_bn_act_bwd_grouped")
     return dz, rg, rb
@@ -467,12 +497,18 @@ class BlockFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, label, cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b,
-                da_w1, da_b1, da_w2, da_b2, n2w, n2b, fc1_w, fc1_b, fc2_w, fc2_b, H, W, drop, dpr, training):
+                da_w1, da_b1, da_w2, da_b2, n2w, n2b, fc1_w, fc1_b, fc2_w, fc2_b, H, W, drop, dpr, training, *gp):
         B, N, C = x.shape
         M, dev = B * N, x.device
         hidden = fc1_w.shape[0]
         x = _contig(x)
         lib = L.lib()
+        ctx.params = (cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b, da_w1, da_b1, da_w2, da_b2,
+                      n2w, n2b, fc1_w, fc1_b, fc2_w, fc2_b) + gp
+        if gp:      # per-group LayerNorm sets: gp = (n1w, n1b, n2w, n2b) of groups 1..G-1 (see _bn_set)
+            if M % (1 + len(gp) // 4):
+                raise ValueError("LayerNorm groups must divide the batch")
+            n1w, n1b, n2w, n2b = ([p] + list(gp[i::4]) for i, p in enumerate((n1w, n1b, n2w, n2b)))
         with _dev_ctx(x):
             x1 = dwconv3(x, cpe_w, cpe_b, B, H, W, H, W, C, 1, residual=True)
             ln1, mean1, rstd1 = layernorm_fwd(x1, n1w, n1b, M, C)
@@ -526,8 +562,6 @@ class BlockFn(torch.autograd.Function):
                 gemm_nt(hact, prep_weight(fc2_w, 0, C, hidden), M, C, hidden, x3, bias=fc2_b, residual=x2, drop_p=p_drop,
                         drop_stream=sid[2], rowscale=dp2, rows_per_scale=N)
         ctx.save_for_backward(x, label, x1, mean1, rstd1, ln1, qkv, gate, hid, stats, y, x2, mean2, rstd2, ln2, u, hact, dp1, dp2, ecrpe)
-        ctx.params = (cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b, da_w1, da_b1, da_w2, da_b2,
-                      n2w, n2b, fc1_w, fc1_b, fc2_w, fc2_b)
         ctx.meta = (B, N, C, H, W, hidden, p_drop, sid, fused_mlp)
         _fwd_mark(ctx)
         return x3
@@ -536,7 +570,8 @@ class BlockFn(torch.autograd.Function):
     def backward(ctx, dx3):
         (x, label, x1, mean1, rstd1, ln1, qkv, gate, hid, stats, y, x2, mean2, rstd2, ln2, u, hact, dp1, dp2, ecrpe) = ctx.saved_tensors
         (cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b, da_w1, da_b1, da_w2, da_b2, n2w, n2b,
-         fc1_w, fc1_b, fc2_w, fc2_b) = ctx.params
+         fc1_w, fc1_b, fc2_w, fc2_b) = ctx.params[:24]
+        gp = ctx.params[24:]
         B, N, C, H, W, hidden, p_drop, sid, fused_mlp = ctx.meta
         M, dev = B * N, x.device
         lib = L.lib()
@@ -545,6 +580,11 @@ class BlockFn(torch.autograd.Function):
                                             "proj_w", "proj_b", "da_w1", "da_b1", "da_w2", "da_b2", "n2w", "n2b", "fc1_w", "fc1_b",
                                             "fc2_w", "fc2_b"), ctx.params)}
         G = {k: v[0] for k, v in T.items()}
+        TG = [gtarget(p) for p in gp]
+        if gp:      # per-group LayerNorm sets: lists over the groups of the parameters and of their gradient targets
+            n1w, n2w = [n1w] + list(gp[0::4]), [n2w] + list(gp[2::4])
+            for i, n in enumerate(("n1w", "n1b", "n2w", "n2b")):
+                G[n] = [G[n]] + [t[0] for t in TG[i::4]]
         with _dev_ctx(x):
             # ---- MLP
             # bias gradients (column sums) are by-products of the kernels that produce each output gradient
@@ -592,7 +632,7 @@ class BlockFn(torch.autograd.Function):
         _grads_done(ctx)
         R = [T[n][1] for n in ("cpe_w", "cpe_b", "c3w", "c3b", "c5w", "c5b", "c7w", "c7b", "n1w", "n1b", "qkv_w", "qkv_b", "proj_w",
                                "proj_b", "da_w1", "da_b1", "da_w2", "da_b2", "n2w", "n2b", "fc1_w", "fc1_b", "fc2_w", "fc2_b")]
-        return (dx.view(B, N, C), None, *R, None, None, None, None, None)
+        return (dx.view(B, N, C), None, *R, None, None, None, None, None, *(t[1] for t in TG))
 
 
 # ------------------------------------------------------------------------------------------------- conv pieces
@@ -600,17 +640,40 @@ def _bn_args(bn):
     return bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.num_batches_tracked
 
 
+# Domain-specific norm sets (model.MDViT_DSN.forward_multi): the norm Functions below take their norm parameters for row
+# group 0 as the usual positional arguments and those of groups 1..G-1, in the same order, group by group, as trailing
+# arguments `gp` (autograd only tracks direct tensor arguments); their `bufs` then hold every group's running buffers, group
+# by group.  With no trailing arguments they run the single-set kernels.
+def _bn_set(gb, bufs, k, nbn):
+    """(gamma, beta, running_mean, running_var, num_batches_tracked) of BatchNorm k of a Function with nbn BatchNorms: tensors with
+    one group, lists over the groups otherwise.  gb = every group's (gamma, beta) pairs, group by group; bufs likewise."""
+    G = len(gb) // (2 * nbn)
+    out = [[gb[g * 2 * nbn + 2 * k + i] for g in range(G)] for i in range(2)] + \
+          [[bufs[g * 3 * nbn + 3 * k + i] for g in range(G)] for i in range(3)]
+    return [v[0] for v in out] if G == 1 else out
+
+
+def _gp_grads(gp, rets):
+    """Gradients to return for the trailing norm arguments: rets = per-norm-slot lists over the groups (from bn_backward etc.)."""
+    if not gp:
+        return ()
+    k = len(rets)
+    return tuple(rets[j % k][1 + j // k] for j in range(len(gp)))
+
+
 class StemFn(torch.autograd.Function):
     """stem = 2x (Conv3x3 s2 no-bias -> BN -> Hardswish), mdvit.py:509-526.  im2col (bf16) + tcgen05 GEMM."""
 
     @staticmethod
-    def forward(ctx, img, w0, g0, b0, w1, g1, b1, bufs, training):
+    def forward(ctx, img, w0, g0, b0, w1, g1, b1, bufs, training, *gp):
         B, _, H, W = img.shape
         dev = img.device
         img = _contig(img.float())
         H1, W1, H2, W2 = H // 2, W // 2, H // 4, W // 4
         M0, M1 = B * H1 * W1, B * H2 * W2
-        rm0, rv0, nb0, rm1, rv1, nb1 = bufs
+        ctx.params = (w0, g0, b0, w1, g1, b1) + gp
+        g0, b0, rm0, rv0, nb0 = _bn_set(ctx.params[1:3] + ctx.params[4:6] + gp, bufs, 0, 2)
+        g1, b1, rm1, rv1, nb1 = _bn_set(ctx.params[1:3] + ctx.params[4:6] + gp, bufs, 1, 2)
         lib = L.lib()
         with _dev_ctx(img):
             # TF32 operands (fp32 in memory) for both stem convs: see mdv_gemm_nt_tf32
@@ -619,6 +682,8 @@ class StemFn(torch.autograd.Function):
             col1 = torch.empty((M1, 288), dtype=F32, device=dev)
             if not training:
                 # eval: BatchNorm (running statistics) + Hardswish folded into the GEMM epilogues
+                if gp:
+                    raise ValueError("per-group norm sets are a train-mode path")
                 a0, y = torch.empty((M0, 32), dtype=F32, device=dev), torch.empty((M1, 64), dtype=F32, device=dev)
                 s0, t0 = bn_fold(g0, b0, rm0, rv0)
                 gemm_nt(col0, prep_weight(w0, 2 | 8, 32, 27, ld=32, cin=3), M0, 32, 32, a0, tf32=True, colscale=s0, bias=t0, act=ACT_HSWISH)
@@ -636,7 +701,7 @@ class StemFn(torch.autograd.Function):
             gemm_nt(col1, prep_weight(w1, 2 | 8, 64, 288, cin=32), M1, 64, 288, z1, tf32=True)
             y, mean1, rstd1 = bn_forward(z1, M1, 64, g1, b1, rm1, rv1, nb1, training, ACT_HSWISH, False)
         ctx.save_for_backward(col0, z0, mean0, rstd0, col1, z1, mean1, rstd1)
-        ctx.params = (w0, g0, b0, w1, g1, b1)
+        ctx.sets = (g0, b0, g1, b1)
         ctx.meta = (B, H1, W1, H2, W2, training)
         _fwd_mark(ctx)
         ctx.set_materialize_grads(False)
@@ -644,13 +709,15 @@ class StemFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dy):
+        gp = ctx.params[6:]
         if dy is None:       # the da_only pass stops at the first patch embedding
-            return (None,) * 9
+            return (None,) * (9 + len(gp))
         B, H1, W1, H2, W2, training = ctx.meta
         if not training:
             raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
         col0, z0, mean0, rstd0, col1, z1, mean1, rstd1 = ctx.saved_tensors
-        w0, g0, b0, w1, g1, b1 = ctx.params
+        w0, w1 = ctx.params[0], ctx.params[3]
+        g0, b0, g1, b1 = ctx.sets
         M0, M1, dev = B * H1 * W1, B * H2 * W2, dy.device
         lib = L.lib()
         dy = _contig(dy.float())
@@ -670,6 +737,8 @@ class StemFn(torch.autograd.Function):
                 gw0p = gemm_tn(dz0, cast_bf16(col0, M0, 32), M0, 32, 32, torch.zeros((32, 32), dtype=F32, device=dev))
                 check(lib.mdv_unperm_conv_grad(ptr(gw0p), 32, ptr(gw0), 32, 3, L.stream()), "mdv_unperm_conv_grad")
         _grads_done(ctx)
+        if gp:
+            return (None, rw0, rg0[0], rb0[0], rw1, rg1[0], rb1[0], None, None) + _gp_grads(gp, [rg0, rb0, rg1, rb1])
         return None, rw0, rg0, rb0, rw1, rg1, rb1, None, None
 
 
@@ -677,16 +746,19 @@ class PatchEmbedFn(torch.autograd.Function):
     """DWCPatchEmbed: depthwise 3x3 (stride s) -> 1x1 conv -> BN -> Hardswish, mdvit.py:114-123."""
 
     @staticmethod
-    def forward(ctx, x, dw_w, pw_w, g, b, bufs, Hi, Wi, stride, training, after_stem=False):
+    def forward(ctx, x, dw_w, pw_w, g, b, bufs, Hi, Wi, stride, training, after_stem=False, *gp):
         B, _, Cin = x.shape
         C = pw_w.shape[0]
         Ho, Wo = (Hi + 2 - 3) // stride + 1, (Wi + 2 - 3) // stride + 1
         M, dev = B * Ho * Wo, x.device
         x = _contig(x)
-        rm, rv, nb = bufs
+        ctx.params = (dw_w, pw_w, g, b) + gp
+        g, b, rm, rv, nb = _bn_set((g, b) + gp, bufs, 0, 1)
         with _dev_ctx(x):
             t = dwconv3(x, dw_w, None, B, Hi, Wi, Ho, Wo, Cin, stride)          # fp32: TF32 operand of the pointwise conv
             if not training:      # eval: BatchNorm + Hardswish folded into the GEMM epilogue
+                if gp:
+                    raise ValueError("per-group norm sets are a train-mode path")
                 y = torch.empty((M, C), dtype=F32, device=dev)
                 sc, sh = bn_fold(g, b, rm, rv)
                 gemm_nt(t, _contig(pw_w).view(C, Cin), M, C, Cin, y, tf32=True, colscale=sc, bias=sh, act=ACT_HSWISH)
@@ -696,7 +768,7 @@ class PatchEmbedFn(torch.autograd.Function):
             gemm_nt(t, _contig(pw_w).view(C, Cin), M, C, Cin, z, tf32=True)
             y, mean, rstd = bn_forward(z, M, C, g, b, rm, rv, nb, training, ACT_HSWISH, False)
         ctx.save_for_backward(x, t, z, mean, rstd)
-        ctx.params = (dw_w, pw_w, g, b)
+        ctx.sets = (g, b)
         ctx.meta = (B, Hi, Wi, Ho, Wo, Cin, C, stride, training)
         _fwd_mark(ctx)
         ctx.after_stem = after_stem
@@ -708,10 +780,12 @@ class PatchEmbedFn(torch.autograd.Function):
         if not training:
             raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
         x, t, z, mean, rstd = ctx.saved_tensors
-        dw_w, pw_w, g, b = ctx.params
+        dw_w, pw_w = ctx.params[:2]
+        g, b = ctx.sets
+        gp = ctx.params[4:]
         if ctx.after_stem and not wgrad_on():
             # nothing upstream of the first patch embedding owns a domain adapter: the da_only pass stops here
-            return (None,) * 11
+            return (None,) * (11 + len(gp))
         M, dev = B * Ho * Wo, dy.device
         dy = _contig(dy.float())
         with _dev_ctx(dy):
@@ -725,6 +799,8 @@ class PatchEmbedFn(torch.autograd.Function):
             g_dw, r_dw = gtarget(dw_w)
             dwconv3_wgrad(dt, x, g_dw, None, B, Hi, Wi, Ho, Wo, Cin, stride)
         _grads_done(ctx)
+        if gp:
+            return (dx.view(B, Hi * Wi, Cin), r_dw, r_pw, rg[0], rb[0], None, None, None, None, None, None) + _gp_grads(gp, [rg, rb])
         return dx.view(B, Hi * Wi, Cin), r_dw, r_pw, rg, rb, None, None, None, None, None, None
 
 
@@ -732,18 +808,23 @@ class BridgeFn(torch.autograd.Function):
     """bridge = 2x (Conv3x3 + bias -> BN -> ReLU), mdvit.py:557-564."""
 
     @staticmethod
-    def forward(ctx, x, w0, c0, g0, b0, w1, c1, g1, b1, bufs, H, W, training):
+    def forward(ctx, x, w0, c0, g0, b0, w1, c1, g1, b1, bufs, H, W, training, *gp):
         B, _, C = x.shape
         C0, C1 = w0.shape[0], w1.shape[0]
         M, dev = B * H * W, x.device
         x = _contig(x)
-        rm0, rv0, nb0, rm1, rv1, nb1 = bufs
+        ctx.params = (w0, c0, g0, b0, w1, c1, g1, b1) + gp
+        gb = (g0, b0, g1, b1) + gp
+        g0, b0, rm0, rv0, nb0 = _bn_set(gb, bufs, 0, 2)
+        g1, b1, rm1, rv1, nb1 = _bn_set(gb, bufs, 1, 2)
         lib = L.lib()
         with _dev_ctx(x):
             col0 = torch.empty((M, 9 * C), dtype=F32, device=dev)
             check(lib.mdv_im2col3(ptr(x), 0, ptr(col0), 0, B, H, W, H, W, C, 1, 9 * C, L.stream()), "mdv_im2col3")
             col1 = torch.empty((M, 9 * C0), dtype=F32, device=dev)
             if not training:      # eval: conv bias + BatchNorm + ReLU folded into the GEMM epilogues
+                if gp:
+                    raise ValueError("per-group norm sets are a train-mode path")
                 a0, y = torch.empty((M, C0), dtype=F32, device=dev), torch.empty((M, C1), dtype=F32, device=dev)
                 s0, t0 = bn_fold(g0, b0, rm0, rv0, c0)
                 gemm_nt(col0, prep_weight(w0, 2 | 8, C0, 9 * C, cin=C), M, C0, 9 * C, a0, tf32=True, colscale=s0, bias=t0, act=ACT_RELU)
@@ -760,7 +841,7 @@ class BridgeFn(torch.autograd.Function):
             gemm_nt(col1, prep_weight(w1, 2 | 8, C1, 9 * C0, cin=C0), M, C1, 9 * C0, z1, bias=c1, tf32=True)
             y, mean1, rstd1 = bn_forward(z1, M, C1, g1, b1, rm1, rv1, nb1, training, ACT_RELU, False)
         ctx.save_for_backward(col0, z0, mean0, rstd0, col1, z1, mean1, rstd1)
-        ctx.params = (w0, c0, g0, b0, w1, c1, g1, b1)
+        ctx.sets = (g0, b0, g1, b1)
         ctx.meta = (B, H, W, C, C0, C1, training)
         _fwd_mark(ctx)
         return y.view(B, H * W, C1)
@@ -771,7 +852,9 @@ class BridgeFn(torch.autograd.Function):
         if not training:
             raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
         col0, z0, mean0, rstd0, col1, z1, mean1, rstd1 = ctx.saved_tensors
-        w0, c0, g0, b0, w1, c1, g1, b1 = ctx.params
+        w0, c0, _, _, w1, c1 = ctx.params[:6]
+        g0, b0, g1, b1 = ctx.sets
+        gp = ctx.params[8:]
         M, dev = B * H * W, dy.device
         lib = L.lib()
         dy = _contig(dy.float())
@@ -795,6 +878,9 @@ class BridgeFn(torch.autograd.Function):
             dz0, rg0, rb0 = bn_backward(da0, z0, mean0, rstd0, g0, b0, ACT_RELU, M, C0)
             rw0, rc0, dx = conv_bwd(dz0, col0, w0, c0, C0, C)
         _grads_done(ctx)
+        if gp:
+            return ((dx.view(B, H * W, C), rw0, rc0, rg0[0], rb0[0], rw1, rc1, rg1[0], rb1[0], None, None, None, None)
+                    + _gp_grads(gp, [rg0, rb0, rg1, rb1]))
         return dx.view(B, H * W, C), rw0, rc0, rg0, rb0, rw1, rc1, rg1, rb1, None, None, None, None
 
 
@@ -803,12 +889,13 @@ class DecoderConvFn(torch.autograd.Function):
     grouped 3x3 (2 in/group) -> 1x1 -> BN -> Hardswish.  conv_before is commuted in front of the resize (exact)."""
 
     @staticmethod
-    def forward(ctx, inp, skip, cb_w, cb_b, dw_w, pw_w, g, b, bufs, h, w, H, W, training):
+    def forward(ctx, inp, skip, cb_w, cb_b, dw_w, pw_w, g, b, bufs, h, w, H, W, training, *gp):
         B, _, Cin = inp.shape
         C = cb_w.shape[0]
         m, M, dev = B * h * w, B * H * W, inp.device
         inp, skip = _contig(inp), _contig(skip)
-        rm, rv, nb = bufs
+        ctx.params = (cb_w, cb_b, dw_w, pw_w, g, b) + gp
+        g, b, rm, rv, nb = _bn_set((g, b) + gp, bufs, 0, 1)
         lib = L.lib()
         with _dev_ctx(inp):
             # both 1x1 convs of the decoder trunk run on TF32 operands (fp32 in memory): see mdv_gemm_nt_tf32
@@ -818,6 +905,8 @@ class DecoderConvFn(torch.autograd.Function):
             gc = torch.empty((M, C), dtype=F32, device=dev)
             check(lib.mdv_gconv2_fwd(ptr(skip), ptr(up), ptr(dw_w), ptr(gc), 0, B, H, W, C, L.stream()), "mdv_gconv2_fwd")
             if not training:      # eval: BatchNorm + Hardswish folded into the GEMM epilogue
+                if gp:
+                    raise ValueError("per-group norm sets are a train-mode path")
                 y = torch.empty((M, C), dtype=F32, device=dev)
                 sc, sh = bn_fold(g, b, rm, rv)
                 gemm_nt(gc, _contig(pw_w).view(C, C), M, C, C, y, tf32=True, colscale=sc, bias=sh, act=ACT_HSWISH)
@@ -827,7 +916,7 @@ class DecoderConvFn(torch.autograd.Function):
             gemm_nt(gc, _contig(pw_w).view(C, C), M, C, C, z, tf32=True)
             y, mean, rstd = bn_forward(z, M, C, g, b, rm, rv, nb, training, ACT_HSWISH, False)
         ctx.save_for_backward(skip, inp, up, gc, z, mean, rstd)
-        ctx.params = (cb_w, cb_b, dw_w, pw_w, g, b)
+        ctx.sets = (g, b)
         ctx.meta = (B, h, w, H, W, Cin, C, training)
         _fwd_mark(ctx)
         return y.view(B, H * W, C)
@@ -838,7 +927,9 @@ class DecoderConvFn(torch.autograd.Function):
         if not training:
             raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
         skip, inp, up, gc, z, mean, rstd = ctx.saved_tensors
-        cb_w, cb_b, dw_w, pw_w, g, b = ctx.params
+        cb_w, cb_b, dw_w, pw_w = ctx.params[:4]
+        g, b = ctx.sets
+        gp = ctx.params[6:]
         m, M, dev = B * h * w, B * H * W, dy.device
         lib = L.lib()
         dy = _contig(dy.float())
@@ -864,6 +955,9 @@ class DecoderConvFn(torch.autograd.Function):
             dinp = torch.empty((m, Cin), dtype=F32, device=dev)
             gemm_nt(dtb, prep_weight(cb_w, 1, C, Cin), m, Cin, C, dinp)
         _grads_done(ctx)
+        if gp:
+            return ((dinp.view(B, h * w, Cin), dskip.view(B, H * W, C), r_cb, r_cbb, r_dw, r_pw, rg[0], rb[0], None, None, None, None, None, None)
+                    + _gp_grads(gp, [rg, rb]))
         return (dinp.view(B, h * w, Cin), dskip.view(B, H * W, C), r_cb, r_cbb, r_dw, r_pw, rg, rb, None, None, None, None, None, None)
 
 

@@ -245,7 +245,7 @@ class MKDTrainer:
         """batches: list of (img [B,3,H,W], label [B,1,H,W] fp32 or uint8, domain index).  Returns [n_dom, 3] losses
         (seg, aux, kt).  The partial sums of all domains are all-reduced in ONE collective after the last forward."""
         # (with_aux=False on a model WITH auxiliary branches keeps the per-domain loop: its forward_multi would compute them)
-        if (self.fuse_domains and (self.with_aux or not hasattr(self.model, "decoder_name")) and len(batches) > 1
+        if (self.fuse_domains and (self.with_aux or getattr(self.model, "decoder_name", None) is None) and len(batches) > 1
                 and hasattr(self.model, "forward_multi") and len({tuple(b[0].shape) for b in batches}) == 1):
             return self._forward_losses_fused(batches)
         outs, auxs = [], []
@@ -258,6 +258,10 @@ class MKDTrainer:
                 ops.set_forward_use_cb(None)
             if self.with_aux:
                 o, a = self.model(img, self._labels_onehot(img.shape[0], d, img.device), str(d))
+            elif getattr(self.model, "domain_specific_norms", False):
+                # (BASE_DSN: the domain key selects the norm set; the label only feeds domain adapters)
+                o = self.model(img, self._labels_onehot(img.shape[0], d, img.device) if self.da_params else None, str(d))
+                o, a = (o[0] if isinstance(o, (list, tuple)) else o), None
             else:
                 o = self.model(img)
                 o, a = (o[0] if isinstance(o, (list, tuple)) else o), None
@@ -306,8 +310,10 @@ class MKDTrainer:
         ops.set_forward_tag(0)
         if recording:
             ops.set_forward_use_cb(lambda tag, params: self.bucketer.record_use([id(p) for p in params if p is not None]))
-        # (a model without auxiliary branches is trained without the domain label, as multi_train_BASE.py does: model(img))
-        res = self.model.forward_multi(x, dl if self.with_aux else None, [str(b[2]) for b in batches])
+        # (a model without auxiliary branches is trained without the domain label, as multi_train_BASE.py does: model(img), unless
+        # it has domain adapters to feed)
+        label = dl if (self.with_aux or (self.da_params and getattr(self.model, "domain_specific_norms", False))) else None
+        res = self.model.forward_multi(x, label, [str(b[2]) for b in batches])
         ops.set_forward_use_cb(None)
         ops.set_forward_tag(None)
         n_total = res[0][0].numel() * self.world
