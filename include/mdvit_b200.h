@@ -126,12 +126,14 @@ int mdv_layernorm_bwd(const float* dy, const float* x, const float* mean, const 
                       float drop_p, const void* rng, uint32_t drop_stream, float* dgamma, float* dbeta,
                       float* dbias_masked /* [C] += column sums of dx_masked, or NULL */, int M, int C, void* stream);
 
-/* ------------------------------------------------------------------ per-group norm parameter sets (MDViT_DSN / BASE_DSN) */
-/* The stacked multi-domain pass of the domain-specific-norm models runs G single-domain mini-batches as one [G*Mg, C]
- * tensor; row group g = rows [g*Mg, (g+1)*Mg) uses norm parameter set g.  A table names one tensor per group (p[g], g < G);
- * it is passed by value, so a captured CUDA graph holds the addresses and no host-to-device copy is needed.  1 <= G <= 8.
- * Two groups naming the same running buffer or the same gradient target would race: those calls return MDV_ERR_ARG
- * before any CUDA call. */
+/* ------------------------------------------------------------------ row groups with norm parameter tables */
+/* The stacked multi-domain pass runs G single-domain mini-batches as one [G*Mg, C] tensor; row group g = rows
+ * [g*Mg, (g+1)*Mg) uses norm parameter set g.  A table names one tensor per group (p[g], g < G); it is passed by value, so a
+ * captured CUDA graph holds the addresses and no host-to-device copy is needed.  1 <= G <= 8, else MDV_ERR_ARG before any
+ * CUDA call.  Entries may repeat: one set named G times is a shared set (MDViT's stacked pass, TransFuse's dataset
+ * groups), G distinct sets are domain-specific norms (MDViT_DSN / BASE_DSN).  Groups that name the same running buffers
+ * update them in group order, and groups that name the same gradient target add to it, exactly as consecutive
+ * single-set calls would. */
 #define MDV_MAX_GROUPS 8
 typedef struct MdvPtrTable {
     void* p[MDV_MAX_GROUPS];
@@ -145,10 +147,11 @@ int mdv_layernorm_bwd_gp(const float* dy, const float* x, const float* mean, con
                          const float* dres, float* dx, void* dx_masked_bf16, const float* rowscale, int rows_per_scale,
                          float drop_p, const void* rng, uint32_t drop_stream, MdvPtrTable dgamma, MdvPtrTable dbeta,
                          float* dbias_masked, int G, int Mg, int C, void* stream);
-/* mdv_bn_train_fwd_grouped / mdv_bn_act_bwd_grouped with one parameter set per group: group g normalises with gamma[g],
- * beta[g] and updates only running_mean[g], running_var[g] (momentum, unbiased variance) and *num_batches_tracked[g] += 1,
- * exactly as nn.BatchNorm2d set g would on its own mini-batch; dgamma[g] / dbeta[g] accumulate group g's sums.  Buffer and
- * gradient entries may be NULL.  Workspaces as for the grouped forms. */
+/* Train-mode BatchNorm2d (+act) on G row groups: group g normalises with its own batch statistics, gamma[g] and beta[g],
+ * and updates running_mean[g], running_var[g] (momentum, unbiased variance) and *num_batches_tracked[g] += 1, as
+ * nn.BatchNorm2d would on that mini-batch; dgamma[g] / dbeta[g] accumulate (+=) group g's sums.  Buffer and gradient entries
+ * may be NULL.  mean/rstd: [G, C].  C % 4 == 0, 32 <= C <= 1024, G*Mg*C < 2^31, else MDV_ERR_UNSUPPORTED.
+ * fwd ws >= 2*C*G doubles; bwd ws >= 2*C*G doubles + 2*C*G floats. */
 int mdv_bn_train_fwd_gp(const float* z, int G, int Mg, int C, float eps, float momentum, MdvPtrTable running_mean,
                         MdvPtrTable running_var, MdvPtrTable num_batches_tracked, MdvPtrTable gamma, MdvPtrTable beta, int act,
                         float* mean, float* rstd, void* y, int y_bf16, void* ws, void* stream);
@@ -158,7 +161,8 @@ int mdv_bn_act_bwd_gp(const float* dy, const float* z, const float* mean, const 
 
 /* ------------------------------------------------------------------ BatchNorm2d (+act) on [M=B*H*W, C] (mpvit.py:119-122 ...) */
 /* training: batch mean / biased var -> mean,rstd; running stats updated with momentum (unbiased var) and
- * *num_batches_tracked += 1.  eval: mean,rstd from the running buffers.  ws >= 2*C doubles. */
+ * *num_batches_tracked += 1 (mdv_bn_train_fwd_gp's statistics with G = 1: shapes outside its limits return
+ * MDV_ERR_UNSUPPORTED).  eval: mean,rstd from the running buffers.  ws >= 2*C doubles. */
 int mdv_bn_stats(const float* z, int M, int C, float eps, float momentum, int training, float* running_mean,
                  float* running_var, long long* num_batches_tracked, float* mean, float* rstd, void* ws, void* stream);
 /* Eval-mode BatchNorm as a per-channel affine map folded into the GEMM that produces its input (MdvGemmEpi.colscale/bias):
@@ -167,23 +171,15 @@ int mdv_bn_fold(const float* gamma, const float* beta, const float* running_mean
                 float eps, float* scale, float* shift, int C, void* stream);
 int mdv_bn_act_fwd(const float* z, const float* mean, const float* rstd, const float* gamma, const float* beta, int act,
                    void* y, int y_bf16, int M, int C, void* stream);
-/* dz for y = act(BN_train(z)); ws >= 2*C doubles + 2*C floats; dgamma/dbeta accumulate. */
+/* dz for y = act(BN_train(z)); ws >= 2*C doubles + 2*C floats; dgamma/dbeta accumulate.  mdv_bn_act_bwd_gp with G = 1:
+ * shapes outside its limits return MDV_ERR_UNSUPPORTED. */
 int mdv_bn_act_bwd(const float* dy, const float* z, const float* mean, const float* rstd, const float* gamma,
                    const float* beta, int act, void* dz, int dz_bf16, float* dgamma, float* dbeta, int M, int C, void* ws,
                    void* stream);
-/* Grouped forms: z is [G*Mg, C], group g = rows [g*Mg, (g+1)*Mg) = one single-domain mini-batch of the stacked multi-domain
- * forward; statistics, running-buffer updates (in group order) and gradients are exactly those of G consecutive
- * nn.BatchNorm2d calls, in 3 launches instead of 4G / 3G.  mean/rstd: [G, C].  C % 4 == 0, 32 <= C <= 1024.
- * fwd ws >= 2*C*G doubles; bwd ws >= 2*C*G doubles + 2*C*G floats. */
-int mdv_bn_train_fwd_grouped(const float* z, int G, int Mg, int C, float eps, float momentum, float* running_mean, float* running_var,
-                             long long* num_batches_tracked, const float* gamma, const float* beta, int act, float* mean, float* rstd,
-                             void* y, int y_bf16, void* ws, void* stream);
-int mdv_bn_act_bwd_grouped(const float* dy, const float* z, const float* mean, const float* rstd, const float* gamma, const float* beta,
-                           int act, void* dz, int dz_bf16, float* dgamma, float* dbeta, int G, int Mg, int C, void* ws, void* stream);
-/* Same with a rank-1 output gradient dy[m,c] = dlog[m] * wrow[c] * dropout2d_mask(m / rows_per_sample, c) generated on the
- * fly: the backward of Dropout2d + the 1-channel `linear_out` head of MLPDecoderFM (Decoders.py:334-337) never
- * materialises the [M, C] gradient of the BatchNorm output. */
-/* (ws here: >= 3*C doubles + (M / rows_per_sample)*C floats) */
+/* mdv_bn_act_bwd with a rank-1 output gradient dy[m,c] = dlog[m] * wrow[c] * dropout2d_mask(m / rows_per_sample, c) generated
+ * on the fly: the backward of Dropout2d + the 1-channel `linear_out` head of MLPDecoderFM (Decoders.py:334-337) never
+ * materialises the [M, C] gradient of the BatchNorm output.  M % rows_per_sample != 0 returns MDV_ERR_UNSUPPORTED.
+ * (ws here: >= 3*C doubles + (M / rows_per_sample)*C floats) */
 int mdv_bn_act_bwd_rank1(const float* dlog, const float* wrow, int rows_per_sample, float drop_p, const void* rng,
                          uint32_t drop_stream, const float* z, const float* mean, const float* rstd, const float* gamma,
                          const float* beta, int act, void* dz, int dz_bf16, float* dgamma, float* dbeta, int M, int C, void* ws,

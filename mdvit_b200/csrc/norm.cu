@@ -13,20 +13,17 @@ constexpr int LN_MAXV = 8;  // float2 per lane -> C <= 512
 // ---------------------------------------------------------------------------------- LayerNorm forward
 // one warp owns R rows per iteration (all loads issued before any arithmetic: at C = 64 a row is only 256 B, and one
 // row per warp leaves HBM latency exposed); a row lives in registers, NV float2 per lane.
-// GP: per-group parameter sets — blockIdx.y is the row group, M its row count, and gamma/beta come from the tables.
-template <int NV, int R, bool GP>
-__global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x, const float* __restrict__ gamma,
-                                                      const float* __restrict__ beta, float eps, bf16* __restrict__ y,
-                                                      float* __restrict__ mean_out, float* __restrict__ rstd_out, int M,
-                                                      const __grid_constant__ MdvPtrTable gtab, const __grid_constant__ MdvPtrTable btab) {
+// blockIdx.y is the row group (M rows); its gamma / beta are gtab.p[blockIdx.y] / btab.p[blockIdx.y].
+template <int NV, int R>
+__global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x, const __grid_constant__ MdvPtrTable gtab,
+                                                      const __grid_constant__ MdvPtrTable btab, float eps, bf16* __restrict__ y,
+                                                      float* __restrict__ mean_out, float* __restrict__ rstd_out, int M) {
     MDV_PDL_SYNC();
     constexpr int C = NV * 64;
     const int lane = threadIdx.x & 31;
-    const int lo = GP ? blockIdx.y * M : 0, hi = lo + M;
-    if (GP) {
-        gamma = (const float*)gtab.p[blockIdx.y];
-        beta = (const float*)btab.p[blockIdx.y];
-    }
+    const int lo = blockIdx.y * M, hi = lo + M;
+    const float* __restrict__ gamma = (const float*)gtab.p[blockIdx.y];
+    const float* __restrict__ beta = (const float*)btab.p[blockIdx.y];
     const int row0 = lo + (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * R;
     if (row0 >= hi) return;
     float2 v[R][NV];
@@ -76,28 +73,25 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x
 // and its column sums (that Linear's bias gradient) are accumulated into dbias_masked.
 // One warp owns R rows per iteration (all of their loads are issued before any arithmetic: with C = 64 a row is only
 // 256 B, so a single row per warp leaves HBM latency exposed); a row lives in registers, NV float2 per lane.
-// GP: blockIdx.y is the row group (M rows) and gamma, dgamma, dbeta come from the tables — a block never crosses a group boundary,
+// blockIdx.y is the row group (M rows) and gamma, dgamma, dbeta come from the tables — a block never crosses a group boundary,
 // so its column partials belong to one group's dgamma / dbeta.
-template <int NV, int R, bool GP>
+template <int NV, int R>
 __global__ void __launch_bounds__(256) ln_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ x,
                                                       const float* __restrict__ mean_in, const float* __restrict__ rstd_in,
-                                                      const float* __restrict__ gamma, const float* __restrict__ dres,
+                                                      const __grid_constant__ MdvPtrTable gtab, const float* __restrict__ dres,
                                                       float* __restrict__ dx, bf16* __restrict__ dx_masked,
                                                       const float* __restrict__ rowscale, int rows_per_scale, float drop_p,
                                                       const unsigned long long* __restrict__ rng, uint32_t drop_stream,
-                                                      float* __restrict__ dgamma, float* __restrict__ dbeta,
-                                                      float* __restrict__ dbias_masked, int M, const __grid_constant__ MdvPtrTable gtab,
-                                                      const __grid_constant__ MdvPtrTable dgtab, const __grid_constant__ MdvPtrTable dbtab) {
+                                                      const __grid_constant__ MdvPtrTable dgtab, const __grid_constant__ MdvPtrTable dbtab,
+                                                      float* __restrict__ dbias_masked, int M) {
     MDV_PDL_SYNC();
     constexpr int C = NV * 64;
     __shared__ float red[8][64];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
-    const int lo = GP ? blockIdx.y * M : 0, hi = lo + M;
-    if (GP) {
-        gamma = (const float*)gtab.p[blockIdx.y];
-        dgamma = (float*)dgtab.p[blockIdx.y];
-        dbeta = (float*)dbtab.p[blockIdx.y];
-    }
+    const int lo = blockIdx.y * M, hi = lo + M;
+    const float* __restrict__ gamma = (const float*)gtab.p[blockIdx.y];
+    float* __restrict__ dgamma = (float*)dgtab.p[blockIdx.y];
+    float* __restrict__ dbeta = (float*)dbtab.p[blockIdx.y];
     float2 ag[NV], ab[NV], am[NV], gm[NV];
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
@@ -211,54 +205,14 @@ __device__ __forceinline__ float act_bwd(float v, int act) {
     return 1.f;
 }
 
-// sums[c] += sum_m z[m,c]; sums[C+c] += sum_m z[m,c]^2   (double accumulators; block = 32 channels x 8 row lanes)
-__global__ void __launch_bounds__(256) bn_stats_kernel(const float* __restrict__ z, double* __restrict__ sums, int M, int C,
-                                                        int rows_per_block) {
-    MDV_PDL_SYNC();
-    __shared__ float sh[2][8][33];
-    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-    const int c = blockIdx.x * 32 + tx;
-    const int r0 = blockIdx.y * rows_per_block, r1 = min(M, r0 + rows_per_block);
-    float s = 0.f, q = 0.f;
-    if (c < C)
-        for (int r = r0 + ty; r < r1; r += 8) {
-            float v = __ldg(z + (size_t)r * C + c);
-            s += v;
-            q += v * v;
-        }
-    sh[0][ty][tx] = s;
-    sh[1][ty][tx] = q;
-    __syncthreads();
-    if (ty < 2 && c < C) {
-        float t = 0.f;
-        for (int i = 0; i < 8; ++i) t += sh[ty][i][tx];
-        atomicAdd(sums + ty * C + c, (double)t);
-    }
-}
-
-// train: mean/rstd from batch sums + running-stat update (unbiased var), eval: from running stats.
-__global__ void bn_finalize_kernel(const double* __restrict__ sums, int M, int C, float eps, float momentum, int training,
-                                   float* __restrict__ running_mean, float* __restrict__ running_var,
-                                   long long* __restrict__ num_batches, float* __restrict__ mean, float* __restrict__ rstd) {
+// eval: mean/rstd from the running buffers
+__global__ void bn_eval_stats_kernel(const float* __restrict__ running_mean, const float* __restrict__ running_var, float eps,
+                                     float* __restrict__ mean, float* __restrict__ rstd, int C) {
     MDV_PDL_SYNC();
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c == 0 && training && num_batches) *num_batches += 1;
     if (c >= C) return;
-    if (training) {
-        double mu = sums[c] / M;
-        double var = sums[C + c] / M - mu * mu;
-        if (var < 0) var = 0;
-        mean[c] = (float)mu;
-        rstd[c] = (float)(1.0 / sqrt(var + (double)eps));
-        if (running_mean) {
-            running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)mu;
-            double unb = M > 1 ? var * M / (M - 1) : var;
-            running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unb;
-        }
-    } else {
-        mean[c] = running_mean[c];
-        rstd[c] = rsqrtf(running_var[c] + eps);
-    }
+    mean[c] = running_mean[c];
+    rstd[c] = rsqrtf(running_var[c] + eps);
 }
 
 template <typename TO>
@@ -285,7 +239,6 @@ __global__ void __launch_bounds__(256) bn_act_fwd_kernel(const float* __restrict
     }
 }
 
-// sums[c] += sum g, sums[C+c] += sum g*xhat with g = dy * act'(bn(z))
 // Rank-1 output gradient (the commuted 1-channel head, Decoders.py:334-337): dy[m,c] = dlog[m] * wrow[c] * dropout2d_mask(m / rps, c)
 // is generated on the fly instead of being materialised as an [M, C] fp32 tensor.
 struct Rank1Dy {
@@ -297,118 +250,12 @@ struct Rank1Dy {
     uint32_t stream;
     const float* wtab;      // [samples, C] = wrow[c] * dropout2d_mask(b, c), precomputed once per call (vectorised kernels)
 };
-__device__ __forceinline__ float rank1_wm(const Rank1Dy& r1, int b, int c, int C) {
-    float wv = __ldg(r1.wrow + c);
-    if (r1.drop_p > 0.f) wv *= drop_scale(rng_key(r1.rng, r1.stream), (unsigned long long)b * C + c, drop_thresh(r1.drop_p), 1.f / (1.f - r1.drop_p));
-    return wv;
-}
 
-__global__ void __launch_bounds__(256) bn_bwd_reduce_kernel(const float* __restrict__ dy, const float* __restrict__ z,
-                                                             const float* __restrict__ mean, const float* __restrict__ rstd,
-                                                             const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                             int act, double* __restrict__ sums, int M, int C, int rows_per_block,
-                                                             Rank1Dy r1) {
-    MDV_PDL_SYNC();
-    __shared__ float sh[2][8][33];
-    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-    const int c = blockIdx.x * 32 + tx;
-    const int r0 = blockIdx.y * rows_per_block, r1e = min(M, r0 + rows_per_block);
-    float s = 0.f, q = 0.f;
-    if (c < C) {
-        const float mu = mean[c], rs = rstd[c], g = gamma[c], b = beta[c];
-        int cur_b = -1;
-        float wm = 0.f;
-        for (int r = r0 + ty; r < r1e; r += 8) {
-            const size_t o = (size_t)r * C + c;
-            const float xh = (__ldg(z + o) - mu) * rs;
-            float d;
-            if (r1.dlog) {
-                const int bb = r / r1.rps;
-                if (bb != cur_b) {
-                    cur_b = bb;
-                    wm = rank1_wm(r1, bb, c, C);
-                }
-                d = __ldg(r1.dlog + r) * wm;
-            } else {
-                d = __ldg(dy + o);
-            }
-            const float gg = d * act_bwd(xh * g + b, act);
-            s += gg;
-            q += gg * xh;
-        }
-    }
-    sh[0][ty][tx] = s;
-    sh[1][ty][tx] = q;
-    __syncthreads();
-    if (ty < 2 && c < C) {
-        float t = 0.f;
-        for (int i = 0; i < 8; ++i) t += sh[ty][i][tx];
-        atomicAdd(sums + ty * C + c, (double)t);
-    }
-}
-
-// coef[c] = sum_g / M, coef[C+c] = sum_gxhat / M;  dgamma += sum_gxhat; dbeta += sum_g
-__global__ void bn_bwd_finalize_kernel(const double* __restrict__ sums, int M, int C, float* __restrict__ coef,
-                                       float* __restrict__ dgamma, float* __restrict__ dbeta) {
-    MDV_PDL_SYNC();
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= C) return;
-    coef[c] = (float)(sums[c] / M);
-    coef[C + c] = (float)(sums[C + c] / M);
-    if (dbeta) atomicAdd(dbeta + c, (float)sums[c]);
-    if (dgamma) atomicAdd(dgamma + c, (float)sums[C + c]);
-}
-
-template <typename TO>
-__global__ void __launch_bounds__(256) bn_bwd_apply_kernel(const float* __restrict__ dy, const float* __restrict__ z,
-                                                            const float* __restrict__ mean, const float* __restrict__ rstd,
-                                                            const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                            int act, const float* __restrict__ coef, TO* __restrict__ dz,
-                                                            int total, int C, Rank1Dy r1) {
-    MDV_PDL_SYNC();
-    const int i = (blockIdx.x * blockDim.x + threadIdx.x) * 4;      // 32-bit: the host checks M*C < 2^31
-    if (i >= total) return;
-    const int c = i % C;
-    float4 zv = *reinterpret_cast<const float4*>(z + i);
-    float4 dv;
-    if (r1.dlog) {
-        // 32-bit index math (total < 2^31 checked on the host); b*C + c is a multiple of 4: two pair-hashes give the 4 masks
-        const int row = i / C;
-        const int bb = row / r1.rps;
-        const float dl = __ldg(r1.dlog + row);
-        const float4 wv = *reinterpret_cast<const float4*>(r1.wrow + c);
-        float m0 = 1.f, m1 = 1.f, m2 = 1.f, m3 = 1.f;
-        if (r1.drop_p > 0.f) {
-            const uint32_t key = rng_key(r1.rng, r1.stream), thr = drop_thresh(r1.drop_p);
-            const float inv = 1.f / (1.f - r1.drop_p);
-            const uint32_t pr = (uint32_t)(bb * C + c) >> 1;
-            const uint32_t h0 = drop_hash(key, pr), h1 = drop_hash(key, pr + 1);
-            m0 = drop_lo(h0, thr, inv); m1 = drop_hi(h0, thr, inv); m2 = drop_lo(h1, thr, inv); m3 = drop_hi(h1, thr, inv);
-        }
-        dv = make_float4(dl * wv.x * m0, dl * wv.y * m1, dl * wv.z * m2, dl * wv.w * m3);
-    } else {
-        dv = *reinterpret_cast<const float4*>(dy + i);
-    }
-    float zz[4] = {zv.x, zv.y, zv.z, zv.w}, dd[4] = {dv.x, dv.y, dv.z, dv.w}, o[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const int cc = c + j;
-        const float rs = __ldg(rstd + cc), g = __ldg(gamma + cc);
-        const float xh = (zz[j] - __ldg(mean + cc)) * rs;
-        const float gg = dd[j] * act_bwd(xh * g + __ldg(beta + cc), act);
-        o[j] = g * rs * (gg - __ldg(coef + cc) - xh * __ldg(coef + C + cc));
-    }
-    if (sizeof(TO) == 4) {
-        *reinterpret_cast<float4*>(reinterpret_cast<float*>(dz) + i) = make_float4(o[0], o[1], o[2], o[3]);
-    } else {
-        *reinterpret_cast<uint2*>(reinterpret_cast<bf16*>(dz) + i) = make_uint2(f2_to_bf2(o[0], o[1]), f2_to_bf2(o[2], o[3]));
-    }
-}
-
-// ------------------------------------------------------------------------------------------------ grouped BatchNorm
+// ------------------------------------------------------------------------------------------------ train-mode BatchNorm
 // The fused multi-domain forward stacks G single-domain mini-batches along the rows; BatchNorm statistics are per group of
 // Mg consecutive rows (one reference forward each).  These kernels handle all groups in ONE launch (grid.z = group) with
-// float4 loads and 4 rows in flight per thread, instead of G launches of scalar-load kernels.
+// float4 loads and 4 rows in flight per thread; a single BatchNorm call is the case G = 1.  Group g's gamma / beta are
+// gt.p[g] / bt.p[g]: one parameter set repeated G times, or one set per group (domain-specific norms).
 // Thread layout: C/4 threads per row (one float4 of channels each), RPI = 256 / (C/4) rows per block iteration.
 // (b*C + c) is a multiple of 4: two pair-hashes give the four Dropout2d masks of a float4 of channels
 __device__ __forceinline__ float4 rank1_w4(const Rank1Dy& r1, int b, int c, int C) {
@@ -430,11 +277,9 @@ __global__ void rank1_table_kernel(Rank1Dy r1, float* __restrict__ wtab, int sam
     *reinterpret_cast<float4*>(wtab + i) = rank1_w4(r1, i / C, i % C, C);
 }
 
-// GP (all grouped kernels below): group g's gamma / beta are gt.p[g] / bt.p[g] (domain-specific norm sets) instead of one shared pair
-template <bool BWD, bool RANK1 = false, bool GP = false>
+template <bool BWD, bool RANK1 = false>
 __global__ void __launch_bounds__(256) bn_reduce_g_kernel(const float* __restrict__ a, const float* __restrict__ z,
-                                                           const float* __restrict__ mean, const float* __restrict__ rstd,
-                                                           const float* __restrict__ gamma, const float* __restrict__ beta, int act,
+                                                           const float* __restrict__ mean, const float* __restrict__ rstd, int act,
                                                            double* __restrict__ sums, int Mg, int C, int rows_per_block,
                                                            Rank1Dy rk, const __grid_constant__ MdvPtrTable gt, const __grid_constant__ MdvPtrTable bt) {
     MDV_PDL_SYNC();
@@ -443,10 +288,8 @@ __global__ void __launch_bounds__(256) bn_reduce_g_kernel(const float* __restric
     const int rpi = 256 / tpr;                    // rows per block iteration
     const int cl = threadIdx.x % tpr, rl = threadIdx.x / tpr;
     const int g = blockIdx.z;
-    if (GP) {
-        gamma = (const float*)gt.p[g];
-        beta = (const float*)bt.p[g];
-    }
+    const float* __restrict__ gamma = (const float*)gt.p[g];
+    const float* __restrict__ beta = (const float*)bt.p[g];
     const int r0 = blockIdx.x * rows_per_block, r1 = min(Mg, r0 + rows_per_block);
     const size_t base = (size_t)g * Mg * C;
     float4 s = make_float4(0.f, 0.f, 0.f, 0.f), q = s;
@@ -519,47 +362,18 @@ __global__ void __launch_bounds__(256) bn_reduce_g_kernel(const float* __restric
     }
 }
 
-// train-mode statistics of G groups; the running buffers are updated group by group IN ORDER, exactly as G consecutive
-// nn.BatchNorm2d forwards would (momentum update is not commutative)
-__global__ void bn_finalize_g_kernel(const double* __restrict__ sums, int G, int Mg, int C, float eps, float momentum,
-                                     float* __restrict__ running_mean, float* __restrict__ running_var,
-                                     long long* __restrict__ num_batches, float* __restrict__ mean, float* __restrict__ rstd) {
-    MDV_PDL_SYNC();
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c == 0 && num_batches) *num_batches += G;
-    if (c >= C) return;
-    float rm = running_mean ? running_mean[c] : 0.f, rv = running_var ? running_var[c] : 0.f;
-    for (int g = 0; g < G; ++g) {
-        const double mu = sums[(size_t)g * 2 * C + c] / Mg;
-        double var = sums[(size_t)g * 2 * C + C + c] / Mg - mu * mu;
-        if (var < 0) var = 0;
-        mean[(size_t)g * C + c] = (float)mu;
-        rstd[(size_t)g * C + c] = (float)(1.0 / sqrt(var + (double)eps));
-        rm = (1.f - momentum) * rm + momentum * (float)mu;
-        const double unb = Mg > 1 ? var * Mg / (Mg - 1) : var;
-        rv = (1.f - momentum) * rv + momentum * (float)unb;
-    }
-    if (running_mean) {
-        running_mean[c] = rm;
-        running_var[c] = rv;
-    }
-}
-
 // y = act(gamma (z - mean) rstd + beta): row-walking like the backward apply kernel (parameters once per thread, 4 rows in flight)
-template <typename TO, bool GP = false>
+template <typename TO>
 __global__ void __launch_bounds__(256) bn_act_fwd_g_kernel(const float* __restrict__ z, const float* __restrict__ mean,
-                                                            const float* __restrict__ rstd, const float* __restrict__ gamma,
-                                                            const float* __restrict__ beta, int act, TO* __restrict__ y, int Mg,
+                                                            const float* __restrict__ rstd, int act, TO* __restrict__ y, int Mg,
                                                             int C, int rows_per_block, const __grid_constant__ MdvPtrTable gt, const __grid_constant__ MdvPtrTable bt) {
     MDV_PDL_SYNC();
     const int tpr = C >> 2, rpi = 256 / tpr;
     const int cl = threadIdx.x % tpr, rl = threadIdx.x / tpr;
     if (rl >= rpi) return;
     const int g = blockIdx.z, c = 4 * cl;
-    if (GP) {
-        gamma = (const float*)gt.p[g];
-        beta = (const float*)bt.p[g];
-    }
+    const float* __restrict__ gamma = (const float*)gt.p[g];
+    const float* __restrict__ beta = (const float*)bt.p[g];
     const int r0 = blockIdx.x * rows_per_block, r1e = min(Mg, r0 + rows_per_block);
     const size_t base = (size_t)g * Mg * C;
     const float4 mu = *reinterpret_cast<const float4*>(mean + (size_t)g * C + c), rs = *reinterpret_cast<const float4*>(rstd + (size_t)g * C + c);
@@ -587,9 +401,46 @@ __global__ void __launch_bounds__(256) bn_act_fwd_g_kernel(const float* __restri
     }
 }
 
-// coef[g][c] = sum_g / Mg, coef[g][C+c] = sum_gxhat / Mg;  dgamma += sum over groups of sum_gxhat; dbeta += ... sum_g
-__global__ void bn_bwd_finalize_g_kernel(const double* __restrict__ sums, int G, int Mg, int C, float* __restrict__ coef,
-                                         float* __restrict__ dgamma, float* __restrict__ dbeta) {
+// Train-mode statistics of G groups; group g updates the running buffers of table entry g (one nn.BatchNorm2d step).  The thread of
+// channel c walks the groups in order, so groups that name the same buffers update them in group order, exactly as consecutive
+// nn.BatchNorm2d forwards would (the momentum update does not commute).
+__global__ void bn_finalize_kernel(const double* __restrict__ sums, int G, int Mg, int C, float eps, float momentum, const __grid_constant__ MdvPtrTable rmt,
+                                      const __grid_constant__ MdvPtrTable rvt, const __grid_constant__ MdvPtrTable nbt, float* __restrict__ mean, float* __restrict__ rstd) {
+    MDV_PDL_SYNC();
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c == 0)
+        for (int g = 0; g < G; ++g)
+            if (nbt.p[g]) *(long long*)nbt.p[g] += 1;
+    if (c >= C) return;
+    float rm = 0.f, rv = 0.f;
+    for (int g = 0; g < G; ++g) {
+        const double mu = sums[(size_t)g * 2 * C + c] / Mg;
+        double var = sums[(size_t)g * 2 * C + C + c] / Mg - mu * mu;
+        if (var < 0) var = 0;
+        mean[(size_t)g * C + c] = (float)mu;
+        rstd[(size_t)g * C + c] = (float)(1.0 / sqrt(var + (double)eps));
+        // a run of consecutive groups naming the same buffer updates it in a register: one load and one store per run
+        float* rmp = (float*)rmt.p[g];
+        float* rvp = (float*)rvt.p[g];
+        if (rmp) {
+            if (g == 0 || rmt.p[g - 1] != rmp) rm = rmp[c];
+            rm = (1.f - momentum) * rm + momentum * (float)mu;
+            if (g + 1 == G || rmt.p[g + 1] != rmp) rmp[c] = rm;
+        }
+        if (rvp) {
+            if (g == 0 || rvt.p[g - 1] != rvp) rv = rvp[c];
+            const double unb = Mg > 1 ? var * Mg / (Mg - 1) : var;
+            rv = (1.f - momentum) * rv + momentum * (float)unb;
+            if (g + 1 == G || rvt.p[g + 1] != rvp) rvp[c] = rv;
+        }
+    }
+}
+
+// coef[g][c] = sum_g / Mg, coef[g][C+c] = sum_gxhat / Mg;  dgamma[g] += group g's sum_gxhat, dbeta[g] += its sum_g.  Consecutive
+// groups that name the same target are summed in double and added with one atomic: one set repeated G times gets the sum over
+// all groups added once.
+__global__ void bn_bwd_finalize_kernel(const double* __restrict__ sums, int G, int Mg, int C, float* __restrict__ coef,
+                                       const __grid_constant__ MdvPtrTable dgt, const __grid_constant__ MdvPtrTable dbt) {
     MDV_PDL_SYNC();
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= C) return;
@@ -600,58 +451,24 @@ __global__ void bn_bwd_finalize_g_kernel(const double* __restrict__ sums, int G,
         coef[(size_t)g * 2 * C + C + c] = (float)(b / Mg);
         sg += a;
         sq += b;
-    }
-    if (dbeta) atomicAdd(dbeta + c, (float)sg);
-    if (dgamma) atomicAdd(dgamma + c, (float)sq);
-}
-
-// per-group parameter sets: group g's statistics update only its own running buffers (one nn.BatchNorm2d step each)
-__global__ void bn_finalize_gp_kernel(const double* __restrict__ sums, int G, int Mg, int C, float eps, float momentum, const __grid_constant__ MdvPtrTable rmt,
-                                      const __grid_constant__ MdvPtrTable rvt, const __grid_constant__ MdvPtrTable nbt, float* __restrict__ mean, float* __restrict__ rstd) {
-    MDV_PDL_SYNC();
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c == 0)
-        for (int g = 0; g < G; ++g)
-            if (nbt.p[g]) *(long long*)nbt.p[g] += 1;
-    if (c >= C) return;
-    for (int g = 0; g < G; ++g) {
-        const double mu = sums[(size_t)g * 2 * C + c] / Mg;
-        double var = sums[(size_t)g * 2 * C + C + c] / Mg - mu * mu;
-        if (var < 0) var = 0;
-        mean[(size_t)g * C + c] = (float)mu;
-        rstd[(size_t)g * C + c] = (float)(1.0 / sqrt(var + (double)eps));
-        float* rm = (float*)rmt.p[g];
-        float* rv = (float*)rvt.p[g];
-        if (rm) rm[c] = (1.f - momentum) * rm[c] + momentum * (float)mu;
-        if (rv) {
-            const double unb = Mg > 1 ? var * Mg / (Mg - 1) : var;
-            rv[c] = (1.f - momentum) * rv[c] + momentum * (float)unb;
+        const bool last = g + 1 == G;
+        if (last || dbt.p[g + 1] != dbt.p[g]) {
+            if (dbt.p[g]) atomicAdd((float*)dbt.p[g] + c, (float)sg);
+            sg = 0.0;
         }
-    }
-}
-
-// coef as above; dgamma[g] += group g's sum_gxhat, dbeta[g] += its sum_g
-__global__ void bn_bwd_finalize_gp_kernel(const double* __restrict__ sums, int G, int Mg, int C, float* __restrict__ coef, const __grid_constant__ MdvPtrTable dgt,
-                                          const __grid_constant__ MdvPtrTable dbt) {
-    MDV_PDL_SYNC();
-    const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= C) return;
-    for (int g = 0; g < G; ++g) {
-        const double a = sums[(size_t)g * 2 * C + c], b = sums[(size_t)g * 2 * C + C + c];
-        coef[(size_t)g * 2 * C + c] = (float)(a / Mg);
-        coef[(size_t)g * 2 * C + C + c] = (float)(b / Mg);
-        if (dbt.p[g]) atomicAdd((float*)dbt.p[g] + c, (float)a);
-        if (dgt.p[g]) atomicAdd((float*)dgt.p[g] + c, (float)b);
+        if (last || dgt.p[g + 1] != dgt.p[g]) {
+            if (dgt.p[g]) atomicAdd((float*)dgt.p[g] + c, (float)sq);
+            sq = 0.0;
+        }
     }
 }
 
 // dz = gamma rstd (g - c0 - xhat c1), g = dy act'(.).  Same thread mapping as bn_reduce_g_kernel: a thread owns 4 channels and walks
 // the rows of its block's band, 4 rows in flight — the per-channel parameters (7 float4) are loaded once instead of once per 16
 // bytes of z, and there is no index arithmetic per element.
-template <typename TO, bool RANK1 = false, bool GP = false>
+template <typename TO, bool RANK1 = false>
 __global__ void __launch_bounds__(256) bn_bwd_apply_g_kernel(const float* __restrict__ dy, const float* __restrict__ z,
-                                                              const float* __restrict__ mean, const float* __restrict__ rstd,
-                                                              const float* __restrict__ gamma, const float* __restrict__ beta, int act,
+                                                              const float* __restrict__ mean, const float* __restrict__ rstd, int act,
                                                               const float* __restrict__ coef, TO* __restrict__ dz, int Mg, int C,
                                                               int rows_per_block, Rank1Dy r1, const __grid_constant__ MdvPtrTable gt, const __grid_constant__ MdvPtrTable bt) {
     MDV_PDL_SYNC();
@@ -660,10 +477,8 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_g_kernel(const float* __rest
     const int cl = threadIdx.x % tpr, rl = threadIdx.x / tpr;
     if (rl >= rpi) return;
     const int g = blockIdx.z;
-    if (GP) {
-        gamma = (const float*)gt.p[g];
-        beta = (const float*)bt.p[g];
-    }
+    const float* __restrict__ gamma = (const float*)gt.p[g];
+    const float* __restrict__ beta = (const float*)bt.p[g];
     const int r0 = blockIdx.x * rows_per_block, r1e = min(Mg, r0 + rows_per_block);
     const size_t base = (size_t)g * Mg * C;
     const int c = 4 * cl;
@@ -738,16 +553,6 @@ int apply_rows_per_block(int Mg, int C, int G) {
     return rpb;
 }
 
-int stats_rows_per_block(int M, int C) {
-    // aim at ~4 waves of 148 SMs
-    int col_blocks = mdv_cdiv(C, 32);
-    int want = (8 * MDV_NUM_SMS) / col_blocks;
-    if (want < 1) want = 1;
-    int rpb = mdv_cdiv(M, want);
-    if (rpb < 64) rpb = 64;
-    return rpb;
-}
-
 }  // namespace
 
 // Rows per warp iteration by width: C = 64 * NV.
@@ -763,15 +568,10 @@ int stats_rows_per_block(int M, int C) {
         default: X(8, 1)        \
     }
 
-static int ln_fwd_launch(bool gp, const float* x, const float* gamma, const float* beta, MdvPtrTable gt, MdvPtrTable bt, float eps,
-                         void* y_bf16, float* mean, float* rstd, int G, int Mg, int C, cudaStream_t st) {
+static int ln_fwd_launch(const float* x, MdvPtrTable gt, MdvPtrTable bt, float eps, void* y_bf16, float* mean, float* rstd, int G, int Mg,
+                         int C, cudaStream_t st) {
 #define MDV_LN_FWD(NV, R)                                                                                                        \
-    if (gp)                                                                                                                      \
-        mdv_launch((ln_fwd_kernel<NV, R, true>), dim3(mdv_cdiv(Mg, 8 * R), G), dim3(256), 0, st, x, gamma, beta, eps,           \
-                   (bf16*)y_bf16, mean, rstd, Mg, gt, bt);                                                                       \
-    else                                                                                                                         \
-        mdv_launch((ln_fwd_kernel<NV, R, false>), dim3(mdv_cdiv(Mg, 8 * R)), dim3(256), 0, st, x, gamma, beta, eps,             \
-                   (bf16*)y_bf16, mean, rstd, Mg, gt, bt);                                                                       \
+    mdv_launch((ln_fwd_kernel<NV, R>), dim3(mdv_cdiv(Mg, 8 * R), G), dim3(256), 0, st, x, gt, bt, eps, (bf16*)y_bf16, mean, rstd, Mg); \
     break;
     MDV_LN_DISPATCH(MDV_LN_FWD)
 #undef MDV_LN_FWD
@@ -779,24 +579,17 @@ static int ln_fwd_launch(bool gp, const float* x, const float* gamma, const floa
     return MDV_OK;
 }
 
-static int ln_bwd_launch(bool gp, const float* dy, const float* x, const float* mean, const float* rstd, const float* gamma, MdvPtrTable gt,
-                         const float* dres, float* dx, void* dx_masked_bf16, const float* rowscale, int rows_per_scale, float drop_p,
-                         const void* rng, uint32_t drop_stream, float* dgamma, float* dbeta, MdvPtrTable dgt, MdvPtrTable dbt,
-                         float* dbias_masked, int G, int Mg, int C, cudaStream_t st) {
+static int ln_bwd_launch(const float* dy, const float* x, const float* mean, const float* rstd, MdvPtrTable gt, const float* dres, float* dx,
+                         void* dx_masked_bf16, const float* rowscale, int rows_per_scale, float drop_p, const void* rng, uint32_t drop_stream,
+                         MdvPtrTable dgt, MdvPtrTable dbt, float* dbias_masked, int G, int Mg, int C, cudaStream_t st) {
     const int rps = rows_per_scale > 0 ? rows_per_scale : 1;
     const int max_blocks = (4 * MDV_NUM_SMS + G - 1) / G;      // ~4 blocks per SM over all groups
 #define MDV_LN_BWD(NV, R)                                                                                                        \
     {                                                                                                                            \
         int blocks = mdv_cdiv(Mg, 8 * R);                                                                                        \
         if (blocks > max_blocks) blocks = max_blocks;                                                                            \
-        if (gp)                                                                                                                  \
-            mdv_launch((ln_bwd_kernel<NV, R, true>), dim3(blocks, G), dim3(256), 0, st, dy, x, mean, rstd, gamma, dres, dx,     \
-                       (bf16*)dx_masked_bf16, rowscale, rps, drop_p, (const unsigned long long*)rng, drop_stream, dgamma, dbeta, \
-                       dbias_masked, Mg, gt, dgt, dbt);                                                                          \
-        else                                                                                                                     \
-            mdv_launch((ln_bwd_kernel<NV, R, false>), dim3(blocks), dim3(256), 0, st, dy, x, mean, rstd, gamma, dres, dx,       \
-                       (bf16*)dx_masked_bf16, rowscale, rps, drop_p, (const unsigned long long*)rng, drop_stream, dgamma, dbeta, \
-                       dbias_masked, Mg, gt, dgt, dbt);                                                                          \
+        mdv_launch((ln_bwd_kernel<NV, R>), dim3(blocks, G), dim3(256), 0, st, dy, x, mean, rstd, gt, dres, dx, (bf16*)dx_masked_bf16, \
+                   rowscale, rps, drop_p, (const unsigned long long*)rng, drop_stream, dgt, dbt, dbias_masked, Mg);              \
     }                                                                                                                            \
     break;
     MDV_LN_DISPATCH(MDV_LN_BWD)
@@ -805,19 +598,11 @@ static int ln_bwd_launch(bool gp, const float* dy, const float* x, const float* 
     return MDV_OK;
 }
 
-// Non-NULL entries p[0..G) of the given tables must be pairwise distinct (two groups writing one buffer would race).
-static bool tables_distinct(int G, std::initializer_list<const MdvPtrTable*> tabs) {
-    const void* seen[5 * MDV_MAX_GROUPS];
-    int n = 0;
-    for (const MdvPtrTable* t : tabs)
-        for (int g = 0; g < G; ++g) {
-            const void* q = t->p[g];
-            if (!q) continue;
-            for (int i = 0; i < n; ++i)
-                if (seen[i] == q) return false;
-            seen[n++] = q;
-        }
-    return true;
+// The table of the single-set entry points: one parameter set, G = 1.
+static MdvPtrTable one_set(const void* p) {
+    MdvPtrTable t = MdvPtrTable();
+    t.p[0] = const_cast<void*>(p);
+    return t;
 }
 
 static bool tables_set(int G, std::initializer_list<const MdvPtrTable*> tabs) {
@@ -832,14 +617,14 @@ static bool ln_shape_ok(int M, int C) { return M > 0 && !(C & 63) && C <= 64 * L
 extern "C" int mdv_layernorm_fwd(const float* x, const float* gamma, const float* beta, float eps, void* y_bf16, float* mean,
                                  float* rstd, int M, int C, void* stream) {
     if (!x || !y_bf16 || !gamma || !beta || !ln_shape_ok(M, C)) return MDV_ERR_ARG;
-    return ln_fwd_launch(false, x, gamma, beta, MdvPtrTable(), MdvPtrTable(), eps, y_bf16, mean, rstd, 1, M, C, (cudaStream_t)stream);
+    return ln_fwd_launch(x, one_set(gamma), one_set(beta), eps, y_bf16, mean, rstd, 1, M, C, (cudaStream_t)stream);
 }
 
 extern "C" int mdv_layernorm_fwd_gp(const float* x, MdvPtrTable gamma, MdvPtrTable beta, float eps, void* y_bf16, float* mean, float* rstd,
                                     int G, int Mg, int C, void* stream) {
     if (G < 1 || G > MDV_MAX_GROUPS || !x || !y_bf16 || !mean || !rstd || !ln_shape_ok(Mg, C)) return MDV_ERR_ARG;
     if (!tables_set(G, {&gamma, &beta}) || (long long)G * Mg >= 0x7fffffffLL) return MDV_ERR_ARG;
-    return ln_fwd_launch(true, x, nullptr, nullptr, gamma, beta, eps, y_bf16, mean, rstd, G, Mg, C, (cudaStream_t)stream);
+    return ln_fwd_launch(x, gamma, beta, eps, y_bf16, mean, rstd, G, Mg, C, (cudaStream_t)stream);
 }
 
 extern "C" int mdv_layernorm_bwd(const float* dy, const float* x, const float* mean, const float* rstd, const float* gamma,
@@ -848,8 +633,8 @@ extern "C" int mdv_layernorm_bwd(const float* dy, const float* x, const float* m
                                  float* dbeta, float* dbias_masked, int M, int C, void* stream) {
     if (!dy || !x || !dx || !gamma || !ln_shape_ok(M, C)) return MDV_ERR_ARG;
     if (dbias_masked && !dx_masked_bf16) return MDV_ERR_ARG;
-    return ln_bwd_launch(false, dy, x, mean, rstd, gamma, MdvPtrTable(), dres, dx, dx_masked_bf16, rowscale, rows_per_scale, drop_p, rng,
-                         drop_stream, dgamma, dbeta, MdvPtrTable(), MdvPtrTable(), dbias_masked, 1, M, C, (cudaStream_t)stream);
+    return ln_bwd_launch(dy, x, mean, rstd, one_set(gamma), dres, dx, dx_masked_bf16, rowscale, rows_per_scale, drop_p, rng, drop_stream,
+                         one_set(dgamma), one_set(dbeta), dbias_masked, 1, M, C, (cudaStream_t)stream);
 }
 
 extern "C" int mdv_layernorm_bwd_gp(const float* dy, const float* x, const float* mean, const float* rstd, MdvPtrTable gamma,
@@ -858,9 +643,26 @@ extern "C" int mdv_layernorm_bwd_gp(const float* dy, const float* x, const float
                                     float* dbias_masked, int G, int Mg, int C, void* stream) {
     if (G < 1 || G > MDV_MAX_GROUPS || !dy || !x || !mean || !rstd || !dx || !ln_shape_ok(Mg, C)) return MDV_ERR_ARG;
     if (dbias_masked && !dx_masked_bf16) return MDV_ERR_ARG;
-    if (!tables_set(G, {&gamma}) || !tables_distinct(G, {&dgamma, &dbeta}) || (long long)G * Mg >= 0x7fffffffLL) return MDV_ERR_ARG;
-    return ln_bwd_launch(true, dy, x, mean, rstd, nullptr, gamma, dres, dx, dx_masked_bf16, rowscale, rows_per_scale, drop_p, rng,
-                         drop_stream, nullptr, nullptr, dgamma, dbeta, dbias_masked, G, Mg, C, (cudaStream_t)stream);
+    if (!tables_set(G, {&gamma}) || (long long)G * Mg >= 0x7fffffffLL) return MDV_ERR_ARG;
+    return ln_bwd_launch(dy, x, mean, rstd, gamma, dres, dx, dx_masked_bf16, rowscale, rows_per_scale, drop_p, rng, drop_stream, dgamma, dbeta,
+                         dbias_masked, G, Mg, C, (cudaStream_t)stream);
+}
+
+// ---- train-mode BatchNorm (+activation): one call = G consecutive nn.BatchNorm2d forwards on [G*Mg, C]
+static bool bn_grouped_ok(int G, int Mg, int C) { return G >= 1 && Mg >= 1 && C >= 32 && C <= 1024 && (C & 3) == 0 && (long long)G * Mg * C < 0x7fffffffLL; }
+
+// Batch statistics of the G row groups -> mean/rstd [G, C]; updates the running buffers of the tables.  ws: 2*C*G doubles.
+static int bn_train_stats(const float* z, int G, int Mg, int C, float eps, float momentum, MdvPtrTable rmt, MdvPtrTable rvt, MdvPtrTable nbt,
+                          float* mean, float* rstd, void* ws, cudaStream_t st) {
+    cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C * G, st);
+    if (e != cudaSuccess) return (int)e;
+    const int rpb = grouped_rows_per_block(Mg, C, G);
+    mdv_launch(bn_reduce_g_kernel<false>, dim3(mdv_cdiv(Mg, rpb), 1, G), dim3(256), 0, st, (const float*)nullptr, z, (const float*)nullptr,
+               (const float*)nullptr, 0, (double*)ws, Mg, C, rpb, Rank1Dy(), MdvPtrTable(), MdvPtrTable());
+    MDV_CHECK_LAUNCH();
+    mdv_launch(bn_finalize_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)ws, G, Mg, C, eps, momentum, rmt, rvt, nbt, mean, rstd);
+    MDV_CHECK_LAUNCH();
+    return MDV_OK;
 }
 
 // ws: >= 2*C doubles (zeroed here).  Writes mean[C], rstd[C]; in training also updates the running buffers.
@@ -871,17 +673,13 @@ extern "C" int mdv_bn_stats(const float* z, int M, int C, float eps, float momen
     cudaStream_t st = (cudaStream_t)stream;
     if (training) {
         if (!z || !ws) return MDV_ERR_ARG;
-        cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C, st);
-        if (e != cudaSuccess) return (int)e;
-        const int rpb = stats_rows_per_block(M, C);
-        dim3 grid(mdv_cdiv(C, 32), mdv_cdiv(M, rpb));
-        mdv_launch(bn_stats_kernel, dim3(grid), dim3(256), 0, st, z, (double*)ws, M, C, rpb);
-        MDV_CHECK_LAUNCH();
-    } else if (!running_mean || !running_var) {
-        return MDV_ERR_ARG;
+        if (!bn_grouped_ok(1, M, C)) return MDV_ERR_UNSUPPORTED;
+        return bn_train_stats(z, 1, M, C, eps, momentum, one_set(running_mean), one_set(running_var), one_set(num_batches_tracked), mean, rstd,
+                              ws, st);
     }
-    mdv_launch(bn_finalize_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)ws, M, C, eps, momentum, training, running_mean,
-                                                         running_var, num_batches_tracked, mean, rstd);
+    if (!running_mean || !running_var) return MDV_ERR_ARG;
+    mdv_launch(bn_eval_stats_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const float*)running_mean, (const float*)running_var, eps, mean,
+               rstd, C);
     MDV_CHECK_LAUNCH();
     return MDV_OK;
 }
@@ -920,17 +718,58 @@ extern "C" int mdv_bn_act_fwd(const float* z, const float* mean, const float* rs
     return MDV_OK;
 }
 
-// ws: >= 2*C doubles + 2*C floats.  dz = d(loss)/dz for y = act(BN_train(z)); dgamma/dbeta accumulate.
-static int bn_act_bwd_impl(const float* dy, const Rank1Dy& r1, const float* z, const float* mean, const float* rstd, const float* gamma,
-                           const float* beta, int act, void* dz, int dz_bf16, float* dgamma, float* dbeta, int M, int C, void* ws,
-                           cudaStream_t st);
+// dz for y = act(BN_train(z)) on G row groups; dgamma/dbeta accumulate through the tables.  With a rank-1 output gradient (r1.dlog,
+// G == 1) the per-(sample, channel) factor wrow[c] * dropout2d mask is tabulated once.
+// ws: 2*C*G doubles of sums, 2*C*G floats of coefficients, then (rank-1) the (Mg / rps) x C factor table.
+static int bn_act_bwd_impl(const float* dy, const Rank1Dy& r1, const float* z, const float* mean, const float* rstd, MdvPtrTable gt,
+                           MdvPtrTable bt, int act, void* dz, int dz_bf16, MdvPtrTable dgt, MdvPtrTable dbt, int G, int Mg, int C, void* ws,
+                           cudaStream_t st) {
+    double* sums = (double*)ws;
+    float* coef = (float*)(sums + (size_t)2 * C * G);
+    cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C * G, st);
+    if (e != cudaSuccess) return (int)e;
+    Rank1Dy rt = r1;
+    if (r1.dlog) {
+        float* wtab = (float*)(sums + (size_t)3 * C * G);
+        const int samples = Mg / r1.rps;
+        rt.wtab = wtab;
+        mdv_launch(rank1_table_kernel, dim3(mdv_cdiv(samples * C / 4, 256)), dim3(256), 0, st, r1, wtab, samples, C);
+        MDV_CHECK_LAUNCH();
+    }
+    const int rpb = grouped_rows_per_block(Mg, C, G);
+    const dim3 rgrid(mdv_cdiv(Mg, rpb), 1, G);
+    if (r1.dlog)
+        mdv_launch((bn_reduce_g_kernel<true, true>), rgrid, dim3(256), 0, st, dy, z, mean, rstd, act, sums, Mg, C, rpb, rt, gt, bt);
+    else
+        mdv_launch(bn_reduce_g_kernel<true>, rgrid, dim3(256), 0, st, dy, z, mean, rstd, act, sums, Mg, C, rpb, rt, gt, bt);
+    MDV_CHECK_LAUNCH();
+    mdv_launch(bn_bwd_finalize_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)sums, G, Mg, C, coef, dgt, dbt);
+    MDV_CHECK_LAUNCH();
+    const int rpa = apply_rows_per_block(Mg, C, G);
+    const dim3 agrid(mdv_cdiv(Mg, rpa), 1, G);
+    if (dz_bf16 && r1.dlog)
+        mdv_launch((bn_bwd_apply_g_kernel<bf16, true>), agrid, dim3(256), 0, st, dy, z, mean, rstd, act, (const float*)coef, (bf16*)dz, Mg, C,
+                   rpa, rt, gt, bt);
+    else if (dz_bf16)
+        mdv_launch(bn_bwd_apply_g_kernel<bf16>, agrid, dim3(256), 0, st, dy, z, mean, rstd, act, (const float*)coef, (bf16*)dz, Mg, C, rpa, rt,
+                   gt, bt);
+    else if (r1.dlog)
+        mdv_launch((bn_bwd_apply_g_kernel<float, true>), agrid, dim3(256), 0, st, dy, z, mean, rstd, act, (const float*)coef, (float*)dz, Mg, C,
+                   rpa, rt, gt, bt);
+    else
+        mdv_launch(bn_bwd_apply_g_kernel<float>, agrid, dim3(256), 0, st, dy, z, mean, rstd, act, (const float*)coef, (float*)dz, Mg, C, rpa, rt,
+                   gt, bt);
+    MDV_CHECK_LAUNCH();
+    return MDV_OK;
+}
 
 extern "C" int mdv_bn_act_bwd(const float* dy, const float* z, const float* mean, const float* rstd, const float* gamma,
                               const float* beta, int act, void* dz, int dz_bf16, float* dgamma, float* dbeta, int M, int C,
                               void* ws, void* stream) {
-    if (!dy || !z || !dz || !ws || M <= 0 || (C & 3)) return MDV_ERR_ARG;
-    Rank1Dy r1 = {};
-    return bn_act_bwd_impl(dy, r1, z, mean, rstd, gamma, beta, act, dz, dz_bf16, dgamma, dbeta, M, C, ws, (cudaStream_t)stream);
+    if (!dy || !z || !mean || !rstd || !gamma || !beta || !dz || !ws || M <= 0 || (C & 3)) return MDV_ERR_ARG;
+    if (!bn_grouped_ok(1, M, C)) return MDV_ERR_UNSUPPORTED;
+    return bn_act_bwd_impl(dy, Rank1Dy(), z, mean, rstd, one_set(gamma), one_set(beta), act, dz, dz_bf16, one_set(dgamma), one_set(dbeta), 1, M,
+                           C, ws, (cudaStream_t)stream);
 }
 
 // Same, with the output gradient given in rank-1 form dy[m,c] = dlog[m] * wrow[c] * dropout2d_mask(m / rows_per_sample, c).
@@ -938,181 +777,38 @@ extern "C" int mdv_bn_act_bwd_rank1(const float* dlog, const float* wrow, int ro
                                     uint32_t drop_stream, const float* z, const float* mean, const float* rstd, const float* gamma,
                                     const float* beta, int act, void* dz, int dz_bf16, float* dgamma, float* dbeta, int M, int C,
                                     void* ws, void* stream) {
-    if (!dlog || !wrow || !z || !dz || !ws || M <= 0 || (C & 3) || rows_per_sample <= 0) return MDV_ERR_ARG;
-    if ((long long)M * C >= 0x7fffffffLL || (long long)(M / rows_per_sample + 1) * C >= 0x7fffffffLL) return MDV_ERR_UNSUPPORTED;
+    if (!dlog || !wrow || !z || !mean || !rstd || !gamma || !beta || !dz || !ws || M <= 0 || (C & 3) || rows_per_sample <= 0)
+        return MDV_ERR_ARG;
+    if (!bn_grouped_ok(1, M, C) || M % rows_per_sample || (long long)(M / rows_per_sample + 1) * C >= 0x7fffffffLL) return MDV_ERR_UNSUPPORTED;
     Rank1Dy r1 = {dlog, wrow, (const unsigned long long*)rng, rows_per_sample, drop_p, drop_stream, nullptr};
-    return bn_act_bwd_impl(nullptr, r1, z, mean, rstd, gamma, beta, act, dz, dz_bf16, dgamma, dbeta, M, C, ws, (cudaStream_t)stream);
-}
-
-static bool bn_grouped_ok(int G, int Mg, int C);
-
-static int bn_act_bwd_impl(const float* dy, const Rank1Dy& r1, const float* z, const float* mean, const float* rstd, const float* gamma,
-                           const float* beta, int act, void* dz, int dz_bf16, float* dgamma, float* dbeta, int M, int C, void* ws,
-                           cudaStream_t st) {
-    if (r1.dlog && bn_grouped_ok(1, M, C) && M % r1.rps == 0) {
-        // rank-1 output gradient through the float4 / 4-rows-in-flight kernels (one group); the per-(sample, channel) factor
-        // wrow[c] * dropout2d mask is tabulated once (ws: 3*C doubles + samples*C floats)
-        double* sums = (double*)ws;
-        float* coef = (float*)(sums + 2 * C);
-        float* wtab = (float*)(sums + 3 * C);
-        const int samples = M / r1.rps;
-        cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C, st);
-        if (e != cudaSuccess) return (int)e;
-        Rank1Dy rt = r1;
-        rt.wtab = wtab;
-        mdv_launch(rank1_table_kernel, dim3(mdv_cdiv(samples * C / 4, 256)), dim3(256), 0, st, r1, wtab, samples, C);
-        MDV_CHECK_LAUNCH();
-        const int rpb = grouped_rows_per_block(M, C, 1);
-        mdv_launch((bn_reduce_g_kernel<true, true>), dim3(mdv_cdiv(M, rpb), 1, 1), dim3(256), 0, st, (const float*)nullptr, z, mean, rstd, gamma, beta, act,
-                   sums, M, C, rpb, rt, MdvPtrTable(), MdvPtrTable());
-        MDV_CHECK_LAUNCH();
-        mdv_launch(bn_bwd_finalize_g_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)sums, 1, M, C, coef, dgamma, dbeta);
-        MDV_CHECK_LAUNCH();
-        const int rpa = apply_rows_per_block(M, C, 1);
-        if (dz_bf16)
-            mdv_launch((bn_bwd_apply_g_kernel<bf16, true>), dim3(mdv_cdiv(M, rpa), 1, 1), dim3(256), 0, st, (const float*)nullptr, z, mean, rstd, gamma, beta,
-                       act, (const float*)coef, (bf16*)dz, M, C, rpa, rt, MdvPtrTable(), MdvPtrTable());
-        else
-            mdv_launch((bn_bwd_apply_g_kernel<float, true>), dim3(mdv_cdiv(M, rpa), 1, 1), dim3(256), 0, st, (const float*)nullptr, z, mean, rstd, gamma, beta,
-                       act, (const float*)coef, (float*)dz, M, C, rpa, rt, MdvPtrTable(), MdvPtrTable());
-        MDV_CHECK_LAUNCH();
-        return MDV_OK;
-    }
-    double* sums = (double*)ws;
-    float* coef = (float*)(sums + 2 * C);
-    cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C, st);
-    if (e != cudaSuccess) return (int)e;
-    const int rpb = stats_rows_per_block(M, C);
-    dim3 grid(mdv_cdiv(C, 32), mdv_cdiv(M, rpb));
-    mdv_launch(bn_bwd_reduce_kernel, dim3(grid), dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, sums, M, C, rpb, r1);
-    MDV_CHECK_LAUNCH();
-    mdv_launch(bn_bwd_finalize_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, sums, M, C, coef, dgamma, dbeta);
-    MDV_CHECK_LAUNCH();
-    if ((long long)M * C >= 0x7fffffffLL) return MDV_ERR_UNSUPPORTED;
-    const int total = M * C;
-    const int blocks = mdv_cdiv(total / 4, 256);
-    if (dz_bf16)
-        mdv_launch(bn_bwd_apply_kernel<bf16>, dim3(blocks), dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, coef, (bf16*)dz, total, C, r1);
-    else
-        mdv_launch(bn_bwd_apply_kernel<float>, dim3(blocks), dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, coef, (float*)dz, total, C, r1);
-    MDV_CHECK_LAUNCH();
-    return MDV_OK;
-}
-
-// ---- grouped train-mode BatchNorm (+activation): one call = G consecutive nn.BatchNorm2d forwards on [G*Mg, C]
-static bool bn_grouped_ok(int G, int Mg, int C) { return G >= 1 && Mg >= 1 && C >= 32 && C <= 1024 && (C & 3) == 0 && (long long)G * Mg * C < 0x7fffffffLL; }
-
-// gp: per-group parameter sets (gamma/beta and the running buffers come from the tables, finalize updates group g's own buffers)
-static int bn_train_fwd_g_impl(bool gp, const float* z, int G, int Mg, int C, float eps, float momentum, float* running_mean,
-                               float* running_var, long long* num_batches_tracked, const float* gamma, const float* beta, MdvPtrTable rmt,
-                               MdvPtrTable rvt, MdvPtrTable nbt, MdvPtrTable gt, MdvPtrTable bt, int act, float* mean, float* rstd, void* y,
-                               int y_bf16, void* ws, cudaStream_t st) {
-    cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C * G, st);
-    if (e != cudaSuccess) return (int)e;
-    const int rpb = grouped_rows_per_block(Mg, C, G);
-    mdv_launch(bn_reduce_g_kernel<false>, dim3(mdv_cdiv(Mg, rpb), 1, G), dim3(256), 0, st, (const float*)nullptr, z, (const float*)nullptr,
-               (const float*)nullptr, (const float*)nullptr, (const float*)nullptr, 0, (double*)ws, Mg, C, rpb, Rank1Dy(), MdvPtrTable(),
-               MdvPtrTable());
-    MDV_CHECK_LAUNCH();
-    if (gp)
-        mdv_launch(bn_finalize_gp_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)ws, G, Mg, C, eps, momentum, rmt, rvt, nbt,
-                   mean, rstd);
-    else
-        mdv_launch(bn_finalize_g_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)ws, G, Mg, C, eps, momentum, running_mean,
-                   running_var, num_batches_tracked, mean, rstd);
-    MDV_CHECK_LAUNCH();
-    const int rpa = apply_rows_per_block(Mg, C, G);
-    const dim3 grid(mdv_cdiv(Mg, rpa), 1, G);
-    if (y_bf16 && gp)
-        mdv_launch(bn_act_fwd_g_kernel<bf16, true>, grid, dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, gamma, beta, act, (bf16*)y, Mg, C,
-                   rpa, gt, bt);
-    else if (y_bf16)
-        mdv_launch(bn_act_fwd_g_kernel<bf16>, grid, dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, gamma, beta, act, (bf16*)y, Mg, C, rpa,
-                   gt, bt);
-    else if (gp)
-        mdv_launch(bn_act_fwd_g_kernel<float, true>, grid, dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, gamma, beta, act, (float*)y, Mg,
-                   C, rpa, gt, bt);
-    else
-        mdv_launch(bn_act_fwd_g_kernel<float>, grid, dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, gamma, beta, act, (float*)y, Mg, C,
-                   rpa, gt, bt);
-    MDV_CHECK_LAUNCH();
-    return MDV_OK;
-}
-
-extern "C" int mdv_bn_train_fwd_grouped(const float* z, int G, int Mg, int C, float eps, float momentum, float* running_mean,
-                                        float* running_var, long long* num_batches_tracked, const float* gamma, const float* beta, int act,
-                                        float* mean, float* rstd, void* y, int y_bf16, void* ws, void* stream) {
-    if (!z || !gamma || !beta || !mean || !rstd || !y || !ws) return MDV_ERR_ARG;
-    if (!bn_grouped_ok(G, Mg, C)) return MDV_ERR_UNSUPPORTED;
-    const MdvPtrTable none = MdvPtrTable();
-    return bn_train_fwd_g_impl(false, z, G, Mg, C, eps, momentum, running_mean, running_var, num_batches_tracked, gamma, beta, none, none, none,
-                               none, none, act, mean, rstd, y, y_bf16, ws, (cudaStream_t)stream);
+    return bn_act_bwd_impl(nullptr, r1, z, mean, rstd, one_set(gamma), one_set(beta), act, dz, dz_bf16, one_set(dgamma), one_set(dbeta), 1, M, C,
+                           ws, (cudaStream_t)stream);
 }
 
 extern "C" int mdv_bn_train_fwd_gp(const float* z, int G, int Mg, int C, float eps, float momentum, MdvPtrTable running_mean,
                                    MdvPtrTable running_var, MdvPtrTable num_batches_tracked, MdvPtrTable gamma, MdvPtrTable beta, int act,
                                    float* mean, float* rstd, void* y, int y_bf16, void* ws, void* stream) {
     if (G < 1 || G > MDV_MAX_GROUPS || !z || !mean || !rstd || !y || !ws || !tables_set(G, {&gamma, &beta})) return MDV_ERR_ARG;
-    if (!tables_distinct(G, {&running_mean, &running_var, &num_batches_tracked})) return MDV_ERR_ARG;
     if (!bn_grouped_ok(G, Mg, C)) return MDV_ERR_UNSUPPORTED;
-    return bn_train_fwd_g_impl(true, z, G, Mg, C, eps, momentum, nullptr, nullptr, nullptr, nullptr, nullptr, running_mean, running_var,
-                               num_batches_tracked, gamma, beta, act, mean, rstd, y, y_bf16, ws, (cudaStream_t)stream);
-}
-
-static int bn_act_bwd_g_impl(bool gp, const float* dy, const float* z, const float* mean, const float* rstd, const float* gamma, const float* beta,
-                             MdvPtrTable gt, MdvPtrTable bt, int act, void* dz, int dz_bf16, float* dgamma, float* dbeta, MdvPtrTable dgt,
-                             MdvPtrTable dbt, int G, int Mg, int C, void* ws, cudaStream_t st) {
-    double* sums = (double*)ws;
-    float* coef = (float*)(sums + (size_t)2 * C * G);
-    cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C * G, st);
-    if (e != cudaSuccess) return (int)e;
-    const int rpb = grouped_rows_per_block(Mg, C, G);
-    const dim3 rgrid(mdv_cdiv(Mg, rpb), 1, G);
-    if (gp)
-        mdv_launch(bn_reduce_g_kernel<true, false, true>, rgrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, sums, Mg, C, rpb, Rank1Dy(),
-                   gt, bt);
-    else
-        mdv_launch(bn_reduce_g_kernel<true>, rgrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, sums, Mg, C, rpb, Rank1Dy(), gt, bt);
-    MDV_CHECK_LAUNCH();
-    if (gp)
-        mdv_launch(bn_bwd_finalize_gp_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)sums, G, Mg, C, coef, dgt, dbt);
-    else
-        mdv_launch(bn_bwd_finalize_g_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, st, (const double*)sums, G, Mg, C, coef, dgamma, dbeta);
-    MDV_CHECK_LAUNCH();
+    cudaStream_t st = (cudaStream_t)stream;
+    const int rc = bn_train_stats(z, G, Mg, C, eps, momentum, running_mean, running_var, num_batches_tracked, mean, rstd, ws, st);
+    if (rc != MDV_OK) return rc;
     const int rpa = apply_rows_per_block(Mg, C, G);
-    const dim3 agrid(mdv_cdiv(Mg, rpa), 1, G);
-    if (dz_bf16 && gp)
-        mdv_launch(bn_bwd_apply_g_kernel<bf16, false, true>, agrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, (const float*)coef,
-                   (bf16*)dz, Mg, C, rpa, Rank1Dy(), gt, bt);
-    else if (dz_bf16)
-        mdv_launch(bn_bwd_apply_g_kernel<bf16>, agrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, (const float*)coef, (bf16*)dz, Mg, C,
-                   rpa, Rank1Dy(), gt, bt);
-    else if (gp)
-        mdv_launch(bn_bwd_apply_g_kernel<float, false, true>, agrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, (const float*)coef,
-                   (float*)dz, Mg, C, rpa, Rank1Dy(), gt, bt);
+    const dim3 grid(mdv_cdiv(Mg, rpa), 1, G);
+    if (y_bf16)
+        mdv_launch(bn_act_fwd_g_kernel<bf16>, grid, dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, act, (bf16*)y, Mg, C, rpa, gamma,
+                   beta);
     else
-        mdv_launch(bn_bwd_apply_g_kernel<float>, agrid, dim3(256), 0, st, dy, z, mean, rstd, gamma, beta, act, (const float*)coef, (float*)dz, Mg, C,
-                   rpa, Rank1Dy(), gt, bt);
+        mdv_launch(bn_act_fwd_g_kernel<float>, grid, dim3(256), 0, st, z, (const float*)mean, (const float*)rstd, act, (float*)y, Mg, C, rpa, gamma,
+                   beta);
     MDV_CHECK_LAUNCH();
     return MDV_OK;
-}
-
-extern "C" int mdv_bn_act_bwd_grouped(const float* dy, const float* z, const float* mean, const float* rstd, const float* gamma,
-                                      const float* beta, int act, void* dz, int dz_bf16, float* dgamma, float* dbeta, int G, int Mg, int C,
-                                      void* ws, void* stream) {
-    if (!dy || !z || !mean || !rstd || !gamma || !beta || !dz || !ws) return MDV_ERR_ARG;
-    if (!bn_grouped_ok(G, Mg, C)) return MDV_ERR_UNSUPPORTED;
-    const MdvPtrTable none = MdvPtrTable();
-    return bn_act_bwd_g_impl(false, dy, z, mean, rstd, gamma, beta, none, none, act, dz, dz_bf16, dgamma, dbeta, none, none, G, Mg, C, ws,
-                             (cudaStream_t)stream);
 }
 
 extern "C" int mdv_bn_act_bwd_gp(const float* dy, const float* z, const float* mean, const float* rstd, MdvPtrTable gamma, MdvPtrTable beta,
                                  int act, void* dz, int dz_bf16, MdvPtrTable dgamma, MdvPtrTable dbeta, int G, int Mg, int C, void* ws,
                                  void* stream) {
     if (G < 1 || G > MDV_MAX_GROUPS || !dy || !z || !mean || !rstd || !dz || !ws || !tables_set(G, {&gamma, &beta})) return MDV_ERR_ARG;
-    if (!tables_distinct(G, {&dgamma, &dbeta})) return MDV_ERR_ARG;
     if (!bn_grouped_ok(G, Mg, C)) return MDV_ERR_UNSUPPORTED;
-    return bn_act_bwd_g_impl(true, dy, z, mean, rstd, nullptr, nullptr, gamma, beta, act, dz, dz_bf16, nullptr, nullptr, dgamma, dbeta, G, Mg, C,
-                             ws, (cudaStream_t)stream);
+    return bn_act_bwd_impl(dy, Rank1Dy(), z, mean, rstd, gamma, beta, act, dz, dz_bf16, dgamma, dbeta, G, Mg, C, ws, (cudaStream_t)stream);
 }

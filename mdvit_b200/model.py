@@ -32,13 +32,13 @@ def _pick(mods, d):
 
 
 def _norm_args(*norms):
-    """The norm arguments of an ops Function (see ops._bn_set).  Each of `norms` is one BatchNorm2d, or the list of the G sets the
-    row groups of a stacked pass use.  Returns group 0's (weight, bias) pairs, every group's running buffers group by group, and
-    groups 1..G-1's (weight, bias) pairs group by group (the Function's trailing arguments)."""
-    sets = [n if isinstance(n, list) else [n] for n in norms]
-    gb = [[t for s in sets for t in (s[g].weight, s[g].bias)] for g in range(len(sets[0]))]
-    bufs = tuple(t for g in range(len(gb)) for s in sets for t in (s[g].running_mean, s[g].running_var, s[g].num_batches_tracked))
-    return gb[0], bufs, tuple(t for pairs in gb[1:] for t in pairs)
+    """The (bufs, trailing norm arguments) of an ops norm Function (see ops._norm_slots).  Each of `norms` is one norm module, or
+    the list of the S modules the row groups of a stacked pass use.  Both are set-major, and within a set follow `norms`: the
+    (weight, bias) of every norm, and the running buffers of every BatchNorm."""
+    sets = list(zip(*(n if isinstance(n, list) else [n] for n in norms)))
+    params = tuple(t for s in sets for n in s for t in (n.weight, n.bias))
+    bufs = tuple(t for s in sets for n in s if isinstance(n, nn.BatchNorm2d) for t in (n.running_mean, n.running_var, n.num_batches_tracked))
+    return bufs, params
 
 
 # ----------------------------------------------------------------------------------------------- parameter containers
@@ -98,8 +98,8 @@ class DWCPatchEmbed(nn.Module):
 
     def forward(self, x, H, W, after_stem=False, d=None):
         pc = self.patch_conv
-        (g, b), bufs, gp = _norm_args(pc.norm(d))
-        y = ops.PatchEmbedFn.apply(x, pc.dwconv.weight, pc.pwconv.weight, g, b, bufs, H, W, pc.stride, self.training, after_stem, *gp)
+        bufs, norm = _norm_args(pc.norm(d))
+        y = ops.PatchEmbedFn.apply(x, pc.dwconv.weight, pc.pwconv.weight, bufs, H, W, pc.stride, self.training, after_stem, *norm)
         s = pc.stride
         return y, (H + 2 - 3) // s + 1, (W + 2 - 3) // s + 1
 
@@ -217,10 +217,7 @@ class SerialBlock_adapt(nn.Module):
         H, W = size
         norm1 = _pick(self.norm1s, d) if self.dsn else self.norm1
         norm2 = _pick(self.norm2s, d) if self.dsn else self.norm2
-        # one LayerNorm pair, or (stacked pass) the G per-domain pairs: groups 1..G-1 go to BlockFn as trailing arguments
-        n1, n2 = (norm1, norm2) if isinstance(norm1, list) else ([norm1], [norm2])
-        gp = tuple(t for a, b in zip(n1[1:], n2[1:]) for t in (a.weight, a.bias, b.weight, b.bias))
-        norm1, norm2 = n1[0], n2[0]
+        _, norm = _norm_args(norm1, norm2)
         att = self.factoratt_crpe
         # dispatch quirks of mdvit.py:350-353 preserved: Sup attention needs a label, plain attention rejects one
         use_label = domain_label is not None and (self.label_only_guard or self.adapt_method is not None)
@@ -231,15 +228,15 @@ class SerialBlock_adapt(nn.Module):
         dl = att.domain_layer
         da = (dl[0].weight, dl[0].bias, dl[2].weight, dl[2].bias) if dl is not None else (None, None, None, None)
         cl = att.crpe.conv_list
-        if not (isinstance(norm1, nn.LayerNorm) and abs(norm1.eps - 1e-6) < 1e-12):
+        n1 = self.norm1s[0] if self.dsn else self.norm1
+        if not (isinstance(n1, nn.LayerNorm) and abs(n1.eps - 1e-6) < 1e-12):
             raise ValueError("mdvit_b200 supports norm_layer=LayerNorm(eps=1e-6) (the reference default)")
         return ops.BlockFn.apply(
             x, domain_label if use_label else None, self.cpe.proj.weight, self.cpe.proj.bias,
             cl[0].weight, cl[0].bias, cl[1].weight, cl[1].bias, cl[2].weight, cl[2].bias,
-            norm1.weight, norm1.bias, att.qkv.weight, att.qkv.bias, att.proj.weight, att.proj.bias,
-            da[0], da[1], da[2], da[3], norm2.weight, norm2.bias,
+            att.qkv.weight, att.qkv.bias, att.proj.weight, att.proj.bias, da[0], da[1], da[2], da[3],
             self.mlp.fc1.weight, self.mlp.fc1.bias, self.mlp.fc2.weight, self.mlp.fc2.bias,
-            H, W, self.drop_rate, self.drop_path_rate, self.training, *gp)
+            H, W, self.drop_rate, self.drop_path_rate, self.training, *norm)
 
 
 class MHSA_stage_adapt(nn.Module):
@@ -271,9 +268,9 @@ class UnetDecodingBlockTransformer(nn.Module):
 
     def forward(self, x, h, w, skip, H, W, domain_label=None, d=None):
         ca = self.conv_after
-        (g, b), bufs, gp = _norm_args(ca.norm(d))
+        bufs, norm = _norm_args(ca.norm(d))
         out = ops.DecoderConvFn.apply(x, skip, self.conv_before.weight, self.conv_before.bias, ca.dwconv.weight, ca.pwconv.weight,
-                                      g, b, bufs, h, w, H, W, self.training, *gp)
+                                      bufs, h, w, H, W, self.training, *norm)
         return self.mhsa_block(out, H, W, domain_label, d)
 
 
@@ -444,8 +441,8 @@ class _Trunk(nn.Module):
             raise RuntimeError("mdvit_b200 runs on CUDA (sm_100a) only; there is no CPU path")
         c0, n0, c1, n1 = self._stem_parts(d)
         H, W = x.shape[2] // 4, x.shape[3] // 4
-        (g0, b0, g1, b1), bufs, gp = _norm_args(n0, n1)
-        t = ops.StemFn.apply(x, c0.weight, g0, b0, c1.weight, g1, b1, bufs, self.training, *gp)
+        bufs, norm = _norm_args(n0, n1)
+        t = ops.StemFn.apply(x, c0.weight, c1.weight, bufs, self.training, *norm)
         enc = []
         for idx in range(self.num_stages):
             t, H, W = self.patch_embed_stages[idx](t, H, W, after_stem=(idx == 0), d=d)
@@ -456,8 +453,8 @@ class _Trunk(nn.Module):
     def _bridge(self, enc, d=None):
         t3, H3, W3 = enc[3]
         c0, n0, c1, n1 = self._bridge_parts(d)
-        (g0, b0, g1, b1), bufs, gp = _norm_args(n0, n1)
-        return ops.BridgeFn.apply(t3, c0.weight, c0.bias, g0, b0, c1.weight, c1.bias, g1, b1, bufs, H3, W3, self.training, *gp)
+        bufs, norm = _norm_args(n0, n1)
+        return ops.BridgeFn.apply(t3, c0.weight, c0.bias, c1.weight, c1.bias, bufs, H3, W3, self.training, *norm)
 
     def _decode_from(self, out, enc, decoders, domain_label, d=None):
         h, w = enc[3][1], enc[3][2]

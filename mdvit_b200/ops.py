@@ -197,35 +197,29 @@ def cast_bf16(x, M, C, out=None, ld_in=None, ld_out=None, rowscale=None, rows_pe
 
 
 def layernorm_fwd(x, w, b, M, C, eps=1e-6):
-    """w, b: one parameter pair, or lists of G pairs (domain-specific norms: rows [g M/G, (g+1) M/G) use pair g)."""
+    """w, b: lists of S parameter tensors.  S = 1 normalises every row with the one set; with S > 1, rows [s M/S, (s+1) M/S)
+    use set s (domain-specific norms)."""
+    S = len(w)
+    if M % S:
+        raise ValueError("LayerNorm groups must divide the batch")
     y = torch.empty((M, C), dtype=BF16, device=x.device)
     mean = torch.empty(M, dtype=F32, device=x.device)
     rstd = torch.empty(M, dtype=F32, device=x.device)
-    if isinstance(w, list):
-        G = len(w)
-        check(L.lib().mdv_layernorm_fwd_gp(ptr(x), ptr_table(w), ptr_table(b), ctypes.c_float(eps), ptr(y), ptr(mean), ptr(rstd), G, M // G, C,
-                                           L.stream()), "mdv_layernorm_fwd_gp")
-        return y, mean, rstd
-    check(L.lib().mdv_layernorm_fwd(ptr(x), ptr(w), ptr(b), ctypes.c_float(eps), ptr(y), ptr(mean), ptr(rstd), M, C, L.stream()),
-          "mdv_layernorm_fwd")
+    check(L.lib().mdv_layernorm_fwd_gp(ptr(x), ptr_table(w), ptr_table(b), ctypes.c_float(eps), ptr(y), ptr(mean), ptr(rstd), S, M // S, C,
+                                       L.stream()), "mdv_layernorm_fwd_gp")
     return y, mean, rstd
 
 
 def layernorm_bwd(dy, x, mean, rstd, w, dres, M, C, dg, db, *, masked=False, rowscale=None, rows_per_scale=1, drop_p=0.0,
                   drop_stream=0, dbias_masked=None):
-    """w, dg, db: tensors, or lists of G (per-group parameter sets, as in layernorm_fwd; dg / db entries may be None)."""
+    """w, dg, db: lists of S, as in layernorm_fwd (dg / db entries may be None)."""
+    S = len(w)
     dx = torch.empty((M, C), dtype=F32, device=x.device)
     dxm = torch.empty((M, C), dtype=BF16, device=x.device) if masked else None
     rng = ptr(rng_tensor(x.device)) if drop_p > 0 else None
-    if isinstance(w, list):
-        G = len(w)
-        check(L.lib().mdv_layernorm_bwd_gp(ptr(dy), ptr(x), ptr(mean), ptr(rstd), ptr_table(w), ptr(dres), ptr(dx), ptr(dxm), ptr(rowscale),
-                                           rows_per_scale, ctypes.c_float(drop_p), rng, drop_stream, ptr_table(dg), ptr_table(db),
-                                           ptr(dbias_masked), G, M // G, C, L.stream()), "mdv_layernorm_bwd_gp")
-        return dx, dxm
-    check(L.lib().mdv_layernorm_bwd(ptr(dy), ptr(x), ptr(mean), ptr(rstd), ptr(w), ptr(dres), ptr(dx), ptr(dxm), ptr(rowscale),
-                                    rows_per_scale, ctypes.c_float(drop_p), rng, drop_stream, ptr(dg), ptr(db), ptr(dbias_masked), M, C,
-                                    L.stream()), "mdv_layernorm_bwd")
+    check(L.lib().mdv_layernorm_bwd_gp(ptr(dy), ptr(x), ptr(mean), ptr(rstd), ptr_table(w), ptr(dres), ptr(dx), ptr(dxm), ptr(rowscale),
+                                       rows_per_scale, ctypes.c_float(drop_p), rng, drop_stream, ptr_table(dg), ptr_table(db),
+                                       ptr(dbias_masked), S, M // S, C, L.stream()), "mdv_layernorm_bwd_gp")
     return dx, dxm
 
 
@@ -274,9 +268,18 @@ def current_bn_groups():
     return _BN_GROUPS
 
 
+def _one_set(*lists):
+    """The tensors of a single norm parameter set: the eval-mode paths take one set."""
+    if len(lists[0]) != 1:
+        raise ValueError("per-group norm sets are a train-mode path")
+    return [t[0] for t in lists]
+
+
 def bn_fold(weight, bias, running_mean, running_var, conv_bias=None, eps=1e-5):
     """Eval-mode BatchNorm as (scale, shift) for the epilogue of the GEMM that feeds it (gemm_nt(colscale=scale, bias=shift,
-    act=...)): the normalised tensor is produced by the GEMM itself, its fp32 pre-activation never reaches HBM."""
+    act=...)): the normalised tensor is produced by the GEMM itself, its fp32 pre-activation never reaches HBM.  The parameters and
+    buffers are one-element lists."""
+    weight, bias, running_mean, running_var = _one_set(weight, bias, running_mean, running_var)
     C = weight.numel()
     st = torch.empty((2, C), dtype=F32, device=weight.device)
     check(L.lib().mdv_bn_fold(ptr(weight), ptr(bias), ptr(running_mean), ptr(running_var), ptr(conv_bias), ctypes.c_float(eps), ptr(st[0]),
@@ -285,57 +288,50 @@ def bn_fold(weight, bias, running_mean, running_var, conv_bias=None, eps=1e-5):
 
 
 def bn_forward(z, M, C, weight, bias, running_mean, running_var, nbt, training, act, out_bf16, eps=1e-5, momentum=0.1):
-    """weight, bias and the three buffers are tensors, or lists of one per BatchNorm group (domain-specific norm sets: group g
-    normalises with set g and updates only its buffers)."""
+    """weight, bias and the three buffers: lists of S parameter sets.  In training each of the G = bn_groups() row groups is
+    normalised with its own batch statistics; with S = 1 the groups share the set (its buffers are updated group by group, in
+    order), with S = G group g uses set g and updates only its buffers.  Eval takes S = 1."""
     dev = z.device
-    G = _BN_GROUPS if training else 1
+    z = z.view(M, C)
+    y = torch.empty((M, C), dtype=BF16 if out_bf16 else F32, device=dev)
+    if not training:
+        weight, bias, running_mean, running_var = _one_set(weight, bias, running_mean, running_var)
+        mean = torch.empty((1, C), dtype=F32, device=dev)
+        rstd = torch.empty((1, C), dtype=F32, device=dev)
+        check(L.lib().mdv_bn_stats(ptr(z), M, C, ctypes.c_float(eps), ctypes.c_float(momentum), 0, ptr(running_mean), ptr(running_var), None,
+                                   ptr(mean), ptr(rstd), None, L.stream()), "mdv_bn_stats")
+        check(L.lib().mdv_bn_act_fwd(ptr(z), ptr(mean), ptr(rstd), ptr(weight), ptr(bias), act, ptr(y), int(out_bf16), M, C, L.stream()),
+              "mdv_bn_act_fwd")
+        return y, mean, rstd
+    G = _BN_GROUPS
     if M % G:
         raise ValueError("BatchNorm groups must divide the batch")
-    Mg = M // G
-    z = z.view(M, C)
+    if len(weight) not in (1, G):
+        raise ValueError("BatchNorm takes one parameter set, or one per bn_groups() group")
+    r = G // len(weight)      # table entries repeat a shared set once per group
     mean = torch.empty((G, C), dtype=F32, device=dev)
     rstd = torch.empty((G, C), dtype=F32, device=dev)
-    y = torch.empty((M, C), dtype=BF16 if out_bf16 else F32, device=dev)
-    if isinstance(weight, list):
-        if not training or len(weight) != G:
-            raise ValueError("per-group BatchNorm parameter sets need train mode and one set per bn_groups() group")
-        ws = torch.empty(2 * C * G, dtype=torch.float64, device=dev)
-        check(L.lib().mdv_bn_train_fwd_gp(ptr(z), G, Mg, C, ctypes.c_float(eps), ctypes.c_float(momentum), ptr_table(running_mean),
-                                          ptr_table(running_var), ptr_table(nbt), ptr_table(weight), ptr_table(bias), act, ptr(mean), ptr(rstd),
-                                          ptr(y), int(out_bf16), ptr(ws), L.stream()), "mdv_bn_train_fwd_gp")
-        return y, mean, rstd
-    if training:
-        ws = torch.empty(2 * C * G, dtype=torch.float64, device=dev)
-        check(L.lib().mdv_bn_train_fwd_grouped(ptr(z), G, Mg, C, ctypes.c_float(eps), ctypes.c_float(momentum), ptr(running_mean),
-                                               ptr(running_var), ptr(nbt), ptr(weight), ptr(bias), act, ptr(mean), ptr(rstd), ptr(y),
-                                               int(out_bf16), ptr(ws), L.stream()), "mdv_bn_train_fwd_grouped")
-        return y, mean, rstd
-    check(L.lib().mdv_bn_stats(ptr(z), M, C, ctypes.c_float(eps), ctypes.c_float(momentum), 0, ptr(running_mean), ptr(running_var), ptr(nbt),
-                               ptr(mean[0]), ptr(rstd[0]), None, L.stream()), "mdv_bn_stats")
-    check(L.lib().mdv_bn_act_fwd(ptr(z), ptr(mean[0]), ptr(rstd[0]), ptr(weight), ptr(bias), act, ptr(y), int(out_bf16), M, C, L.stream()),
-          "mdv_bn_act_fwd")
+    ws = torch.empty(2 * C * G, dtype=torch.float64, device=dev)
+    check(L.lib().mdv_bn_train_fwd_gp(ptr(z), G, M // G, C, ctypes.c_float(eps), ctypes.c_float(momentum), ptr_table(running_mean * r),
+                                      ptr_table(running_var * r), ptr_table(nbt * r), ptr_table(weight * r), ptr_table(bias * r), act, ptr(mean),
+                                      ptr(rstd), ptr(y), int(out_bf16), ptr(ws), L.stream()), "mdv_bn_train_fwd_gp")
     return y, mean, rstd
 
 
 def bn_backward(dy, z, mean, rstd, weight, bias, act, M, C, dz_bf16=True):
-    """Returns dz and the values to return from backward for (gamma, beta).  mean/rstd are [G, C]: one row per group."""
+    """Returns dz and the lists of values to return from backward for the S sets' gamma and beta (as given to bn_forward).
+    mean/rstd are [G, C]: one row per group."""
     dev = z.device
     G = mean.shape[0]
-    Mg = M // G
+    r = G // len(weight)
     dy, z = dy.view(M, C), z.view(M, C)
     dz = torch.empty((M, C), dtype=BF16 if dz_bf16 else F32, device=dev)
     ws = torch.empty(3 * C * G, dtype=torch.float64, device=dev)
-    if isinstance(weight, list):      # per-group parameter sets (see bn_forward): lists of gradient targets and return values
-        tg, tb = [gtarget(w) for w in weight], [gtarget(b) for b in bias]
-        check(L.lib().mdv_bn_act_bwd_gp(ptr(dy), ptr(z), ptr(mean), ptr(rstd), ptr_table(weight), ptr_table(bias), act, ptr(dz), int(dz_bf16),
-                                        ptr_table([t[0] for t in tg]), ptr_table([t[0] for t in tb]), G, Mg, C, ptr(ws), L.stream()),
-              "mdv_bn_act_bwd_gp")
-        return dz, [t[1] for t in tg], [t[1] for t in tb]
-    dg, rg = gtarget(weight)
-    db, rb = gtarget(bias)
-    check(L.lib().mdv_bn_act_bwd_grouped(ptr(dy), ptr(z), ptr(mean), ptr(rstd), ptr(weight), ptr(bias), act, ptr(dz), int(dz_bf16), ptr(dg),
-                                         ptr(db), G, Mg, C, ptr(ws), L.stream()), "mdv_bn_act_bwd_grouped")
-    return dz, rg, rb
+    tg, tb = [gtarget(w) for w in weight], [gtarget(b) for b in bias]
+    check(L.lib().mdv_bn_act_bwd_gp(ptr(dy), ptr(z), ptr(mean), ptr(rstd), ptr_table(weight * r), ptr_table(bias * r), act, ptr(dz),
+                                    int(dz_bf16), ptr_table([t[0] for t in tg] * r), ptr_table([t[0] for t in tb] * r), G, M // G, C, ptr(ws),
+                                    L.stream()), "mdv_bn_act_bwd_gp")
+    return dz, [t[1] for t in tg], [t[1] for t in tb]
 
 
 def upsample_fwd(x, out, B, Hi, Wi, Ho, Wo, C, ld_in=None, ld_out=None):
@@ -491,24 +487,20 @@ _FUSED_MLP = not bool(int(_os.environ.get("MDV_NO_FUSED_MLP", "0")))
 
 # ------------------------------------------------------------------------------------------------- SerialBlock
 class BlockFn(torch.autograd.Function):
-    """SerialBlock_adapt.forward (mdvit.py:346-361) incl. ConvPosEnc, FactorAtt_ConvRelPosEnc(_Sup) and Mlp."""
-
-    NP = 24  # number of parameter tensors passed after (x, label)
+    """SerialBlock_adapt.forward (mdvit.py:346-361) incl. ConvPosEnc, FactorAtt_ConvRelPosEnc(_Sup) and Mlp.  The trailing `norm`
+    arguments are norm1 and norm2 of S sets (see _norm_slots)."""
 
     @staticmethod
-    def forward(ctx, x, label, cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b,
-                da_w1, da_b1, da_w2, da_b2, n2w, n2b, fc1_w, fc1_b, fc2_w, fc2_b, H, W, drop, dpr, training, *gp):
+    def forward(ctx, x, label, cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, qkv_w, qkv_b, proj_w, proj_b,
+                da_w1, da_b1, da_w2, da_b2, fc1_w, fc1_b, fc2_w, fc2_b, H, W, drop, dpr, training, *norm):
         B, N, C = x.shape
         M, dev = B * N, x.device
         hidden = fc1_w.shape[0]
         x = _contig(x)
         lib = L.lib()
-        ctx.params = (cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b, da_w1, da_b1, da_w2, da_b2,
-                      n2w, n2b, fc1_w, fc1_b, fc2_w, fc2_b) + gp
-        if gp:      # per-group LayerNorm sets: gp = (n1w, n1b, n2w, n2b) of groups 1..G-1 (see _bn_set)
-            if M % (1 + len(gp) // 4):
-                raise ValueError("LayerNorm groups must divide the batch")
-            n1w, n1b, n2w, n2b = ([p] + list(gp[i::4]) for i, p in enumerate((n1w, n1b, n2w, n2b)))
+        ctx.params = (cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, qkv_w, qkv_b, proj_w, proj_b, da_w1, da_b1, da_w2, da_b2,
+                      fc1_w, fc1_b, fc2_w, fc2_b) + norm
+        (n1w, n1b), (n2w, n2b) = _norm_slots(norm, 2)
         with _dev_ctx(x):
             x1 = dwconv3(x, cpe_w, cpe_b, B, H, W, H, W, C, 1, residual=True)
             ln1, mean1, rstd1 = layernorm_fwd(x1, n1w, n1b, M, C)
@@ -569,22 +561,20 @@ class BlockFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dx3):
         (x, label, x1, mean1, rstd1, ln1, qkv, gate, hid, stats, y, x2, mean2, rstd2, ln2, u, hact, dp1, dp2, ecrpe) = ctx.saved_tensors
-        (cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b, da_w1, da_b1, da_w2, da_b2, n2w, n2b,
-         fc1_w, fc1_b, fc2_w, fc2_b) = ctx.params[:24]
-        gp = ctx.params[24:]
+        names = ("cpe_w", "cpe_b", "c3w", "c3b", "c5w", "c5b", "c7w", "c7b", "qkv_w", "qkv_b", "proj_w", "proj_b", "da_w1", "da_b1",
+                 "da_w2", "da_b2", "fc1_w", "fc1_b", "fc2_w", "fc2_b")
+        (cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, qkv_w, qkv_b, proj_w, proj_b, da_w1, da_b1, da_w2, da_b2,
+         fc1_w, fc1_b, fc2_w, fc2_b) = ctx.params[:20]
+        norm = ctx.params[20:]
         B, N, C, H, W, hidden, p_drop, sid, fused_mlp = ctx.meta
         M, dev = B * N, x.device
         lib = L.lib()
         dx3 = _contig(dx3.float())
-        T = {n: gtarget(p, da=n.startswith("da_")) for n, p in zip(("cpe_w", "cpe_b", "c3w", "c3b", "c5w", "c5b", "c7w", "c7b", "n1w", "n1b", "qkv_w", "qkv_b",
-                                            "proj_w", "proj_b", "da_w1", "da_b1", "da_w2", "da_b2", "n2w", "n2b", "fc1_w", "fc1_b",
-                                            "fc2_w", "fc2_b"), ctx.params)}
+        T = {n: gtarget(p, da=n.startswith("da_")) for n, p in zip(names, ctx.params)}
         G = {k: v[0] for k, v in T.items()}
-        TG = [gtarget(p) for p in gp]
-        if gp:      # per-group LayerNorm sets: lists over the groups of the parameters and of their gradient targets
-            n1w, n2w = [n1w] + list(gp[0::4]), [n2w] + list(gp[2::4])
-            for i, n in enumerate(("n1w", "n1b", "n2w", "n2b")):
-                G[n] = [G[n]] + [t[0] for t in TG[i::4]]
+        TN = [gtarget(p) for p in norm]
+        (n1w, _), (n2w, _) = _norm_slots(norm, 2)
+        (G["n1w"], G["n1b"]), (G["n2w"], G["n2b"]) = _norm_slots([t[0] for t in TN], 2)
         with _dev_ctx(x):
             # ---- MLP
             # bias gradients (column sums) are by-products of the kernels that produce each output gradient
@@ -630,9 +620,7 @@ class BlockFn(torch.autograd.Function):
             dx = dwconv3(dx1, cpe_w, None, B, H, W, H, W, C, 1, transposed=True, residual=True)
             dwconv3_wgrad(dx1, x, G["cpe_w"], G["cpe_b"], B, H, W, H, W, C, 1)
         _grads_done(ctx)
-        R = [T[n][1] for n in ("cpe_w", "cpe_b", "c3w", "c3b", "c5w", "c5b", "c7w", "c7b", "n1w", "n1b", "qkv_w", "qkv_b", "proj_w",
-                               "proj_b", "da_w1", "da_b1", "da_w2", "da_b2", "n2w", "n2b", "fc1_w", "fc1_b", "fc2_w", "fc2_b")]
-        return (dx.view(B, N, C), None, *R, None, None, None, None, None, *(t[1] for t in TG))
+        return (dx.view(B, N, C), None, *(T[n][1] for n in names), None, None, None, None, None, *(t[1] for t in TN))
 
 
 # ------------------------------------------------------------------------------------------------- conv pieces
@@ -640,40 +628,39 @@ def _bn_args(bn):
     return bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.num_batches_tracked
 
 
-# Domain-specific norm sets (model.MDViT_DSN.forward_multi): the norm Functions below take their norm parameters for row
-# group 0 as the usual positional arguments and those of groups 1..G-1, in the same order, group by group, as trailing
-# arguments `gp` (autograd only tracks direct tensor arguments); their `bufs` then hold every group's running buffers, group
-# by group.  With no trailing arguments they run the single-set kernels.
-def _bn_set(gb, bufs, k, nbn):
-    """(gamma, beta, running_mean, running_var, num_batches_tracked) of BatchNorm k of a Function with nbn BatchNorms: tensors with
-    one group, lists over the groups otherwise.  gb = every group's (gamma, beta) pairs, group by group; bufs likewise."""
-    G = len(gb) // (2 * nbn)
-    out = [[gb[g * 2 * nbn + 2 * k + i] for g in range(G)] for i in range(2)] + \
-          [[bufs[g * 3 * nbn + 3 * k + i] for g in range(G)] for i in range(3)]
-    return [v[0] for v in out] if G == 1 else out
+# The norm Functions below (and BlockFn) take the norm parameters of S sets as trailing tensor arguments `norm` (autograd only
+# tracks direct tensor arguments): set by set, and within a set the Function's k norm slots in order, each as (weight, bias).
+# Their `bufs` hold each set's running buffers in the same order, (running_mean, running_var, num_batches_tracked) per slot.
+# S = 1 is a plain module; S > 1 is the stacked pass of the domain-specific-norm models, where row group g uses set g
+# (model._norm_args builds both).
+def _norm_slots(norm, k, bufs=()):
+    """Per-slot lists over the S sets: k lists [weights, biases], extended by [running_means, running_vars, nbts] when bufs are
+    given."""
+    slots = [[list(norm[2 * j + i::2 * k]) for i in range(2)] for j in range(k)]
+    if bufs:
+        for j, sl in enumerate(slots):
+            sl += [list(bufs[3 * j + i::3 * k]) for i in range(3)]
+    return slots
 
 
-def _gp_grads(gp, rets):
-    """Gradients to return for the trailing norm arguments: rets = per-norm-slot lists over the groups (from bn_backward etc.)."""
-    if not gp:
-        return ()
-    k = len(rets)
-    return tuple(rets[j % k][1 + j // k] for j in range(len(gp)))
+def _norm_grads(*slots):
+    """The values backward returns for the trailing norm arguments: slots = each slot's (weight grads, bias grads) lists over the
+    sets, flattened in _norm_slots' order."""
+    return tuple(r for s in range(len(slots[0][0])) for gw, gb in slots for r in (gw[s], gb[s]))
 
 
 class StemFn(torch.autograd.Function):
     """stem = 2x (Conv3x3 s2 no-bias -> BN -> Hardswish), mdvit.py:509-526.  im2col (bf16) + tcgen05 GEMM."""
 
     @staticmethod
-    def forward(ctx, img, w0, g0, b0, w1, g1, b1, bufs, training, *gp):
+    def forward(ctx, img, w0, w1, bufs, training, *norm):
         B, _, H, W = img.shape
         dev = img.device
         img = _contig(img.float())
         H1, W1, H2, W2 = H // 2, W // 2, H // 4, W // 4
         M0, M1 = B * H1 * W1, B * H2 * W2
-        ctx.params = (w0, g0, b0, w1, g1, b1) + gp
-        g0, b0, rm0, rv0, nb0 = _bn_set(ctx.params[1:3] + ctx.params[4:6] + gp, bufs, 0, 2)
-        g1, b1, rm1, rv1, nb1 = _bn_set(ctx.params[1:3] + ctx.params[4:6] + gp, bufs, 1, 2)
+        ctx.params = (w0, w1) + norm
+        (g0, b0, rm0, rv0, nb0), (g1, b1, rm1, rv1, nb1) = _norm_slots(norm, 2, bufs)
         lib = L.lib()
         with _dev_ctx(img):
             # TF32 operands (fp32 in memory) for both stem convs: see mdv_gemm_nt_tf32
@@ -682,8 +669,6 @@ class StemFn(torch.autograd.Function):
             col1 = torch.empty((M1, 288), dtype=F32, device=dev)
             if not training:
                 # eval: BatchNorm (running statistics) + Hardswish folded into the GEMM epilogues
-                if gp:
-                    raise ValueError("per-group norm sets are a train-mode path")
                 a0, y = torch.empty((M0, 32), dtype=F32, device=dev), torch.empty((M1, 64), dtype=F32, device=dev)
                 s0, t0 = bn_fold(g0, b0, rm0, rv0)
                 gemm_nt(col0, prep_weight(w0, 2 | 8, 32, 27, ld=32, cin=3), M0, 32, 32, a0, tf32=True, colscale=s0, bias=t0, act=ACT_HSWISH)
@@ -701,7 +686,6 @@ class StemFn(torch.autograd.Function):
             gemm_nt(col1, prep_weight(w1, 2 | 8, 64, 288, cin=32), M1, 64, 288, z1, tf32=True)
             y, mean1, rstd1 = bn_forward(z1, M1, 64, g1, b1, rm1, rv1, nb1, training, ACT_HSWISH, False)
         ctx.save_for_backward(col0, z0, mean0, rstd0, col1, z1, mean1, rstd1)
-        ctx.sets = (g0, b0, g1, b1)
         ctx.meta = (B, H1, W1, H2, W2, training)
         _fwd_mark(ctx)
         ctx.set_materialize_grads(False)
@@ -709,15 +693,14 @@ class StemFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dy):
-        gp = ctx.params[6:]
         if dy is None:       # the da_only pass stops at the first patch embedding
-            return (None,) * (9 + len(gp))
+            return (None,) * (3 + len(ctx.params))
         B, H1, W1, H2, W2, training = ctx.meta
         if not training:
             raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
         col0, z0, mean0, rstd0, col1, z1, mean1, rstd1 = ctx.saved_tensors
-        w0, w1 = ctx.params[0], ctx.params[3]
-        g0, b0, g1, b1 = ctx.sets
+        w0, w1 = ctx.params[:2]
+        (g0, b0), (g1, b1) = _norm_slots(ctx.params[2:], 2)
         M0, M1, dev = B * H1 * W1, B * H2 * W2, dy.device
         lib = L.lib()
         dy = _contig(dy.float())
@@ -737,28 +720,24 @@ class StemFn(torch.autograd.Function):
                 gw0p = gemm_tn(dz0, cast_bf16(col0, M0, 32), M0, 32, 32, torch.zeros((32, 32), dtype=F32, device=dev))
                 check(lib.mdv_unperm_conv_grad(ptr(gw0p), 32, ptr(gw0), 32, 3, L.stream()), "mdv_unperm_conv_grad")
         _grads_done(ctx)
-        if gp:
-            return (None, rw0, rg0[0], rb0[0], rw1, rg1[0], rb1[0], None, None) + _gp_grads(gp, [rg0, rb0, rg1, rb1])
-        return None, rw0, rg0, rb0, rw1, rg1, rb1, None, None
+        return (None, rw0, rw1, None, None) + _norm_grads((rg0, rb0), (rg1, rb1))
 
 
 class PatchEmbedFn(torch.autograd.Function):
     """DWCPatchEmbed: depthwise 3x3 (stride s) -> 1x1 conv -> BN -> Hardswish, mdvit.py:114-123."""
 
     @staticmethod
-    def forward(ctx, x, dw_w, pw_w, g, b, bufs, Hi, Wi, stride, training, after_stem=False, *gp):
+    def forward(ctx, x, dw_w, pw_w, bufs, Hi, Wi, stride, training, after_stem, *norm):
         B, _, Cin = x.shape
         C = pw_w.shape[0]
         Ho, Wo = (Hi + 2 - 3) // stride + 1, (Wi + 2 - 3) // stride + 1
         M, dev = B * Ho * Wo, x.device
         x = _contig(x)
-        ctx.params = (dw_w, pw_w, g, b) + gp
-        g, b, rm, rv, nb = _bn_set((g, b) + gp, bufs, 0, 1)
+        ctx.params = (dw_w, pw_w) + norm
+        ((g, b, rm, rv, nb),) = _norm_slots(norm, 1, bufs)
         with _dev_ctx(x):
             t = dwconv3(x, dw_w, None, B, Hi, Wi, Ho, Wo, Cin, stride)          # fp32: TF32 operand of the pointwise conv
             if not training:      # eval: BatchNorm + Hardswish folded into the GEMM epilogue
-                if gp:
-                    raise ValueError("per-group norm sets are a train-mode path")
                 y = torch.empty((M, C), dtype=F32, device=dev)
                 sc, sh = bn_fold(g, b, rm, rv)
                 gemm_nt(t, _contig(pw_w).view(C, Cin), M, C, Cin, y, tf32=True, colscale=sc, bias=sh, act=ACT_HSWISH)
@@ -768,7 +747,6 @@ class PatchEmbedFn(torch.autograd.Function):
             gemm_nt(t, _contig(pw_w).view(C, Cin), M, C, Cin, z, tf32=True)
             y, mean, rstd = bn_forward(z, M, C, g, b, rm, rv, nb, training, ACT_HSWISH, False)
         ctx.save_for_backward(x, t, z, mean, rstd)
-        ctx.sets = (g, b)
         ctx.meta = (B, Hi, Wi, Ho, Wo, Cin, C, stride, training)
         _fwd_mark(ctx)
         ctx.after_stem = after_stem
@@ -781,11 +759,10 @@ class PatchEmbedFn(torch.autograd.Function):
             raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
         x, t, z, mean, rstd = ctx.saved_tensors
         dw_w, pw_w = ctx.params[:2]
-        g, b = ctx.sets
-        gp = ctx.params[4:]
+        ((g, b),) = _norm_slots(ctx.params[2:], 1)
         if ctx.after_stem and not wgrad_on():
             # nothing upstream of the first patch embedding owns a domain adapter: the da_only pass stops here
-            return (None,) * (11 + len(gp))
+            return (None,) * (7 + len(ctx.params))
         M, dev = B * Ho * Wo, dy.device
         dy = _contig(dy.float())
         with _dev_ctx(dy):
@@ -799,32 +776,26 @@ class PatchEmbedFn(torch.autograd.Function):
             g_dw, r_dw = gtarget(dw_w)
             dwconv3_wgrad(dt, x, g_dw, None, B, Hi, Wi, Ho, Wo, Cin, stride)
         _grads_done(ctx)
-        if gp:
-            return (dx.view(B, Hi * Wi, Cin), r_dw, r_pw, rg[0], rb[0], None, None, None, None, None, None) + _gp_grads(gp, [rg, rb])
-        return dx.view(B, Hi * Wi, Cin), r_dw, r_pw, rg, rb, None, None, None, None, None, None
+        return (dx.view(B, Hi * Wi, Cin), r_dw, r_pw, None, None, None, None, None, None) + _norm_grads((rg, rb))
 
 
 class BridgeFn(torch.autograd.Function):
     """bridge = 2x (Conv3x3 + bias -> BN -> ReLU), mdvit.py:557-564."""
 
     @staticmethod
-    def forward(ctx, x, w0, c0, g0, b0, w1, c1, g1, b1, bufs, H, W, training, *gp):
+    def forward(ctx, x, w0, c0, w1, c1, bufs, H, W, training, *norm):
         B, _, C = x.shape
         C0, C1 = w0.shape[0], w1.shape[0]
         M, dev = B * H * W, x.device
         x = _contig(x)
-        ctx.params = (w0, c0, g0, b0, w1, c1, g1, b1) + gp
-        gb = (g0, b0, g1, b1) + gp
-        g0, b0, rm0, rv0, nb0 = _bn_set(gb, bufs, 0, 2)
-        g1, b1, rm1, rv1, nb1 = _bn_set(gb, bufs, 1, 2)
+        ctx.params = (w0, c0, w1, c1) + norm
+        (g0, b0, rm0, rv0, nb0), (g1, b1, rm1, rv1, nb1) = _norm_slots(norm, 2, bufs)
         lib = L.lib()
         with _dev_ctx(x):
             col0 = torch.empty((M, 9 * C), dtype=F32, device=dev)
             check(lib.mdv_im2col3(ptr(x), 0, ptr(col0), 0, B, H, W, H, W, C, 1, 9 * C, L.stream()), "mdv_im2col3")
             col1 = torch.empty((M, 9 * C0), dtype=F32, device=dev)
             if not training:      # eval: conv bias + BatchNorm + ReLU folded into the GEMM epilogues
-                if gp:
-                    raise ValueError("per-group norm sets are a train-mode path")
                 a0, y = torch.empty((M, C0), dtype=F32, device=dev), torch.empty((M, C1), dtype=F32, device=dev)
                 s0, t0 = bn_fold(g0, b0, rm0, rv0, c0)
                 gemm_nt(col0, prep_weight(w0, 2 | 8, C0, 9 * C, cin=C), M, C0, 9 * C, a0, tf32=True, colscale=s0, bias=t0, act=ACT_RELU)
@@ -841,7 +812,6 @@ class BridgeFn(torch.autograd.Function):
             gemm_nt(col1, prep_weight(w1, 2 | 8, C1, 9 * C0, cin=C0), M, C1, 9 * C0, z1, bias=c1, tf32=True)
             y, mean1, rstd1 = bn_forward(z1, M, C1, g1, b1, rm1, rv1, nb1, training, ACT_RELU, False)
         ctx.save_for_backward(col0, z0, mean0, rstd0, col1, z1, mean1, rstd1)
-        ctx.sets = (g0, b0, g1, b1)
         ctx.meta = (B, H, W, C, C0, C1, training)
         _fwd_mark(ctx)
         return y.view(B, H * W, C1)
@@ -852,9 +822,8 @@ class BridgeFn(torch.autograd.Function):
         if not training:
             raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
         col0, z0, mean0, rstd0, col1, z1, mean1, rstd1 = ctx.saved_tensors
-        w0, c0, _, _, w1, c1 = ctx.params[:6]
-        g0, b0, g1, b1 = ctx.sets
-        gp = ctx.params[8:]
+        w0, c0, w1, c1 = ctx.params[:4]
+        (g0, b0), (g1, b1) = _norm_slots(ctx.params[4:], 2)
         M, dev = B * H * W, dy.device
         lib = L.lib()
         dy = _contig(dy.float())
@@ -878,10 +847,7 @@ class BridgeFn(torch.autograd.Function):
             dz0, rg0, rb0 = bn_backward(da0, z0, mean0, rstd0, g0, b0, ACT_RELU, M, C0)
             rw0, rc0, dx = conv_bwd(dz0, col0, w0, c0, C0, C)
         _grads_done(ctx)
-        if gp:
-            return ((dx.view(B, H * W, C), rw0, rc0, rg0[0], rb0[0], rw1, rc1, rg1[0], rb1[0], None, None, None, None)
-                    + _gp_grads(gp, [rg0, rb0, rg1, rb1]))
-        return dx.view(B, H * W, C), rw0, rc0, rg0, rb0, rw1, rc1, rg1, rb1, None, None, None, None
+        return (dx.view(B, H * W, C), rw0, rc0, rw1, rc1, None, None, None, None) + _norm_grads((rg0, rb0), (rg1, rb1))
 
 
 class DecoderConvFn(torch.autograd.Function):
@@ -889,13 +855,13 @@ class DecoderConvFn(torch.autograd.Function):
     grouped 3x3 (2 in/group) -> 1x1 -> BN -> Hardswish.  conv_before is commuted in front of the resize (exact)."""
 
     @staticmethod
-    def forward(ctx, inp, skip, cb_w, cb_b, dw_w, pw_w, g, b, bufs, h, w, H, W, training, *gp):
+    def forward(ctx, inp, skip, cb_w, cb_b, dw_w, pw_w, bufs, h, w, H, W, training, *norm):
         B, _, Cin = inp.shape
         C = cb_w.shape[0]
         m, M, dev = B * h * w, B * H * W, inp.device
         inp, skip = _contig(inp), _contig(skip)
-        ctx.params = (cb_w, cb_b, dw_w, pw_w, g, b) + gp
-        g, b, rm, rv, nb = _bn_set((g, b) + gp, bufs, 0, 1)
+        ctx.params = (cb_w, cb_b, dw_w, pw_w) + norm
+        ((g, b, rm, rv, nb),) = _norm_slots(norm, 1, bufs)
         lib = L.lib()
         with _dev_ctx(inp):
             # both 1x1 convs of the decoder trunk run on TF32 operands (fp32 in memory): see mdv_gemm_nt_tf32
@@ -905,8 +871,6 @@ class DecoderConvFn(torch.autograd.Function):
             gc = torch.empty((M, C), dtype=F32, device=dev)
             check(lib.mdv_gconv2_fwd(ptr(skip), ptr(up), ptr(dw_w), ptr(gc), 0, B, H, W, C, L.stream()), "mdv_gconv2_fwd")
             if not training:      # eval: BatchNorm + Hardswish folded into the GEMM epilogue
-                if gp:
-                    raise ValueError("per-group norm sets are a train-mode path")
                 y = torch.empty((M, C), dtype=F32, device=dev)
                 sc, sh = bn_fold(g, b, rm, rv)
                 gemm_nt(gc, _contig(pw_w).view(C, C), M, C, C, y, tf32=True, colscale=sc, bias=sh, act=ACT_HSWISH)
@@ -916,7 +880,6 @@ class DecoderConvFn(torch.autograd.Function):
             gemm_nt(gc, _contig(pw_w).view(C, C), M, C, C, z, tf32=True)
             y, mean, rstd = bn_forward(z, M, C, g, b, rm, rv, nb, training, ACT_HSWISH, False)
         ctx.save_for_backward(skip, inp, up, gc, z, mean, rstd)
-        ctx.sets = (g, b)
         ctx.meta = (B, h, w, H, W, Cin, C, training)
         _fwd_mark(ctx)
         return y.view(B, H * W, C)
@@ -928,8 +891,7 @@ class DecoderConvFn(torch.autograd.Function):
             raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
         skip, inp, up, gc, z, mean, rstd = ctx.saved_tensors
         cb_w, cb_b, dw_w, pw_w = ctx.params[:4]
-        g, b = ctx.sets
-        gp = ctx.params[6:]
+        ((g, b),) = _norm_slots(ctx.params[4:], 1)
         m, M, dev = B * h * w, B * H * W, dy.device
         lib = L.lib()
         dy = _contig(dy.float())
@@ -955,10 +917,8 @@ class DecoderConvFn(torch.autograd.Function):
             dinp = torch.empty((m, Cin), dtype=F32, device=dev)
             gemm_nt(dtb, prep_weight(cb_w, 1, C, Cin), m, Cin, C, dinp)
         _grads_done(ctx)
-        if gp:
-            return ((dinp.view(B, h * w, Cin), dskip.view(B, H * W, C), r_cb, r_cbb, r_dw, r_pw, rg[0], rb[0], None, None, None, None, None, None)
-                    + _gp_grads(gp, [rg, rb]))
-        return (dinp.view(B, h * w, Cin), dskip.view(B, H * W, C), r_cb, r_cbb, r_dw, r_pw, rg, rb, None, None, None, None, None, None)
+        return ((dinp.view(B, h * w, Cin), dskip.view(B, H * W, C), r_cb, r_cbb, r_dw, r_pw, None, None, None, None, None, None)
+                + _norm_grads((rg, rb)))
 
 
 def _sum_tokens(t, B, H, W, C):
@@ -990,7 +950,7 @@ class DeepLabFn(torch.autograd.Function):
 
         def bn(k, z, rows):
             rm, rv, nb = bufs[k]
-            y, mean, rstd = bn_forward(z, rows, Co, gs[k], bs[k], rm, rv, nb, training, ACT_RELU, False)
+            y, mean, rstd = bn_forward(z, rows, Co, [gs[k]], [bs[k]], [rm], [rv], [nb], training, ACT_RELU, False)
             saved[k] = (z, mean, rstd)
             return y
 
@@ -1045,7 +1005,7 @@ class DeepLabFn(torch.autograd.Function):
 
         def bn_bwd(k, d, rows):
             z, mean, rstd = flat[3 * k:3 * k + 3]
-            dz, rg, rb = bn_backward(d, z, mean, rstd, gs[k], bs[k], ACT_RELU, rows, Co)
+            dz, (rg,), (rb,) = bn_backward(d, z, mean, rstd, [gs[k]], [bs[k]], ACT_RELU, rows, Co)
             rets[3 * k + 1], rets[3 * k + 2] = rg, rb
             return dz
 
@@ -1190,7 +1150,7 @@ class DeiTBlockFn(torch.autograd.Function):
         x = _contig(x.float())
         lib = L.lib()
         with _dev_ctx(x):
-            ln1, mean1, rstd1 = layernorm_fwd(x, n1w, n1b, M, C, eps)
+            ln1, mean1, rstd1 = layernorm_fwd(x, [n1w], [n1b], M, C, eps)
             qkv = torch.empty((M, 3 * C), dtype=BF16, device=dev)
             gemm_nt(ln1, prep_weight(qkv_w, 0, 3 * C, C), M, 3 * C, C, qkv, bias=qkv_b)
             gate = hid = None
@@ -1206,7 +1166,7 @@ class DeiTBlockFn(torch.autograd.Function):
             check(lib.mdv_sdpa_fwd(ptr(qkv), ptr(gate), ptr(y), ptr(lse), B, N, C, heads, ctypes.c_float(scale), L.stream()), "mdv_sdpa_fwd")
             x2 = torch.empty((M, C), dtype=F32, device=dev)
             gemm_nt(y, prep_weight(proj_w, 0, C, C), M, C, C, x2, bias=proj_b, residual=x)
-            ln2, mean2, rstd2 = layernorm_fwd(x2, n2w, n2b, M, C, eps)
+            ln2, mean2, rstd2 = layernorm_fwd(x2, [n2w], [n2b], M, C, eps)
             u = torch.empty((M, hidden), dtype=BF16, device=dev)
             hact = torch.empty((M, hidden), dtype=BF16, device=dev)
             gemm_nt(ln2, prep_weight(fc1_w, 0, hidden, C), M, hidden, C, hact, bias=fc1_b, act=ACT_GELU, out_preact=u, preact_mode=1)
@@ -1238,7 +1198,8 @@ class DeiTBlockFn(torch.autograd.Function):
             gemm_tn(du, ln2, M, hidden, C, G["fc1_w"])
             dln2 = torch.empty((M, C), dtype=F32, device=dev)
             gemm_nt(du, prep_weight(P["fc1_w"], 1, hidden, C), M, C, hidden, dln2)
-            dx2, d_proj = layernorm_bwd(dln2, x2, mean2, rstd2, P["n2w"], dx3, M, C, G["n2w"], G["n2b"], masked=True, dbias_masked=G["proj_b"])
+            dx2, d_proj = layernorm_bwd(dln2, x2, mean2, rstd2, [P["n2w"]], dx3, M, C, [G["n2w"]], [G["n2b"]], masked=True,
+                                        dbias_masked=G["proj_b"])
             gemm_tn(d_proj, y, M, C, C, G["proj_w"])
             dy = torch.empty((M, C), dtype=BF16, device=dev)
             gemm_nt(d_proj, prep_weight(P["proj_w"], 1, C, C), M, C, C, dy)
@@ -1255,7 +1216,7 @@ class DeiTBlockFn(torch.autograd.Function):
             colsum(dqkv, M, 3 * C, G["qkv_b"])
             dln1 = torch.empty((M, C), dtype=F32, device=dev)
             gemm_nt(dqkv, prep_weight(P["qkv_w"], 1, 3 * C, C), M, C, 3 * C, dln1)
-            dx, _ = layernorm_bwd(dln1, x, mean1, rstd1, P["n1w"], dx2, M, C, G["n1w"], G["n1b"])
+            dx, _ = layernorm_bwd(dln1, x, mean1, rstd1, [P["n1w"]], dx2, M, C, [G["n1w"]], [G["n1b"]])
         _grads_done(ctx)
         return (dx.view(B, N, C), None, *[T[n][1] for n in names], None, None, None)
 
@@ -1306,7 +1267,7 @@ class LayerNormOutFn(torch.autograd.Function):
         B, N, C = x.shape
         x = _contig(x.float())
         with _dev_ctx(x):
-            y, mean, rstd = layernorm_fwd(x, w, b, B * N, C, eps)
+            y, mean, rstd = layernorm_fwd(x, [w], [b], B * N, C, eps)
         ctx.save_for_backward(x, mean, rstd)
         ctx.params = (w, b)
         _fwd_mark(ctx)
@@ -1321,7 +1282,7 @@ class LayerNormOutFn(torch.autograd.Function):
         with _dev_ctx(x):
             g_w, r_w = gtarget(w)
             g_b, r_b = gtarget(b)
-            dx, _ = layernorm_bwd(dy, x, mean, rstd, w, None, B * N, C, g_w, g_b)
+            dx, _ = layernorm_bwd(dy, x, mean, rstd, [w], None, B * N, C, [g_w], [g_b])
         _grads_done(ctx)
         return dx.view(B, N, C), r_w, r_b, None
 
@@ -1431,7 +1392,7 @@ class AuxFn(torch.autograd.Function):
                 acts.append(a)
                 ys.append((gemm_nt(a, cast_bf16(wps[i - 1], hc, Ci), Mi, hc, Ci, torch.empty((Mi, hc), dtype=F32, device=dev), bias=cb[i]), Hi, Wi))
             upsample_add(z, ys, B, H, W, hc)
-            a5, mean, rstd = bn_forward(z, M0, hc, g, b, rm, rv, nb, training, ACT_RELU, True)
+            a5, mean, rstd = bn_forward(z, M0, hc, [g], [b], [rm], [rv], [nb], training, ACT_RELU, True)
             p2 = drop2d if training else 0.0
             sid = new_stream_id() if p2 > 0 else 0
             lo = torch.empty(M0, dtype=F32, device=dev)
@@ -1729,9 +1690,9 @@ class ConvBnActFn(torch.autograd.Function):
                 rm, rv, nb = bufs
                 z = conv_out(bias=cbias)
                 if residual is None:
-                    y, mean, rstd = bn_forward(z, M, Cout, gamma, beta, rm, rv, nb, training, act, False)
+                    y, mean, rstd = bn_forward(z, M, Cout, [gamma], [beta], [rm], [rv], [nb], training, act, False)
                 else:
-                    t, mean, rstd = bn_forward(z, M, Cout, gamma, beta, rm, rv, nb, training, ACT_NONE, False)
+                    t, mean, rstd = bn_forward(z, M, Cout, [gamma], [beta], [rm], [rv], [nb], training, ACT_NONE, False)
                     y = torch.empty((M, Cout), dtype=F32, device=dev)
                     check(lib.mdv_add_act(ptr(t), ptr(_contig(residual)), ptr(y), M * Cout, act, L.stream()), "mdv_add_act")
         need_y = act == ACT_RELU and (residual is not None or not has_bn)
@@ -1776,7 +1737,7 @@ class ConvBnActFn(torch.autograd.Function):
                 if has_res:
                     dres = g.view(B, Ho * Wo, Cout)
                 if has_bn:
-                    dz, rg, rb = bn_backward(g, z, mean, rstd, gamma, beta, ACT_NONE if has_res else act, M, Cout)
+                    dz, (rg,), (rb,) = bn_backward(g, z, mean, rstd, [gamma], [beta], ACT_NONE if has_res else act, M, Cout)
                 else:
                     dz = cast_bf16(g, M, Cout)
                 gb, rcb = gtarget(cbias)
@@ -1840,7 +1801,7 @@ class BnActFn(torch.autograd.Function):
         x = _contig(x)
         rm, rv, nb = bufs
         with _dev_ctx(x):
-            y, mean, rstd = bn_forward(x.view(B * N, C), B * N, C, gamma, beta, rm, rv, nb, training, act, False)
+            y, mean, rstd = bn_forward(x.view(B * N, C), B * N, C, [gamma], [beta], [rm], [rv], [nb], training, act, False)
         ctx.save_for_backward(x, mean, rstd)
         ctx.params = (gamma, beta)
         ctx.meta = (B, N, C, act, training)
@@ -1856,7 +1817,7 @@ class BnActFn(torch.autograd.Function):
         gamma, beta = ctx.params
         dy = _contig(dy.float())
         with _dev_ctx(dy):
-            dx, rg, rb = bn_backward(dy, x, mean, rstd, gamma, beta, act, B * N, C, dz_bf16=False)
+            dx, (rg,), (rb,) = bn_backward(dy, x, mean, rstd, [gamma], [beta], act, B * N, C, dz_bf16=False)
         _grads_done(ctx)
         return dx.view(B, N, C), rg, rb, None, None, None
 

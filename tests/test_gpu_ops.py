@@ -296,9 +296,10 @@ def test_batchnorm_train_fwd_bwd_and_running_stats(env, M, C, act):
 
 @pytest.mark.parametrize("G,Mg,C,act,bf16_out", [(4, 512, 32, 3, False), (4, 1000, 64, 3, True), (1, 128, 1024, 2, False), (4, 3000, 320, 2, False),
                                                   (2, 4096, 512, 2, True), (4, 77, 128, 3, False)])
-def test_batchnorm_grouped_equals_consecutive_batchnorm_calls(env, G, Mg, C, act, bf16_out):
-    """mdv_bn_train_fwd_grouped / mdv_bn_act_bwd_grouped on G stacked mini-batches == G consecutive nn.BatchNorm2d forwards
-    (train mode: per-group batch statistics, running buffers updated in group order) and their autograd."""
+def test_batchnorm_shared_set_table_equals_consecutive_batchnorm_calls(env, G, Mg, C, act, bf16_out):
+    """mdv_bn_train_fwd_gp / mdv_bn_act_bwd_gp on G stacked mini-batches with tables that repeat one parameter set G times ==
+    G consecutive nn.BatchNorm2d forwards (train mode: per-group batch statistics, running buffers updated in group order,
+    num_batches_tracked += G) and their autograd (gradients summed over the groups)."""
     L, lib, dev = env
     torch.manual_seed(G * C + Mg)
     M = G * Mg
@@ -311,8 +312,9 @@ def test_batchnorm_grouped_equals_consecutive_batchnorm_calls(env, G, Mg, C, act
     mean, rstd = torch.empty(G, C, device=dev), torch.empty(G, C, device=dev)
     y = torch.empty(M, C, device=dev, dtype=torch.bfloat16 if bf16_out else torch.float32)
     ws = torch.empty(2 * C * G, dtype=torch.float64, device=dev)
-    L.check(lib.mdv_bn_train_fwd_grouped(L.ptr(z), G, Mg, C, 1e-5, 0.1, L.ptr(rm), L.ptr(rv), L.ptr(nbt), L.ptr(g), L.ptr(b), act, L.ptr(mean),
-                                         L.ptr(rstd), L.ptr(y), int(bf16_out), L.ptr(ws), L.stream()), "bn_g")
+    L.check(lib.mdv_bn_train_fwd_gp(L.ptr(z), G, Mg, C, 1e-5, 0.1, L.ptr_table([rm] * G), L.ptr_table([rv] * G), L.ptr_table([nbt] * G),
+                                    L.ptr_table([g] * G), L.ptr_table([b] * G), act, L.ptr(mean), L.ptr(rstd), L.ptr(y), int(bf16_out), L.ptr(ws),
+                                    L.stream()), "bn_g")
     actf = F.relu if act == 2 else F.hardswish
     ref = torch.cat([actf(F.batch_norm(z[i * Mg:(i + 1) * Mg], rm_ref, rv_ref, g, b, True, 0.1, 1e-5)) for i in range(G)])
     assert rel(y, ref) < (BF16_TOL if bf16_out else F32_TOL)
@@ -321,8 +323,8 @@ def test_batchnorm_grouped_equals_consecutive_batchnorm_calls(env, G, Mg, C, act
     (ref * dy).sum().backward()
     dz, dg, db = torch.empty(M, C, device=dev), torch.zeros(C, device=dev), torch.zeros(C, device=dev)
     ws2 = torch.empty(3 * C * G, dtype=torch.float64, device=dev)
-    L.check(lib.mdv_bn_act_bwd_grouped(L.ptr(dy), L.ptr(z), L.ptr(mean), L.ptr(rstd), L.ptr(g), L.ptr(b), act, L.ptr(dz), 0, L.ptr(dg), L.ptr(db),
-                                       G, Mg, C, L.ptr(ws2), L.stream()), "bn_bwd_g")
+    L.check(lib.mdv_bn_act_bwd_gp(L.ptr(dy), L.ptr(z), L.ptr(mean), L.ptr(rstd), L.ptr_table([g] * G), L.ptr_table([b] * G), act, L.ptr(dz), 0,
+                                  L.ptr_table([dg] * G), L.ptr_table([db] * G), G, Mg, C, L.ptr(ws2), L.stream()), "bn_bwd_g")
     assert rel(dz, z.grad) < 1e-3 and rel(dg, g.grad) < 1e-3 and rel(db, b.grad) < 1e-3
 
 
