@@ -70,6 +70,15 @@ int mdv_gemm_nt(const void* A, int lda, const void* W, int ldw, int M, int N, in
  * section 7); the transformer blocks' GEMMs, whose outputs are small additive branches, stay bf16. */
 int mdv_gemm_nt_tf32(const float* A, int lda, const float* W, int ldw, int M, int N, int K, const MdvGemmEpi* epi, void* stream);
 
+/* mdv_gemm_nt_tf32 with one folded eval-mode BatchNorm set per SAMPLE (mixed-domain inference of the domain-specific-norm
+ * models): epi->colscale and epi->bias are [S, N] tables, and row m uses row s = sample_set[m / rows_per_sample] of both,
+ *   v = acc * colscale[s*N + n] + bias[s*N + n],  then the activation and the rest of the epilogue as above.
+ * sample_set is a DEVICE int32 vector read by the kernel, so a captured CUDA graph serves any domain mix.  A row whose index is
+ * outside [0, S) reads no table entry and is written as NaN.  S outside 1..8, rows_per_sample < 1, or a NULL sample_set /
+ * colscale returns MDV_ERR_ARG before any CUDA call. */
+int mdv_gemm_nt_tf32_sets(const float* A, int lda, const float* W, int ldw, int M, int N, int K, const MdvGemmEpi* epi,
+                          const int* sample_set, int rows_per_sample, int S, void* stream);
+
 /* 3x3 / stride 1 / padding 1 convolution of an NHWC activation as ONE implicit GEMM (no im2col matrix): the A tiles of the K = 9*Cin
  * reduction are fetched straight from x [B,H,W,Cin] (pixel pitch ldx) by 4-D TMA boxes, whose out-of-range zero fill is the padding:
  *   out[(b,y,x), n] = epi( sum_{tap=(i,j), c} x[b, y + s(i-1), x + s(j-1), c] . Wm[n, tap*Cin + c] ),   s = flip ? -1 : +1.
@@ -143,6 +152,12 @@ typedef struct MdvPtrTable {
  * sums over group g only and may each be NULL; dbias_masked (a shared bias) is one [C] sum over all rows. */
 int mdv_layernorm_fwd_gp(const float* x, MdvPtrTable gamma, MdvPtrTable beta, float eps, void* y_bf16, float* mean, float* rstd,
                          int G, int Mg, int C, void* stream);
+/* mdv_layernorm_fwd with one parameter set per SAMPLE (mixed-domain inference): row m uses gamma[s], beta[s] with
+ * s = sample_set[m / rows_per_sample], read on the device (DEVICE int32 vector).  A row whose index is outside [0, S) reads no
+ * table entry and is written as NaN.  mean / rstd may be NULL (inference needs neither).  1 <= S <= 8, a gamma / beta for every
+ * set, rows_per_sample >= 1 and a non-NULL sample_set, else MDV_ERR_ARG before any CUDA call. */
+int mdv_layernorm_fwd_sets(const float* x, MdvPtrTable gamma, MdvPtrTable beta, float eps, void* y_bf16, float* mean, float* rstd,
+                           const int* sample_set, int rows_per_sample, int S, int M, int C, void* stream);
 int mdv_layernorm_bwd_gp(const float* dy, const float* x, const float* mean, const float* rstd, MdvPtrTable gamma,
                          const float* dres, float* dx, void* dx_masked_bf16, const float* rowscale, int rows_per_scale,
                          float drop_p, const void* rng, uint32_t drop_stream, MdvPtrTable dgamma, MdvPtrTable dbeta,
@@ -169,6 +184,11 @@ int mdv_bn_stats(const float* z, int M, int C, float eps, float momentum, int tr
  * scale[c] = gamma[c] / sqrt(running_var[c] + eps);  shift[c] = beta[c] + (conv_bias[c] - running_mean[c]) * scale[c]. */
 int mdv_bn_fold(const float* gamma, const float* beta, const float* running_mean, const float* running_var, const float* conv_bias,
                 float eps, float* scale, float* shift, int C, void* stream);
+/* mdv_bn_fold for S parameter sets in one launch: scale / shift are [S, C], row s from gamma[s], beta[s], running_mean[s],
+ * running_var[s]; conv_bias ([C] or NULL) is shared by all sets.  mdv_bn_fold is the S = 1 call.  1 <= S <= 8 and every table
+ * entry set, else MDV_ERR_ARG before any CUDA call. */
+int mdv_bn_fold_sets(MdvPtrTable gamma, MdvPtrTable beta, MdvPtrTable running_mean, MdvPtrTable running_var, const float* conv_bias,
+                     float eps, float* scale, float* shift, int S, int C, void* stream);
 int mdv_bn_act_fwd(const float* z, const float* mean, const float* rstd, const float* gamma, const float* beta, int act,
                    void* y, int y_bf16, int M, int C, void* stream);
 /* dz for y = act(BN_train(z)); ws >= 2*C doubles + 2*C floats; dgamma/dbeta accumulate.  mdv_bn_act_bwd_gp with G = 1:

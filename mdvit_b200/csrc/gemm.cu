@@ -52,6 +52,10 @@ struct GemmParams {
     // NT only, implicit-GEMM 3x3 convolution (mdv_conv3_gemm): A is an NHWC activation read through a 4-D tensor map; k-block kc
     // belongs to tap kc / conv_cin and channels kc % conv_cin.., and its A tile is the output tile's pixels shifted by that tap
     int conv_cin, conv_w, conv_hw, conv_flip;
+    // NT only, per-sample norm sets (mdv_gemm_nt_tf32_sets): epi.colscale / epi.bias are [nsets, N] tables and row m uses
+    // table row sample_set[m / rows_per_sample]; NULL = the plain [N] vectors
+    const int* sample_set;
+    int rows_per_sample, nsets;
     MdvGemmEpi epi;
 };
 
@@ -335,11 +339,21 @@ __global__ void __launch_bounds__(32 * (4 + NEPI), 1)
                 float f[32];
 #pragma unroll
                 for (int j = 0; j < 32; ++j) f[j] = __uint_as_float(v[j]);
+                int sset = 0;
                 if (!LIGHT && e.colscale) {
                     // eval-mode BatchNorm folded into the GEMM: v = acc * scale[n] + shift[n] (shift arrives as `bias`)
+                    // per-sample norm sets: this row's table row; an index outside [0, nsets) reads no table row (set 0 stands
+                    // in) and the row is stored as NaN
+                    if (p.sample_set && row_ok) {
+                        sset = __ldg(p.sample_set + row / p.rows_per_sample);
+                        if ((unsigned)sset >= (unsigned)p.nsets) sset = -1;
+                    }
+                    const int soff = sset > 0 ? sset * p.N : 0;
+                    const float* const sc_p = e.colscale + soff;
+                    const float* const sh_p = e.bias ? e.bias + soff : nullptr;
 #pragma unroll
                     for (int j = 0; j < 32; ++j)
-                        if (col0 + j < p.N) f[j] = fmaf(f[j], __ldg(e.colscale + col0 + j), e.bias ? __ldg(e.bias + col0 + j) : 0.f);
+                        if (col0 + j < p.N) f[j] = fmaf(f[j], __ldg(sc_p + col0 + j), sh_p ? __ldg(sh_p + col0 + j) : 0.f);
                 } else if (bias_p) {
 #pragma unroll
                     for (int j = 0; j < 32; j += 4) {
@@ -465,6 +479,10 @@ __global__ void __launch_bounds__(32 * (4 + NEPI), 1)
                         }
                     }
                 }
+                if (!LIGHT && sset < 0) {
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) f[j] = __int_as_float(0x7fffffff);      // out-of-range set index (after the
+                }                                                                      // activation: ReLU would drop a NaN)
                 if (colsum_p && !row_ok) {
 #pragma unroll
                     for (int j = 0; j < 32; ++j) f[j] = 0.f;      // rows past M are clipped by the TMA store; keep them out of the sums
@@ -669,14 +687,22 @@ struct ConvGeom {      // implicit 3x3 convolution mode of gemm_nt_impl (mdv_con
     int B, H, W, Cin, flip;
 };
 
+struct SampleSets {      // per-sample norm sets of mdv_gemm_nt_tf32_sets
+    const int* idx;
+    int rows_per_sample, S;
+};
+
 static int gemm_nt_impl(const void* A, int lda, const void* W, int ldw, int M, int N, int K, const MdvGemmEpi* epi, int tf32, void* stream,
-                        const ConvGeom* cv = nullptr) {
+                        const ConvGeom* cv = nullptr, const SampleSets* sets = nullptr) {
     if (!A || !W || !epi || !epi->out || M <= 0 || N <= 0 || K <= 0) return MDV_ERR_ARG;
     if ((N & 3) || (K & (tf32 ? 3 : 7)) || epi->accumulate) return MDV_ERR_ARG;
     GemmParams p = {};
     p.M = M; p.N = N; p.K = K;
     if (cv) {
         p.conv_cin = cv->Cin; p.conv_w = cv->W; p.conv_hw = cv->H * cv->W; p.conv_flip = cv->flip;
+    }
+    if (sets) {
+        p.sample_set = sets->idx; p.rows_per_sample = sets->rows_per_sample; p.nsets = sets->S;
     }
     p.epi = *epi;
     p.tf32 = tf32;
@@ -724,6 +750,13 @@ extern "C" int mdv_gemm_nt(const void* A, int lda, const void* W, int ldw, int M
 extern "C" int mdv_gemm_nt_tf32(const float* A, int lda, const float* W, int ldw, int M, int N, int K, const MdvGemmEpi* epi,
                                 void* stream) {
     return gemm_nt_impl(A, lda, W, ldw, M, N, K, epi, 1, stream);
+}
+
+extern "C" int mdv_gemm_nt_tf32_sets(const float* A, int lda, const float* W, int ldw, int M, int N, int K, const MdvGemmEpi* epi,
+                                     const int* sample_set, int rows_per_sample, int S, void* stream) {
+    if (!epi || !epi->colscale || !sample_set || rows_per_sample < 1 || S < 1 || S > MDV_MAX_GROUPS) return MDV_ERR_ARG;
+    const SampleSets sets = {sample_set, rows_per_sample, S};
+    return gemm_nt_impl(A, lda, W, ldw, M, N, K, epi, 1, stream, nullptr, &sets);
 }
 
 // out[(b,y,x), n] = epi( sum_{tap=(i,j), c} x[b, y + s(i-1), x + s(j-1), c] . Wm[n, tap*Cin + c] ),  s = flip ? -1 : +1, zero outside

@@ -13,17 +13,18 @@ constexpr int LN_MAXV = 8;  // float2 per lane -> C <= 512
 // ---------------------------------------------------------------------------------- LayerNorm forward
 // one warp owns R rows per iteration (all loads issued before any arithmetic: at C = 64 a row is only 256 B, and one
 // row per warp leaves HBM latency exposed); a row lives in registers, NV float2 per lane.
-// blockIdx.y is the row group (M rows); its gamma / beta are gtab.p[blockIdx.y] / btab.p[blockIdx.y].
+// blockIdx.y is the row group (M rows); its gamma / beta are gtab.p[blockIdx.y] / btab.p[blockIdx.y].  With a sample_set
+// (per-sample sets, one group) row `row` uses gtab.p[s] / btab.p[s], s = sample_set[row / rows_per_sample]; an s outside
+// [0, nsets) reads no table entry and the row is written as NaN.  mean_out / rstd_out may be NULL.
 template <int NV, int R>
 __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x, const __grid_constant__ MdvPtrTable gtab,
                                                       const __grid_constant__ MdvPtrTable btab, float eps, bf16* __restrict__ y,
-                                                      float* __restrict__ mean_out, float* __restrict__ rstd_out, int M) {
+                                                      float* __restrict__ mean_out, float* __restrict__ rstd_out, int M,
+                                                      const int* __restrict__ sample_set, int rows_per_sample, int nsets) {
     MDV_PDL_SYNC();
     constexpr int C = NV * 64;
     const int lane = threadIdx.x & 31;
     const int lo = blockIdx.y * M, hi = lo + M;
-    const float* __restrict__ gamma = (const float*)gtab.p[blockIdx.y];
-    const float* __restrict__ beta = (const float*)btab.p[blockIdx.y];
     const int row0 = lo + (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * R;
     if (row0 >= hi) return;
     float2 v[R][NV];
@@ -34,16 +35,34 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x
 #pragma unroll
         for (int i = 0; i < NV; ++i) v[r][i] = *reinterpret_cast<const float2*>(xr + i * 64 + lane * 2);
     }
+    // the set of the parameters in g / b: the row group, or (per-sample sets) the set of the warp's first row; a row of
+    // another sample reloads them (-1: an out-of-range index, whose row reads no table entry)
+    auto set_of = [&](int row) {
+        const int k = __ldg(sample_set + row / rows_per_sample);
+        return (unsigned)k < (unsigned)nsets ? k : -1;
+    };
+    int kcur = sample_set ? set_of(row0) : (int)blockIdx.y;
     float2 g[NV], b[NV];
+    auto load_set = [&](int k) {
+        const float* __restrict__ gamma = (const float*)gtab.p[k];
+        const float* __restrict__ beta = (const float*)btab.p[k];
 #pragma unroll
-    for (int i = 0; i < NV; ++i) {
-        g[i] = *reinterpret_cast<const float2*>(gamma + i * 64 + lane * 2);
-        b[i] = *reinterpret_cast<const float2*>(beta + i * 64 + lane * 2);
-    }
+        for (int i = 0; i < NV; ++i) {
+            g[i] = *reinterpret_cast<const float2*>(gamma + i * 64 + lane * 2);
+            b[i] = *reinterpret_cast<const float2*>(beta + i * 64 + lane * 2);
+        }
+    };
+    if (kcur >= 0) load_set(kcur);
 #pragma unroll
     for (int r = 0; r < R; ++r) {
         const int row = row0 + r;
         if (row >= hi) break;
+        if (sample_set && r > 0) {
+            const int k = set_of(row);
+            if (k != kcur && k >= 0) load_set(k);
+            kcur = k;
+        }
+        const bool bad = kcur < 0;
         float s = 0.f;
 #pragma unroll
         for (int i = 0; i < NV; ++i) s += v[r][i].x + v[r][i].y;
@@ -59,8 +78,8 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x
 #pragma unroll
         for (int i = 0; i < NV; ++i)
             *reinterpret_cast<uint32_t*>(yr + i * 64 + lane * 2) =
-                f2_to_bf2((v[r][i].x - mean) * rstd * g[i].x + b[i].x, (v[r][i].y - mean) * rstd * g[i].y + b[i].y);
-        if (lane == 0) {
+                bad ? 0x7fc07fc0u : f2_to_bf2((v[r][i].x - mean) * rstd * g[i].x + b[i].x, (v[r][i].y - mean) * rstd * g[i].y + b[i].y);
+        if (lane == 0 && mean_out) {
             mean_out[row] = mean;
             rstd_out[row] = rstd;
         }
@@ -568,10 +587,12 @@ int apply_rows_per_block(int Mg, int C, int G) {
         default: X(8, 1)        \
     }
 
+// sample_set != NULL: per-sample sets (G = 1, nsets table entries); else row group g of G uses table entry g
 static int ln_fwd_launch(const float* x, MdvPtrTable gt, MdvPtrTable bt, float eps, void* y_bf16, float* mean, float* rstd, int G, int Mg,
-                         int C, cudaStream_t st) {
+                         int C, cudaStream_t st, const int* sample_set = nullptr, int rows_per_sample = 1, int nsets = 0) {
 #define MDV_LN_FWD(NV, R)                                                                                                        \
-    mdv_launch((ln_fwd_kernel<NV, R>), dim3(mdv_cdiv(Mg, 8 * R), G), dim3(256), 0, st, x, gt, bt, eps, (bf16*)y_bf16, mean, rstd, Mg); \
+    mdv_launch((ln_fwd_kernel<NV, R>), dim3(mdv_cdiv(Mg, 8 * R), G), dim3(256), 0, st, x, gt, bt, eps, (bf16*)y_bf16, mean, rstd, Mg, \
+               sample_set, rows_per_sample, nsets);                                                                             \
     break;
     MDV_LN_DISPATCH(MDV_LN_FWD)
 #undef MDV_LN_FWD
@@ -625,6 +646,13 @@ extern "C" int mdv_layernorm_fwd_gp(const float* x, MdvPtrTable gamma, MdvPtrTab
     if (G < 1 || G > MDV_MAX_GROUPS || !x || !y_bf16 || !mean || !rstd || !ln_shape_ok(Mg, C)) return MDV_ERR_ARG;
     if (!tables_set(G, {&gamma, &beta}) || (long long)G * Mg >= 0x7fffffffLL) return MDV_ERR_ARG;
     return ln_fwd_launch(x, gamma, beta, eps, y_bf16, mean, rstd, G, Mg, C, (cudaStream_t)stream);
+}
+
+extern "C" int mdv_layernorm_fwd_sets(const float* x, MdvPtrTable gamma, MdvPtrTable beta, float eps, void* y_bf16, float* mean, float* rstd,
+                                      const int* sample_set, int rows_per_sample, int S, int M, int C, void* stream) {
+    if (S < 1 || S > MDV_MAX_GROUPS || !x || !y_bf16 || !sample_set || rows_per_sample < 1 || !ln_shape_ok(M, C)) return MDV_ERR_ARG;
+    if (!tables_set(S, {&gamma, &beta})) return MDV_ERR_ARG;
+    return ln_fwd_launch(x, gamma, beta, eps, y_bf16, mean, rstd, 1, M, C, (cudaStream_t)stream, sample_set, rows_per_sample, S);
 }
 
 extern "C" int mdv_layernorm_bwd(const float* dy, const float* x, const float* mean, const float* rstd, const float* gamma,
@@ -684,24 +712,42 @@ extern "C" int mdv_bn_stats(const float* z, int M, int C, float eps, float momen
     return MDV_OK;
 }
 
-__global__ void bn_fold_kernel(const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ rm,
-                               const float* __restrict__ rv, const float* __restrict__ cbias, float eps, float* __restrict__ scale,
-                               float* __restrict__ shift, int C) {
+// Eval-mode BatchNorm folds of S parameter sets (blockIdx.y = set): scale / shift are [S, C]; the conv bias is shared.
+__global__ void bn_fold_kernel(const __grid_constant__ MdvPtrTable gt, const __grid_constant__ MdvPtrTable bt,
+                               const __grid_constant__ MdvPtrTable rmt, const __grid_constant__ MdvPtrTable rvt,
+                               const float* __restrict__ cbias, float eps, float* __restrict__ scale, float* __restrict__ shift, int C) {
     MDV_PDL_SYNC();
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= C) return;
+    const int k = blockIdx.y;
+    const float* __restrict__ gamma = (const float*)gt.p[k];
+    const float* __restrict__ beta = (const float*)bt.p[k];
+    const float* __restrict__ rm = (const float*)rmt.p[k];
+    const float* __restrict__ rv = (const float*)rvt.p[k];
     const float s = gamma[c] * rsqrtf(rv[c] + eps);
-    scale[c] = s;
-    shift[c] = beta[c] + ((cbias ? cbias[c] : 0.f) - rm[c]) * s;
+    scale[(size_t)k * C + c] = s;
+    shift[(size_t)k * C + c] = beta[c] + ((cbias ? cbias[c] : 0.f) - rm[c]) * s;
+}
+
+static int bn_fold_launch(MdvPtrTable gt, MdvPtrTable bt, MdvPtrTable rmt, MdvPtrTable rvt, const float* conv_bias, float eps, float* scale,
+                          float* shift, int S, int C, cudaStream_t st) {
+    mdv_launch(bn_fold_kernel, dim3(mdv_cdiv(C, 128), S), dim3(128), 0, st, gt, bt, rmt, rvt, conv_bias, eps, scale, shift, C);
+    MDV_CHECK_LAUNCH();
+    return MDV_OK;
 }
 
 extern "C" int mdv_bn_fold(const float* gamma, const float* beta, const float* running_mean, const float* running_var,
                            const float* conv_bias, float eps, float* scale, float* shift, int C, void* stream) {
     if (!gamma || !beta || !running_mean || !running_var || !scale || !shift || C <= 0) return MDV_ERR_ARG;
-    mdv_launch(bn_fold_kernel, dim3(mdv_cdiv(C, 128)), dim3(128), 0, (cudaStream_t)stream, gamma, beta, running_mean, running_var, conv_bias, eps,
-               scale, shift, C);
-    MDV_CHECK_LAUNCH();
-    return MDV_OK;
+    return bn_fold_launch(one_set(gamma), one_set(beta), one_set(running_mean), one_set(running_var), conv_bias, eps, scale, shift, 1, C,
+                          (cudaStream_t)stream);
+}
+
+extern "C" int mdv_bn_fold_sets(MdvPtrTable gamma, MdvPtrTable beta, MdvPtrTable running_mean, MdvPtrTable running_var, const float* conv_bias,
+                                float eps, float* scale, float* shift, int S, int C, void* stream) {
+    if (S < 1 || S > MDV_MAX_GROUPS || !scale || !shift || C <= 0) return MDV_ERR_ARG;
+    if (!tables_set(S, {&gamma, &beta, &running_mean, &running_var})) return MDV_ERR_ARG;
+    return bn_fold_launch(gamma, beta, running_mean, running_var, conv_bias, eps, scale, shift, S, C, (cudaStream_t)stream);
 }
 
 extern "C" int mdv_bn_act_fwd(const float* z, const float* mean, const float* rstd, const float* gamma, const float* beta,

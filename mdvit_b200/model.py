@@ -673,6 +673,58 @@ class MDViT_DSN(_Trunk):
     def _bridge_parts(self, d=None):
         return self.bridge_conv1, _pick(self.bridge_norms1, d), self.bridge_conv2, _pick(self.bridge_norms2, d)
 
+    def _sample_sets(self, domains, B, device):
+        """domains -> the int32 [B] CUDA vector of per-sample norm sets.  Sequences and CPU tensors are checked here (length, range,
+        integer keys); a CUDA tensor is only checked for length and dtype and converted on the device, never read back, so the call
+        stays graph-capturable (an out-of-range value there gives NaN rows, see mdv_gemm_nt_tf32_sets)."""
+        S = len(self.stem_1.bns)
+        if torch.is_tensor(domains):
+            if domains.dim() != 1 or domains.shape[0] != B:
+                raise ValueError(f"forward_mixed needs one domain per sample: {B} samples, domains of shape {tuple(domains.shape)}")
+            if domains.dtype.is_floating_point or domains.dtype.is_complex or domains.dtype == torch.bool:
+                raise TypeError(f"forward_mixed needs integer domain keys, got {domains.dtype}")
+            if domains.is_cuda:
+                return domains.to(device=device, dtype=torch.int32).contiguous()
+            keys = [int(k) for k in domains.tolist()]
+        else:
+            domains = list(domains)
+            if len(domains) != B:
+                raise ValueError(f"forward_mixed needs one domain per sample: {B} samples, {len(domains)} domains")
+            keys = []
+            for k in domains:
+                if isinstance(k, bool) or not isinstance(k, (int, str)) or (isinstance(k, str) and not k.strip().lstrip("-").isdigit()):
+                    raise TypeError(f"forward_mixed domain keys are ints or integer strings, got {k!r}")
+                keys.append(int(k))
+        bad = [k for k in keys if not 0 <= k < S]
+        if bad:
+            raise ValueError(f"domain keys must lie in [0, {S}): got {bad}")
+        return torch.tensor(keys, dtype=torch.int32).to(device)
+
+    def forward_mixed(self, x, domain_label, domains):
+        """Inference on a batch that mixes domains: sample b is normalised with norm set int(domains[b]) in every BatchNorm and
+        LayerNorm, in ONE trunk, bridge, decoder and head pass (the norm kernels read the set index per sample on the device; see
+        ops.norm_sets).  Equivalent to forward(x[b:b+1], domain_label[b:b+1], str(domains[b]))[0] per sample.
+        domains: one key per sample — a sequence of str / int, a CPU integer tensor, or a CUDA integer tensor of length B (the
+        last is never read back: write new keys into a captured tensor and replay the graph).  domain_label follows forward's
+        rule (required for adapt_method='Sup', None otherwise).  Returns the main logits [B, 1, H, W]; the auxiliary decoders do
+        not run (the reference's test loop discards them, multi_train_MDViT.py:377-378).  Eval mode only."""
+        if self.training:
+            raise RuntimeError("forward_mixed is an inference path (eval mode); the multi-domain training pass is forward_multi")
+        S = len(self.stem_1.bns)
+        if S > 8:
+            raise ValueError(f"forward_mixed supports up to 8 norm sets (MDV_MAX_GROUPS), the model has {S}")
+        if x.dim() != 4:
+            raise ValueError("input must be [B,3,H,W]")
+        sample_set = self._sample_sets(domains, x.shape[0], x.device)
+        if not x.is_cuda:
+            raise RuntimeError("mdvit_b200 runs on CUDA (sm_100a) only; there is no CPU path")
+        keys = [str(i) for i in range(S)]
+        img_size = x.shape[2:]
+        with ops.norm_sets(sample_set):
+            enc = self._trunk_forward(x, domain_label, keys)
+            dec4, h, w = self._decode(enc, domain_label, keys)
+            return self._head(dec4, h, w, img_size)
+
     def forward(self, x, domain_label=None, d=None, out_feat=False, out_seg=True):
         img_size = x.shape[2:]
         int(d)      # the reference indexes its norm lists with int(d) everywhere (mdvit.py:65,398,917): d is required

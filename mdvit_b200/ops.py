@@ -145,9 +145,10 @@ def prep_weight(w, mode, rows, cols, ld=None, cin=0):
 # ------------------------------------------------------------------------------------------------- thin wrappers
 def gemm_nt(A, W, M, N, K, out, *, lda=None, ldw=None, ldc=None, bias=None, residual=None, act=ACT_NONE, out_preact=None,
             mul_gelu_grad=None, drop_p=0.0, drop_stream=0, rowscale=None, rows_per_scale=1, accumulate=False, colsum=None,
-            preact_mode=0, mul_mode=0, tf32=False, colscale=None):
+            preact_mode=0, mul_mode=0, tf32=False, colscale=None, sample_set=None, rows_per_sample=1):
     """out = epilogue(A . W^T).  A, W bf16 — or both fp32 with tf32=True (TF32 tensor-core math: the conv trunk, see
-    include/mdvit_b200.h mdv_gemm_nt_tf32)."""
+    include/mdvit_b200.h mdv_gemm_nt_tf32).  With a sample_set (int32 [B] on the device, tf32 only), colscale / bias are [S, N]
+    folded-BatchNorm tables and row m uses table row sample_set[m // rows_per_sample] (mdv_gemm_nt_tf32_sets)."""
     e = GemmEpi()
     e.bias, e.residual, e.mul_gelu_grad, e.out_preact = ptr(bias), ptr(residual), ptr(mul_gelu_grad), ptr(out_preact)
     e.out, e.rowscale, e.colsum, e.colscale = ptr(out), ptr(rowscale), ptr(colsum), ptr(colscale)
@@ -163,7 +164,12 @@ def gemm_nt(A, W, M, N, K, out, *, lda=None, ldw=None, ldc=None, bias=None, resi
     e.preact_mode, e.mul_mode = preact_mode, mul_mode
     e.dropout_p = float(drop_p)
     e.drop_stream = drop_stream
-    if tf32:
+    if sample_set is not None:
+        if not tf32 or A.dtype != F32 or W.dtype != F32:
+            raise TypeError("the per-sample-set GEMM is a tf32 GEMM: it needs fp32 operands")
+        check(L.lib().mdv_gemm_nt_tf32_sets(ptr(A), lda or K, ptr(W), ldw or K, M, N, K, ctypes.byref(e), ptr(sample_set), rows_per_sample,
+                                            colscale.shape[0], L.stream()), "mdv_gemm_nt_tf32_sets")
+    elif tf32:
         if A.dtype != F32 or W.dtype != F32:
             raise TypeError("tf32 GEMM needs fp32 operands")
         check(L.lib().mdv_gemm_nt_tf32(ptr(A), lda or K, ptr(W), ldw or K, M, N, K, ctypes.byref(e), L.stream()), "mdv_gemm_nt_tf32")
@@ -196,10 +202,18 @@ def cast_bf16(x, M, C, out=None, ld_in=None, ld_out=None, rowscale=None, rows_pe
     return out
 
 
-def layernorm_fwd(x, w, b, M, C, eps=1e-6):
+def layernorm_fwd(x, w, b, M, C, eps=1e-6, rows_per_sample=None):
     """w, b: lists of S parameter tensors.  S = 1 normalises every row with the one set; with S > 1, rows [s M/S, (s+1) M/S)
-    use set s (domain-specific norms)."""
+    use set s (domain-specific norms) — or, inside norm_sets(), row m uses set sample_set[m // rows_per_sample]; mean / rstd are
+    then None (inference needs neither)."""
     S = len(w)
+    if S > 1 and _NORM_SETS is not None:
+        if rows_per_sample is None:
+            raise ValueError("per-sample norm sets need rows_per_sample")
+        y = torch.empty((M, C), dtype=BF16, device=x.device)
+        check(L.lib().mdv_layernorm_fwd_sets(ptr(x), ptr_table(w), ptr_table(b), ctypes.c_float(eps), ptr(y), None, None, ptr(_NORM_SETS),
+                                             rows_per_sample, S, M, C, L.stream()), "mdv_layernorm_fwd_sets")
+        return y, None, None
     if M % S:
         raise ValueError("LayerNorm groups must divide the batch")
     y = torch.empty((M, C), dtype=BF16, device=x.device)
@@ -268,17 +282,62 @@ def current_bn_groups():
     return _BN_GROUPS
 
 
+# Per-sample norm sets: the mixed-domain inference pass of the domain-specific-norm models (model.MDViT_DSN.forward_mixed) gives
+# every norm Function all S sets, and sample b of the batch is normalised with set sample_set[b].  The index vector lives on the
+# device and the kernels read it, so one captured graph serves any domain mix.  Eval only: the train-mode paths keep their row
+# groups (bn_groups).
+_NORM_SETS = None
+
+
+class norm_sets:
+    def __init__(self, sample_set):
+        if sample_set.dtype != torch.int32 or not sample_set.is_cuda or sample_set.dim() != 1:
+            raise TypeError("norm_sets takes a 1-D int32 CUDA tensor of per-sample set indices")
+        self.sample_set = sample_set
+
+    def __enter__(self):
+        global _NORM_SETS
+        self.prev, _NORM_SETS = _NORM_SETS, self.sample_set
+        return self.sample_set
+
+    def __exit__(self, *exc):
+        global _NORM_SETS
+        _NORM_SETS = self.prev
+
+
+def current_norm_sets():
+    return _NORM_SETS
+
+
+def _check_norm_sets(training):
+    if training and _NORM_SETS is not None:
+        raise RuntimeError("ops.norm_sets (per-sample norm sets) is an eval-mode path; training uses per-group sets (bn_groups)")
+
+
 def _one_set(*lists):
-    """The tensors of a single norm parameter set: the eval-mode paths take one set."""
+    """The tensors of a single norm parameter set: the eval-mode paths take one set (or S sets inside norm_sets)."""
     if len(lists[0]) != 1:
         raise ValueError("per-group norm sets are a train-mode path")
     return [t[0] for t in lists]
 
 
+def _sets_kw(scale, rows_per_sample):
+    """The gemm_nt arguments that select a folded BatchNorm's set per sample: none for one set ([C] scale), the norm_sets index
+    vector for S sets ([S, C] scale from bn_fold)."""
+    return {} if scale.dim() == 1 else {"sample_set": _NORM_SETS, "rows_per_sample": rows_per_sample}
+
+
 def bn_fold(weight, bias, running_mean, running_var, conv_bias=None, eps=1e-5):
     """Eval-mode BatchNorm as (scale, shift) for the epilogue of the GEMM that feeds it (gemm_nt(colscale=scale, bias=shift,
     act=...)): the normalised tensor is produced by the GEMM itself, its fp32 pre-activation never reaches HBM.  The parameters and
-    buffers are one-element lists."""
+    buffers are lists of S sets: S = 1 gives [C] vectors; S > 1 (inside norm_sets only) gives [S, C] tables in one launch, for
+    gemm_nt(..., **_sets_kw(scale, rows_per_sample))."""
+    if len(weight) > 1 and _NORM_SETS is not None:
+        S, C = len(weight), weight[0].numel()
+        st = torch.empty((2, S, C), dtype=F32, device=weight[0].device)
+        check(L.lib().mdv_bn_fold_sets(ptr_table(weight), ptr_table(bias), ptr_table(running_mean), ptr_table(running_var), ptr(conv_bias),
+                                       ctypes.c_float(eps), ptr(st[0]), ptr(st[1]), S, C, L.stream()), "mdv_bn_fold_sets")
+        return st[0], st[1]
     weight, bias, running_mean, running_var = _one_set(weight, bias, running_mean, running_var)
     C = weight.numel()
     st = torch.empty((2, C), dtype=F32, device=weight.device)
@@ -501,9 +560,10 @@ class BlockFn(torch.autograd.Function):
         ctx.params = (cpe_w, cpe_b, c3w, c3b, c5w, c5b, c7w, c7b, qkv_w, qkv_b, proj_w, proj_b, da_w1, da_b1, da_w2, da_b2,
                       fc1_w, fc1_b, fc2_w, fc2_b) + norm
         (n1w, n1b), (n2w, n2b) = _norm_slots(norm, 2)
+        _check_norm_sets(training)
         with _dev_ctx(x):
             x1 = dwconv3(x, cpe_w, cpe_b, B, H, W, H, W, C, 1, residual=True)
-            ln1, mean1, rstd1 = layernorm_fwd(x1, n1w, n1b, M, C)
+            ln1, mean1, rstd1 = layernorm_fwd(x1, n1w, n1b, M, C, rows_per_sample=N)
             qkv = torch.empty((M, 3 * C), dtype=BF16, device=dev)
             gemm_nt(ln1, prep_weight(qkv_w, 0, 3 * C, C), M, 3 * C, C, qkv, bias=qkv_b)
             gate = hid = None
@@ -533,7 +593,7 @@ class BlockFn(torch.autograd.Function):
             x2 = torch.empty((M, C), dtype=F32, device=dev)
             gemm_nt(y, prep_weight(proj_w, 0, C, C), M, C, C, x2, bias=proj_b, residual=x1, drop_p=p_drop, drop_stream=sid[0],
                     rowscale=dp1, rows_per_scale=N)
-            ln2, mean2, rstd2 = layernorm_fwd(x2, n2w, n2b, M, C)
+            ln2, mean2, rstd2 = layernorm_fwd(x2, n2w, n2b, M, C, rows_per_sample=N)
             need_grad = any(ctx.needs_input_grad)
             x3 = torch.empty((B, N, C), dtype=F32, device=dev)
             fused_mlp = bool(lib.mdv_mlp_supported(C, hidden)) and _FUSED_MLP
@@ -661,6 +721,7 @@ class StemFn(torch.autograd.Function):
         M0, M1 = B * H1 * W1, B * H2 * W2
         ctx.params = (w0, w1) + norm
         (g0, b0, rm0, rv0, nb0), (g1, b1, rm1, rv1, nb1) = _norm_slots(norm, 2, bufs)
+        _check_norm_sets(training)
         lib = L.lib()
         with _dev_ctx(img):
             # TF32 operands (fp32 in memory) for both stem convs: see mdv_gemm_nt_tf32
@@ -671,10 +732,12 @@ class StemFn(torch.autograd.Function):
                 # eval: BatchNorm (running statistics) + Hardswish folded into the GEMM epilogues
                 a0, y = torch.empty((M0, 32), dtype=F32, device=dev), torch.empty((M1, 64), dtype=F32, device=dev)
                 s0, t0 = bn_fold(g0, b0, rm0, rv0)
-                gemm_nt(col0, prep_weight(w0, 2 | 8, 32, 27, ld=32, cin=3), M0, 32, 32, a0, tf32=True, colscale=s0, bias=t0, act=ACT_HSWISH)
+                gemm_nt(col0, prep_weight(w0, 2 | 8, 32, 27, ld=32, cin=3), M0, 32, 32, a0, tf32=True, colscale=s0, bias=t0, act=ACT_HSWISH,
+                        **_sets_kw(s0, H1 * W1))
                 check(lib.mdv_im2col3(ptr(a0), 0, ptr(col1), 0, B, H1, W1, H2, W2, 32, 2, 288, L.stream()), "mdv_im2col3")
                 s1, t1 = bn_fold(g1, b1, rm1, rv1)
-                gemm_nt(col1, prep_weight(w1, 2 | 8, 64, 288, cin=32), M1, 64, 288, y, tf32=True, colscale=s1, bias=t1, act=ACT_HSWISH)
+                gemm_nt(col1, prep_weight(w1, 2 | 8, 64, 288, cin=32), M1, 64, 288, y, tf32=True, colscale=s1, bias=t1, act=ACT_HSWISH,
+                        **_sets_kw(s1, H2 * W2))
                 ctx.meta = (B, H1, W1, H2, W2, training)
                 ctx.set_materialize_grads(False)
                 return y.view(B, H2 * W2, 64)
@@ -735,12 +798,13 @@ class PatchEmbedFn(torch.autograd.Function):
         x = _contig(x)
         ctx.params = (dw_w, pw_w) + norm
         ((g, b, rm, rv, nb),) = _norm_slots(norm, 1, bufs)
+        _check_norm_sets(training)
         with _dev_ctx(x):
             t = dwconv3(x, dw_w, None, B, Hi, Wi, Ho, Wo, Cin, stride)          # fp32: TF32 operand of the pointwise conv
             if not training:      # eval: BatchNorm + Hardswish folded into the GEMM epilogue
                 y = torch.empty((M, C), dtype=F32, device=dev)
                 sc, sh = bn_fold(g, b, rm, rv)
-                gemm_nt(t, _contig(pw_w).view(C, Cin), M, C, Cin, y, tf32=True, colscale=sc, bias=sh, act=ACT_HSWISH)
+                gemm_nt(t, _contig(pw_w).view(C, Cin), M, C, Cin, y, tf32=True, colscale=sc, bias=sh, act=ACT_HSWISH, **_sets_kw(sc, Ho * Wo))
                 ctx.meta = (B, Hi, Wi, Ho, Wo, Cin, C, stride, training)
                 return y.view(B, Ho * Wo, C)
             z = torch.empty((M, C), dtype=F32, device=dev)
@@ -790,6 +854,7 @@ class BridgeFn(torch.autograd.Function):
         x = _contig(x)
         ctx.params = (w0, c0, w1, c1) + norm
         (g0, b0, rm0, rv0, nb0), (g1, b1, rm1, rv1, nb1) = _norm_slots(norm, 2, bufs)
+        _check_norm_sets(training)
         lib = L.lib()
         with _dev_ctx(x):
             col0 = torch.empty((M, 9 * C), dtype=F32, device=dev)
@@ -798,10 +863,12 @@ class BridgeFn(torch.autograd.Function):
             if not training:      # eval: conv bias + BatchNorm + ReLU folded into the GEMM epilogues
                 a0, y = torch.empty((M, C0), dtype=F32, device=dev), torch.empty((M, C1), dtype=F32, device=dev)
                 s0, t0 = bn_fold(g0, b0, rm0, rv0, c0)
-                gemm_nt(col0, prep_weight(w0, 2 | 8, C0, 9 * C, cin=C), M, C0, 9 * C, a0, tf32=True, colscale=s0, bias=t0, act=ACT_RELU)
+                gemm_nt(col0, prep_weight(w0, 2 | 8, C0, 9 * C, cin=C), M, C0, 9 * C, a0, tf32=True, colscale=s0, bias=t0, act=ACT_RELU,
+                        **_sets_kw(s0, H * W))
                 check(lib.mdv_im2col3(ptr(a0), 0, ptr(col1), 0, B, H, W, H, W, C0, 1, 9 * C0, L.stream()), "mdv_im2col3")
                 s1, t1 = bn_fold(g1, b1, rm1, rv1, c1)
-                gemm_nt(col1, prep_weight(w1, 2 | 8, C1, 9 * C0, cin=C0), M, C1, 9 * C0, y, tf32=True, colscale=s1, bias=t1, act=ACT_RELU)
+                gemm_nt(col1, prep_weight(w1, 2 | 8, C1, 9 * C0, cin=C0), M, C1, 9 * C0, y, tf32=True, colscale=s1, bias=t1, act=ACT_RELU,
+                        **_sets_kw(s1, H * W))
                 ctx.meta = (B, H, W, C, C0, C1, training)
                 return y.view(B, H * W, C1)
             z0 = torch.empty((M, C0), dtype=F32, device=dev)
@@ -862,6 +929,7 @@ class DecoderConvFn(torch.autograd.Function):
         inp, skip = _contig(inp), _contig(skip)
         ctx.params = (cb_w, cb_b, dw_w, pw_w) + norm
         ((g, b, rm, rv, nb),) = _norm_slots(norm, 1, bufs)
+        _check_norm_sets(training)
         lib = L.lib()
         with _dev_ctx(inp):
             # both 1x1 convs of the decoder trunk run on TF32 operands (fp32 in memory): see mdv_gemm_nt_tf32
@@ -873,7 +941,7 @@ class DecoderConvFn(torch.autograd.Function):
             if not training:      # eval: BatchNorm + Hardswish folded into the GEMM epilogue
                 y = torch.empty((M, C), dtype=F32, device=dev)
                 sc, sh = bn_fold(g, b, rm, rv)
-                gemm_nt(gc, _contig(pw_w).view(C, C), M, C, C, y, tf32=True, colscale=sc, bias=sh, act=ACT_HSWISH)
+                gemm_nt(gc, _contig(pw_w).view(C, C), M, C, C, y, tf32=True, colscale=sc, bias=sh, act=ACT_HSWISH, **_sets_kw(sc, H * W))
                 ctx.meta = (B, h, w, H, W, Cin, C, training)
                 return y.view(B, H * W, C)
             z = torch.empty((M, C), dtype=F32, device=dev)
