@@ -321,17 +321,17 @@ def _one_set(*lists):
     return [t[0] for t in lists]
 
 
-def _sets_kw(scale, rows_per_sample):
-    """The gemm_nt arguments that select a folded BatchNorm's set per sample: none for one set ([C] scale), the norm_sets index
-    vector for S sets ([S, C] scale from bn_fold)."""
-    return {} if scale.dim() == 1 else {"sample_set": _NORM_SETS, "rows_per_sample": rows_per_sample}
+def _require_train_bn(training):
+    """Backward of a Function whose forward ran BatchNorm in eval mode: that forward saved no batch statistics."""
+    if not training:
+        raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
 
 
 def bn_fold(weight, bias, running_mean, running_var, conv_bias=None, eps=1e-5):
     """Eval-mode BatchNorm as (scale, shift) for the epilogue of the GEMM that feeds it (gemm_nt(colscale=scale, bias=shift,
     act=...)): the normalised tensor is produced by the GEMM itself, its fp32 pre-activation never reaches HBM.  The parameters and
     buffers are lists of S sets: S = 1 gives [C] vectors; S > 1 (inside norm_sets only) gives [S, C] tables in one launch, for
-    gemm_nt(..., **_sets_kw(scale, rows_per_sample))."""
+    the per-sample-set GEMM (see _conv_bn_fwd)."""
     if len(weight) > 1 and _NORM_SETS is not None:
         S, C = len(weight), weight[0].numel()
         st = torch.empty((2, S, C), dtype=F32, device=weight[0].device)
@@ -709,6 +709,67 @@ def _norm_grads(*slots):
     return tuple(r for s in range(len(slots[0][0])) for gw, gb in slots for r in (gw[s], gb[s]))
 
 
+def _conv_bn_fwd(A, w, M, K, slot, act, training, rows_per_sample, conv_bias=None):
+    """One conv -> BatchNorm -> act stage of the MDViT conv trunk: a TF32 GEMM of the fp32 operand A [M, K] (the im2col matrix of a
+    3x3 conv in mdv_im2col3 order, padded to K columns, or the input of a 1x1 conv) with the conv weight w [Cout, Cin, k, k].
+    slot = (weights, biases, running_means, running_vars, nbts), lists over the S norm sets (_norm_slots).
+    Training: the GEMM writes z = conv + conv_bias, and bn_forward normalises each bn_groups() row group with its batch statistics.
+    Eval: the running statistics and conv_bias fold into the GEMM epilogue (bn_fold), so z never reaches HBM; inside norm_sets with
+    S > 1, row m takes the folded set of sample sample_set[m // rows_per_sample].
+    Returns (y [M, Cout] fp32, (z, mean, rstd) to save for backward; all None in eval)."""
+    g, b, rm, rv, nb = slot
+    _check_norm_sets(training)
+    if not training:
+        scale, shift = bn_fold(g, b, rm, rv, conv_bias)
+    Cout, Cin = w.shape[:2]
+    Wt = prep_weight(w, 2 | 8, Cout, 9 * Cin, ld=K, cin=Cin) if w.shape[2] == 3 else _contig(w).view(Cout, K)
+    out = torch.empty((M, Cout), dtype=F32, device=A.device)
+    if training:
+        gemm_nt(A, Wt, M, Cout, K, out, bias=conv_bias, tf32=True)
+        y, mean, rstd = bn_forward(out, M, Cout, g, b, rm, rv, nb, training, act, False)
+        return y, (out, mean, rstd)
+    gemm_nt(A, Wt, M, Cout, K, out, tf32=True, colscale=scale, bias=shift, act=act, sample_set=_NORM_SETS if scale.dim() == 2 else None,
+            rows_per_sample=rows_per_sample)
+    return out, (None, None, None)
+
+
+def _conv1_wgrad(dz, a, w):
+    """Weight gradient of a 1x1 conv w [Cout, Cin, 1, 1] from dz [M, Cout] and its input a [M, Cin]; an fp32 a is cast to the bf16
+    operand only when the gradient is wanted.  Returns what backward returns for w."""
+    Cout, Cin = w.shape[:2]
+    gw, rw = gtarget(w, (Cout, Cin))
+    if gw is not None:
+        M = dz.shape[0]
+        gemm_tn(dz, a if a.dtype == BF16 else cast_bf16(a, M, Cin), M, Cout, Cin, gw)
+    return rw
+
+
+def _conv3_wgrad(dz, col, w):
+    """Weight gradient of a 3x3 conv w [Cout, Cin, 3, 3] from dz [M, Cout] and its im2col matrix col [M, ld] ((tap, channel) column
+    order, ld >= 9 Cin; fp32 is cast to the bf16 operand only when the gradient is wanted): gemm_tn into a zeroed [Cout, ld] buffer,
+    unpermuted into w's layout.  Returns what backward returns for w."""
+    gw, rw = gtarget(w)
+    if gw is not None:
+        (M, ld), Cout, Cin = col.shape, w.shape[0], w.shape[1]
+        gwp = gemm_tn(dz, col if col.dtype == BF16 else cast_bf16(col, M, ld), M, Cout, ld, torch.zeros((Cout, ld), dtype=F32, device=dz.device))
+        check(L.lib().mdv_unperm_conv_grad(ptr(gwp), ld, ptr(gw), Cout, Cin, L.stream()), "mdv_unperm_conv_grad")
+    return rw
+
+
+def _conv3_bwd(dz, col, w, cb, B, H, W, Ho, Wo, stride):
+    """Backward of a 3x3 conv (padding 1, stride `stride`, [B, H, W, Cin] -> [B, Ho, Wo, Cout]) run as im2col matrix col
+    [B*Ho*Wo, 9 Cin] times w^T, plus conv bias cb (or None).  Returns (w's gradient, cb's gradient, dx [B*H*W, Cin] fp32)."""
+    Cout, Cin = w.shape[:2]
+    M, dev = dz.shape[0], dz.device
+    rw = _conv3_wgrad(dz, col, w)
+    gb, rb = gtarget(cb)
+    colsum(dz, M, Cout, gb)
+    dcol = gemm_nt(dz, prep_weight(w, 3, Cout, 9 * Cin, cin=Cin), M, 9 * Cin, Cout, torch.empty((M, 9 * Cin), dtype=F32, device=dev))
+    dx = torch.empty((B * H * W, Cin), dtype=F32, device=dev)
+    check(L.lib().mdv_col2im3(ptr(dcol), ptr(dx), B, H, W, Ho, Wo, Cin, stride, 9 * Cin, L.stream()), "mdv_col2im3")
+    return rw, rb, dx
+
+
 class StemFn(torch.autograd.Function):
     """stem = 2x (Conv3x3 s2 no-bias -> BN -> Hardswish), mdvit.py:509-526.  im2col (bf16) + tcgen05 GEMM."""
 
@@ -720,35 +781,17 @@ class StemFn(torch.autograd.Function):
         H1, W1, H2, W2 = H // 2, W // 2, H // 4, W // 4
         M0, M1 = B * H1 * W1, B * H2 * W2
         ctx.params = (w0, w1) + norm
-        (g0, b0, rm0, rv0, nb0), (g1, b1, rm1, rv1, nb1) = _norm_slots(norm, 2, bufs)
-        _check_norm_sets(training)
+        slot0, slot1 = _norm_slots(norm, 2, bufs)
         lib = L.lib()
         with _dev_ctx(img):
             # TF32 operands (fp32 in memory) for both stem convs: see mdv_gemm_nt_tf32
             col0 = torch.empty((M0, 32), dtype=F32, device=dev)
             check(lib.mdv_im2col_stem(ptr(img), ptr(col0), 0, B, H, W, L.stream()), "mdv_im2col_stem")
+            a0, saved0 = _conv_bn_fwd(col0, w0, M0, 32, slot0, ACT_HSWISH, training, H1 * W1)
             col1 = torch.empty((M1, 288), dtype=F32, device=dev)
-            if not training:
-                # eval: BatchNorm (running statistics) + Hardswish folded into the GEMM epilogues
-                a0, y = torch.empty((M0, 32), dtype=F32, device=dev), torch.empty((M1, 64), dtype=F32, device=dev)
-                s0, t0 = bn_fold(g0, b0, rm0, rv0)
-                gemm_nt(col0, prep_weight(w0, 2 | 8, 32, 27, ld=32, cin=3), M0, 32, 32, a0, tf32=True, colscale=s0, bias=t0, act=ACT_HSWISH,
-                        **_sets_kw(s0, H1 * W1))
-                check(lib.mdv_im2col3(ptr(a0), 0, ptr(col1), 0, B, H1, W1, H2, W2, 32, 2, 288, L.stream()), "mdv_im2col3")
-                s1, t1 = bn_fold(g1, b1, rm1, rv1)
-                gemm_nt(col1, prep_weight(w1, 2 | 8, 64, 288, cin=32), M1, 64, 288, y, tf32=True, colscale=s1, bias=t1, act=ACT_HSWISH,
-                        **_sets_kw(s1, H2 * W2))
-                ctx.meta = (B, H1, W1, H2, W2, training)
-                ctx.set_materialize_grads(False)
-                return y.view(B, H2 * W2, 64)
-            z0 = torch.empty((M0, 32), dtype=F32, device=dev)
-            gemm_nt(col0, prep_weight(w0, 2 | 8, 32, 27, ld=32, cin=3), M0, 32, 32, z0, tf32=True)
-            a0, mean0, rstd0 = bn_forward(z0, M0, 32, g0, b0, rm0, rv0, nb0, training, ACT_HSWISH, False)
             check(lib.mdv_im2col3(ptr(a0), 0, ptr(col1), 0, B, H1, W1, H2, W2, 32, 2, 288, L.stream()), "mdv_im2col3")
-            z1 = torch.empty((M1, 64), dtype=F32, device=dev)
-            gemm_nt(col1, prep_weight(w1, 2 | 8, 64, 288, cin=32), M1, 64, 288, z1, tf32=True)
-            y, mean1, rstd1 = bn_forward(z1, M1, 64, g1, b1, rm1, rv1, nb1, training, ACT_HSWISH, False)
-        ctx.save_for_backward(col0, z0, mean0, rstd0, col1, z1, mean1, rstd1)
+            y, saved1 = _conv_bn_fwd(col1, w1, M1, 288, slot1, ACT_HSWISH, training, H2 * W2)
+        ctx.save_for_backward(col0, *saved0, col1, *saved1)
         ctx.meta = (B, H1, W1, H2, W2, training)
         _fwd_mark(ctx)
         ctx.set_materialize_grads(False)
@@ -759,29 +802,16 @@ class StemFn(torch.autograd.Function):
         if dy is None:       # the da_only pass stops at the first patch embedding
             return (None,) * (3 + len(ctx.params))
         B, H1, W1, H2, W2, training = ctx.meta
-        if not training:
-            raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
+        _require_train_bn(training)
         col0, z0, mean0, rstd0, col1, z1, mean1, rstd1 = ctx.saved_tensors
         w0, w1 = ctx.params[:2]
         (g0, b0), (g1, b1) = _norm_slots(ctx.params[2:], 2)
-        M0, M1, dev = B * H1 * W1, B * H2 * W2, dy.device
-        lib = L.lib()
         dy = _contig(dy.float())
         with _dev_ctx(dy):
-            dz1, rg1, rb1 = bn_backward(dy, z1, mean1, rstd1, g1, b1, ACT_HSWISH, M1, 64)
-            gw1, rw1 = gtarget(w1)
-            if gw1 is not None:     # (weight gradients run on bf16 operands: cast the saved fp32 im2col matrices)
-                gw1p = gemm_tn(dz1, cast_bf16(col1, M1, 288), M1, 64, 288, torch.zeros((64, 288), dtype=F32, device=dev))
-                check(lib.mdv_unperm_conv_grad(ptr(gw1p), 288, ptr(gw1), 64, 32, L.stream()), "mdv_unperm_conv_grad")
-            dcol1 = torch.empty((M1, 288), dtype=F32, device=dev)
-            gemm_nt(dz1, prep_weight(w1, 3, 64, 288, cin=32), M1, 288, 64, dcol1)
-            da0 = torch.empty((M0, 32), dtype=F32, device=dev)
-            check(lib.mdv_col2im3(ptr(dcol1), ptr(da0), B, H1, W1, H2, W2, 32, 2, 288, L.stream()), "mdv_col2im3")
-            dz0, rg0, rb0 = bn_backward(da0, z0, mean0, rstd0, g0, b0, ACT_HSWISH, M0, 32)
-            gw0, rw0 = gtarget(w0)
-            if gw0 is not None:
-                gw0p = gemm_tn(dz0, cast_bf16(col0, M0, 32), M0, 32, 32, torch.zeros((32, 32), dtype=F32, device=dev))
-                check(lib.mdv_unperm_conv_grad(ptr(gw0p), 32, ptr(gw0), 32, 3, L.stream()), "mdv_unperm_conv_grad")
+            dz1, rg1, rb1 = bn_backward(dy, z1, mean1, rstd1, g1, b1, ACT_HSWISH, B * H2 * W2, 64)
+            rw1, _, da0 = _conv3_bwd(dz1, col1, w1, None, B, H1, W1, H2, W2, 2)
+            dz0, rg0, rb0 = bn_backward(da0, z0, mean0, rstd0, g0, b0, ACT_HSWISH, B * H1 * W1, 32)
+            rw0 = _conv3_wgrad(dz0, col0, w0)
         _grads_done(ctx)
         return (None, rw0, rw1, None, None) + _norm_grads((rg0, rb0), (rg1, rb1))
 
@@ -794,22 +824,13 @@ class PatchEmbedFn(torch.autograd.Function):
         B, _, Cin = x.shape
         C = pw_w.shape[0]
         Ho, Wo = (Hi + 2 - 3) // stride + 1, (Wi + 2 - 3) // stride + 1
-        M, dev = B * Ho * Wo, x.device
+        M = B * Ho * Wo
         x = _contig(x)
         ctx.params = (dw_w, pw_w) + norm
-        ((g, b, rm, rv, nb),) = _norm_slots(norm, 1, bufs)
-        _check_norm_sets(training)
+        (slot,) = _norm_slots(norm, 1, bufs)
         with _dev_ctx(x):
             t = dwconv3(x, dw_w, None, B, Hi, Wi, Ho, Wo, Cin, stride)          # fp32: TF32 operand of the pointwise conv
-            if not training:      # eval: BatchNorm + Hardswish folded into the GEMM epilogue
-                y = torch.empty((M, C), dtype=F32, device=dev)
-                sc, sh = bn_fold(g, b, rm, rv)
-                gemm_nt(t, _contig(pw_w).view(C, Cin), M, C, Cin, y, tf32=True, colscale=sc, bias=sh, act=ACT_HSWISH, **_sets_kw(sc, Ho * Wo))
-                ctx.meta = (B, Hi, Wi, Ho, Wo, Cin, C, stride, training)
-                return y.view(B, Ho * Wo, C)
-            z = torch.empty((M, C), dtype=F32, device=dev)
-            gemm_nt(t, _contig(pw_w).view(C, Cin), M, C, Cin, z, tf32=True)
-            y, mean, rstd = bn_forward(z, M, C, g, b, rm, rv, nb, training, ACT_HSWISH, False)
+            y, (z, mean, rstd) = _conv_bn_fwd(t, pw_w, M, Cin, slot, ACT_HSWISH, training, Ho * Wo)
         ctx.save_for_backward(x, t, z, mean, rstd)
         ctx.meta = (B, Hi, Wi, Ho, Wo, Cin, C, stride, training)
         _fwd_mark(ctx)
@@ -819,8 +840,7 @@ class PatchEmbedFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dy):
         B, Hi, Wi, Ho, Wo, Cin, C, stride, training = ctx.meta
-        if not training:
-            raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
+        _require_train_bn(training)
         x, t, z, mean, rstd = ctx.saved_tensors
         dw_w, pw_w = ctx.params[:2]
         ((g, b),) = _norm_slots(ctx.params[2:], 1)
@@ -831,9 +851,7 @@ class PatchEmbedFn(torch.autograd.Function):
         dy = _contig(dy.float())
         with _dev_ctx(dy):
             dz, rg, rb = bn_backward(dy, z, mean, rstd, g, b, ACT_HSWISH, M, C)
-            g_pw, r_pw = gtarget(pw_w, (C, Cin))
-            if g_pw is not None:
-                gemm_tn(dz, cast_bf16(t, M, Cin), M, C, Cin, g_pw)
+            r_pw = _conv1_wgrad(dz, t, pw_w)
             dt = torch.empty((M, Cin), dtype=F32, device=dev)
             gemm_nt(dz, prep_weight(pw_w, 1, C, Cin), M, Cin, C, dt)
             dx = dwconv3(dt, dw_w, None, B, Ho, Wo, Hi, Wi, Cin, stride, transposed=True)
@@ -853,32 +871,16 @@ class BridgeFn(torch.autograd.Function):
         M, dev = B * H * W, x.device
         x = _contig(x)
         ctx.params = (w0, c0, w1, c1) + norm
-        (g0, b0, rm0, rv0, nb0), (g1, b1, rm1, rv1, nb1) = _norm_slots(norm, 2, bufs)
-        _check_norm_sets(training)
+        slot0, slot1 = _norm_slots(norm, 2, bufs)
         lib = L.lib()
         with _dev_ctx(x):
             col0 = torch.empty((M, 9 * C), dtype=F32, device=dev)
             check(lib.mdv_im2col3(ptr(x), 0, ptr(col0), 0, B, H, W, H, W, C, 1, 9 * C, L.stream()), "mdv_im2col3")
             col1 = torch.empty((M, 9 * C0), dtype=F32, device=dev)
-            if not training:      # eval: conv bias + BatchNorm + ReLU folded into the GEMM epilogues
-                a0, y = torch.empty((M, C0), dtype=F32, device=dev), torch.empty((M, C1), dtype=F32, device=dev)
-                s0, t0 = bn_fold(g0, b0, rm0, rv0, c0)
-                gemm_nt(col0, prep_weight(w0, 2 | 8, C0, 9 * C, cin=C), M, C0, 9 * C, a0, tf32=True, colscale=s0, bias=t0, act=ACT_RELU,
-                        **_sets_kw(s0, H * W))
-                check(lib.mdv_im2col3(ptr(a0), 0, ptr(col1), 0, B, H, W, H, W, C0, 1, 9 * C0, L.stream()), "mdv_im2col3")
-                s1, t1 = bn_fold(g1, b1, rm1, rv1, c1)
-                gemm_nt(col1, prep_weight(w1, 2 | 8, C1, 9 * C0, cin=C0), M, C1, 9 * C0, y, tf32=True, colscale=s1, bias=t1, act=ACT_RELU,
-                        **_sets_kw(s1, H * W))
-                ctx.meta = (B, H, W, C, C0, C1, training)
-                return y.view(B, H * W, C1)
-            z0 = torch.empty((M, C0), dtype=F32, device=dev)
-            gemm_nt(col0, prep_weight(w0, 2 | 8, C0, 9 * C, cin=C), M, C0, 9 * C, z0, bias=c0, tf32=True)
-            a0, mean0, rstd0 = bn_forward(z0, M, C0, g0, b0, rm0, rv0, nb0, training, ACT_RELU, False)
+            a0, saved0 = _conv_bn_fwd(col0, w0, M, 9 * C, slot0, ACT_RELU, training, H * W, c0)
             check(lib.mdv_im2col3(ptr(a0), 0, ptr(col1), 0, B, H, W, H, W, C0, 1, 9 * C0, L.stream()), "mdv_im2col3")
-            z1 = torch.empty((M, C1), dtype=F32, device=dev)
-            gemm_nt(col1, prep_weight(w1, 2 | 8, C1, 9 * C0, cin=C0), M, C1, 9 * C0, z1, bias=c1, tf32=True)
-            y, mean1, rstd1 = bn_forward(z1, M, C1, g1, b1, rm1, rv1, nb1, training, ACT_RELU, False)
-        ctx.save_for_backward(col0, z0, mean0, rstd0, col1, z1, mean1, rstd1)
+            y, saved1 = _conv_bn_fwd(col1, w1, M, 9 * C0, slot1, ACT_RELU, training, H * W, c1)
+        ctx.save_for_backward(col0, *saved0, col1, *saved1)
         ctx.meta = (B, H, W, C, C0, C1, training)
         _fwd_mark(ctx)
         return y.view(B, H * W, C1)
@@ -886,33 +888,17 @@ class BridgeFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dy):
         B, H, W, C, C0, C1, training = ctx.meta
-        if not training:
-            raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
+        _require_train_bn(training)
         col0, z0, mean0, rstd0, col1, z1, mean1, rstd1 = ctx.saved_tensors
         w0, c0, w1, c1 = ctx.params[:4]
         (g0, b0), (g1, b1) = _norm_slots(ctx.params[4:], 2)
-        M, dev = B * H * W, dy.device
-        lib = L.lib()
+        M = B * H * W
         dy = _contig(dy.float())
-
-        def conv_bwd(dz, col, w, cb, Cout, Cin):
-            gw, rw = gtarget(w)
-            if gw is not None:
-                gwp = gemm_tn(dz, cast_bf16(col, M, 9 * Cin), M, Cout, 9 * Cin, torch.zeros((Cout, 9 * Cin), dtype=F32, device=dev))
-                check(lib.mdv_unperm_conv_grad(ptr(gwp), 9 * Cin, ptr(gw), Cout, Cin, L.stream()), "mdv_unperm_conv_grad")
-            gb, rb = gtarget(cb)
-            colsum(dz, M, Cout, gb)
-            dcol = torch.empty((M, 9 * Cin), dtype=F32, device=dev)
-            gemm_nt(dz, prep_weight(w, 3, Cout, 9 * Cin, cin=Cin), M, 9 * Cin, Cout, dcol)
-            dx = torch.empty((M, Cin), dtype=F32, device=dev)
-            check(lib.mdv_col2im3(ptr(dcol), ptr(dx), B, H, W, H, W, Cin, 1, 9 * Cin, L.stream()), "mdv_col2im3")
-            return rw, rb, dx
-
         with _dev_ctx(dy):
             dz1, rg1, rb1 = bn_backward(dy, z1, mean1, rstd1, g1, b1, ACT_RELU, M, C1)
-            rw1, rc1, da0 = conv_bwd(dz1, col1, w1, c1, C1, C0)
+            rw1, rc1, da0 = _conv3_bwd(dz1, col1, w1, c1, B, H, W, H, W, 1)
             dz0, rg0, rb0 = bn_backward(da0, z0, mean0, rstd0, g0, b0, ACT_RELU, M, C0)
-            rw0, rc0, dx = conv_bwd(dz0, col0, w0, c0, C0, C)
+            rw0, rc0, dx = _conv3_bwd(dz0, col0, w0, c0, B, H, W, H, W, 1)
         _grads_done(ctx)
         return (dx.view(B, H * W, C), rw0, rc0, rw1, rc1, None, None, None, None) + _norm_grads((rg0, rb0), (rg1, rb1))
 
@@ -928,8 +914,7 @@ class DecoderConvFn(torch.autograd.Function):
         m, M, dev = B * h * w, B * H * W, inp.device
         inp, skip = _contig(inp), _contig(skip)
         ctx.params = (cb_w, cb_b, dw_w, pw_w) + norm
-        ((g, b, rm, rv, nb),) = _norm_slots(norm, 1, bufs)
-        _check_norm_sets(training)
+        (slot,) = _norm_slots(norm, 1, bufs)
         lib = L.lib()
         with _dev_ctx(inp):
             # both 1x1 convs of the decoder trunk run on TF32 operands (fp32 in memory): see mdv_gemm_nt_tf32
@@ -938,15 +923,7 @@ class DecoderConvFn(torch.autograd.Function):
             up = upsample_fwd(t, torch.empty((M, C), dtype=F32, device=dev), B, h, w, H, W, C)
             gc = torch.empty((M, C), dtype=F32, device=dev)
             check(lib.mdv_gconv2_fwd(ptr(skip), ptr(up), ptr(dw_w), ptr(gc), 0, B, H, W, C, L.stream()), "mdv_gconv2_fwd")
-            if not training:      # eval: BatchNorm + Hardswish folded into the GEMM epilogue
-                y = torch.empty((M, C), dtype=F32, device=dev)
-                sc, sh = bn_fold(g, b, rm, rv)
-                gemm_nt(gc, _contig(pw_w).view(C, C), M, C, C, y, tf32=True, colscale=sc, bias=sh, act=ACT_HSWISH, **_sets_kw(sc, H * W))
-                ctx.meta = (B, h, w, H, W, Cin, C, training)
-                return y.view(B, H * W, C)
-            z = torch.empty((M, C), dtype=F32, device=dev)
-            gemm_nt(gc, _contig(pw_w).view(C, C), M, C, C, z, tf32=True)
-            y, mean, rstd = bn_forward(z, M, C, g, b, rm, rv, nb, training, ACT_HSWISH, False)
+            y, (z, mean, rstd) = _conv_bn_fwd(gc, pw_w, M, C, slot, ACT_HSWISH, training, H * W)
         ctx.save_for_backward(skip, inp, up, gc, z, mean, rstd)
         ctx.meta = (B, h, w, H, W, Cin, C, training)
         _fwd_mark(ctx)
@@ -955,8 +932,7 @@ class DecoderConvFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dy):
         B, h, w, H, W, Cin, C, training = ctx.meta
-        if not training:
-            raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
+        _require_train_bn(training)
         skip, inp, up, gc, z, mean, rstd = ctx.saved_tensors
         cb_w, cb_b, dw_w, pw_w = ctx.params[:4]
         ((g, b),) = _norm_slots(ctx.params[4:], 1)
@@ -965,9 +941,7 @@ class DecoderConvFn(torch.autograd.Function):
         dy = _contig(dy.float())
         with _dev_ctx(dy):
             dz, rg, rb = bn_backward(dy, z, mean, rstd, g, b, ACT_HSWISH, M, C)
-            g_pw, r_pw = gtarget(pw_w, (C, C))
-            if g_pw is not None:
-                gemm_tn(dz, cast_bf16(gc, M, C), M, C, C, g_pw)
+            r_pw = _conv1_wgrad(dz, gc, pw_w)
             dgc = torch.empty((M, C), dtype=F32, device=dev)
             gemm_nt(dz, prep_weight(pw_w, 1, C, C), M, C, C, dgc)
             dskip = torch.empty((M, C), dtype=F32, device=dev)
@@ -977,9 +951,7 @@ class DecoderConvFn(torch.autograd.Function):
                   "mdv_gconv2_bwd")
             dt = upsample_bwd(dup, B, h, w, H, W, C)
             dtb = cast_bf16(dt, m, C)
-            g_cb, r_cb = gtarget(cb_w, (C, Cin))
-            if g_cb is not None:
-                gemm_tn(dtb, cast_bf16(inp, m, Cin), m, C, Cin, g_cb)
+            r_cb = _conv1_wgrad(dtb, inp, cb_w)
             g_cbb, r_cbb = gtarget(cb_b)
             colsum(dt, m, C, g_cbb)
             dinp = torch.empty((m, Cin), dtype=F32, device=dev)
@@ -1061,8 +1033,7 @@ class DeepLabFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dy):
         B, N, Cin, Co, H, W, dils, drop_p, sid, training = ctx.meta
-        if not training:
-            raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
+        _require_train_bn(training)
         xb, pooled, cat, col2, *flat = ctx.saved_tensors
         wgb = ctx.params
         ws, gs, bs = wgb[0::3], wgb[1::3], wgb[2::3]
@@ -1077,22 +1048,10 @@ class DeepLabFn(torch.autograd.Function):
             rets[3 * k + 1], rets[3 * k + 2] = rg, rb
             return dz
 
-        def wgrad3(k, dz, col, cin):
-            gw, rw = gtarget(ws[k])
-            if gw is not None:
-                gwp = gemm_tn(dz, col, M, Co, 9 * cin, torch.zeros((Co, 9 * cin), dtype=F32, device=dev))
-                check(lib.mdv_unperm_conv_grad(ptr(gwp), 9 * cin, ptr(gw), Co, cin, L.stream()), "mdv_unperm_conv_grad")
-            rets[3 * k] = rw
-
-        def wgrad1(k, dz, a, rows, cin):
-            gw, rw = gtarget(ws[k], (Co, cin))
-            gemm_tn(dz, a, rows, Co, cin, gw)
-            rets[3 * k] = rw
-
         with _dev_ctx(dy):
             # 3x3 conv
             dz = bn_bwd(6, dy, M)
-            wgrad3(6, dz, col2, Co)
+            rets[3 * 6] = _conv3_wgrad(dz, col2, ws[6])
             dcol = gemm_nt(dz, prep_weight(ws[6], 3, Co, 9 * Co, cin=Co), M, 9 * Co, Co, torch.empty((M, 9 * Co), dtype=F32, device=dev))
             dpj = torch.empty((M, Co), dtype=F32, device=dev)
             check(lib.mdv_col2im3_dil(ptr(dcol), ptr(dpj), B, H, W, Co, 1, 9 * Co, 0, L.stream()), "mdv_col2im3_dil")
@@ -1100,7 +1059,7 @@ class DeepLabFn(torch.autograd.Function):
                 dpj = cast_bf16(dpj, M, Co, drop_p=drop_p, drop_stream=sid).float()
             # project
             dz = bn_bwd(5, dpj, M)
-            wgrad1(5, dz, cat, M, 5 * Co)
+            rets[3 * 5] = _conv1_wgrad(dz, cat, ws[5])
             wt = prep_weight(ws[5], 1, Co, 5 * Co)                       # [5 Co, Co]: rows = input channels of the concat
 
             def dcat(k):      # gradient of branch k's slice of the concat (contiguous)
@@ -1108,7 +1067,7 @@ class DeepLabFn(torch.autograd.Function):
 
             # image pooling: the broadcast's transpose sums over the tokens of an image
             dzp = bn_bwd(4, _sum_tokens(dcat(4), B, H, W, Co), B)
-            wgrad1(4, dzp, pooled, B, Cin)
+            rets[3 * 4] = _conv1_wgrad(dzp, pooled, ws[4])
             inv_n = torch.full((B,), 1.0 / N, dtype=F32, device=dev)
             dpool = gemm_nt(dzp, prep_weight(ws[4], 1, Co, Cin), B, Cin, Co, torch.empty((B, Cin), dtype=F32, device=dev), rowscale=inv_n,
                             rows_per_scale=1)
@@ -1120,12 +1079,12 @@ class DeepLabFn(torch.autograd.Function):
                 dzk = bn_bwd(k, dcat(k), M)
                 if wgrad_on():
                     check(lib.mdv_im2col3_dil(ptr(xb), 1, ptr(col), B, H, W, Cin, dils[k - 1], 9 * Cin, L.stream()), "mdv_im2col3_dil")
-                wgrad3(k, dzk, col, Cin)
+                rets[3 * k] = _conv3_wgrad(dzk, col, ws[k])
                 gemm_nt(dzk, prep_weight(ws[k], 3, Co, 9 * Cin, cin=Cin), M, 9 * Cin, Co, dcolk)
                 check(lib.mdv_col2im3_dil(ptr(dcolk), ptr(dx), B, H, W, Cin, dils[k - 1], 9 * Cin, 1, L.stream()), "mdv_col2im3_dil")
             # 1x1 branch: dx += dz0 . W0
             dz0 = bn_bwd(0, dcat(0), M)
-            wgrad1(0, dz0, xb, M, Cin)
+            rets[3 * 0] = _conv1_wgrad(dz0, xb, ws[0])
             gemm_nt(dz0, prep_weight(ws[0], 1, Co, Cin), M, Cin, Co, dx, residual=dx)
         _grads_done(ctx)
         return (dx.view(B, N, Cin), None, None, None, None, None, None, *rets)
@@ -1480,8 +1439,7 @@ class AuxFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dout):
         B, sizes, Ho, Wo, hc, K, C5, p2, sid, training, Cs = ctx.meta
-        if not training:
-            raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
+        _require_train_bn(training)
         z, mean, rstd, a5, *rest = ctx.saved_tensors
         acts, wts = rest[:4], rest[4:]
         l1w, l1b, l2w, l2b, l3w, l3b, l4w, l4b, fw, fb, g, b, ow, ob = ctx.params
@@ -1773,8 +1731,8 @@ class ConvBnActFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dy):
         B, H, W, Ho, Wo, Cin, Cout, k, stride, pad, ld, kind, act, training, has_res, has_bn = ctx.meta
-        if has_bn and not training:
-            raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
+        if has_bn:
+            _require_train_bn(training)
         A, z, mean, rstd, y = ctx.saved_tensors
         w, cbias, gamma, beta = ctx.params
         M, dev = B * Ho * Wo, dy.device
@@ -1810,29 +1768,29 @@ class ConvBnActFn(torch.autograd.Function):
                     dz = cast_bf16(g, M, Cout)
                 gb, rcb = gtarget(cbias)
                 colsum(dz, M, Cout, gb)
-                gw, rw = gtarget(w)
-                if gw is not None:
-                    if kind == "k3i" and _IMPLICIT_CONV and Cin % 64 == 0 and W <= 64 and 64 % W == 0 and (H * W) % 64 == 0:
+                implicit_wgrad = kind == "k3i" and _IMPLICIT_CONV and Cin % 64 == 0 and W <= 64 and 64 % W == 0 and (H * W) % 64 == 0
+                if kind == "k3":
+                    rw = _conv3_wgrad(dz, A, w)
+                elif kind == "k3i" and not implicit_wgrad:
+                    Ab = None
+                    if wgrad_on():      # the im2col matrix exists only here, in bf16, as the weight-gradient GEMM's operand
+                        Ab = torch.empty((M, ld), dtype=BF16, device=dev)
+                        check(lib.mdv_im2col3(ptr(A), 0, ptr(Ab), 1, B, H, W, Ho, Wo, Cin, 1, ld, L.stream()), "mdv_im2col3")
+                    rw = _conv3_wgrad(dz, Ab, w)
+                else:
+                    gw, rw = gtarget(w)
+                    if gw is None:
+                        pass
+                    elif kind == "k3i":
                         # implicit weight-gradient GEMM: B tiles straight from a bf16 copy of the map
                         gwp = torch.zeros((Cout, ld), dtype=F32, device=dev)
                         check(lib.mdv_conv3_wgrad(ptr(dz), Cout, ptr(cast_bf16(A, M, Cin)), Cin, B, H, W, Cin, Cout, ptr(gwp), ld, L.stream()),
                               "mdv_conv3_wgrad")
                         check(lib.mdv_unperm_conv_grad(ptr(gwp), ld, ptr(gw), Cout, Cin, L.stream()), "mdv_unperm_conv_grad")
-                        Ab = None
-                    elif kind == "k3i":      # the im2col matrix exists only here, in bf16, as the weight-gradient GEMM's operand
-                        Ab = torch.empty((M, ld), dtype=BF16, device=dev)
-                        check(lib.mdv_im2col3(ptr(A), 0, ptr(Ab), 1, B, H, W, Ho, Wo, Cin, 1, ld, L.stream()), "mdv_im2col3")
-                    else:
-                        Ab = cast_bf16(A, M, ld)
-                    if Ab is None:
-                        pass
-                    elif kind in ("k3", "k3i"):
-                        gwp = gemm_tn(dz, Ab, M, Cout, ld, torch.zeros((Cout, ld), dtype=F32, device=dev))
-                        check(lib.mdv_unperm_conv_grad(ptr(gwp), ld, ptr(gw), Cout, Cin, L.stream()), "mdv_unperm_conv_grad")
                     elif ld == K:
-                        gemm_tn(dz, Ab, M, Cout, K, gw.view(Cout, K))
+                        gemm_tn(dz, cast_bf16(A, M, ld), M, Cout, K, gw.view(Cout, K))
                     else:
-                        gwp = gemm_tn(dz, Ab, M, Cout, ld, torch.zeros((Cout, ld), dtype=F32, device=dev))
+                        gwp = gemm_tn(dz, cast_bf16(A, M, ld), M, Cout, ld, torch.zeros((Cout, ld), dtype=F32, device=dev))
                         check(lib.mdv_add_f32(ptr(gwp), 0, ld, ptr(gw), K, Cout, K, 1, L.stream()), "mdv_add_f32")
                 dcol = None
                 if need_dx:
@@ -1879,8 +1837,7 @@ class BnActFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dy):
         B, N, C, act, training = ctx.meta
-        if not training:
-            raise RuntimeError("mdvit_b200: backward through eval-mode BatchNorm is not supported")
+        _require_train_bn(training)
         x, mean, rstd = ctx.saved_tensors
         gamma, beta = ctx.params
         dy = _contig(dy.float())

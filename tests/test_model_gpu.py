@@ -142,6 +142,20 @@ def test_forward_variants_and_dispatch_quirks(dev):
         assert rel_l2(o2[0], o0[0]) < 5e-3 and rel_l2(o2[1], o3[1]) < 5e-3 and rel_l2(o0[1], o3[1]) > 2e-2
 
 
+@pytest.mark.parametrize("kind", ["MDViT", "MDViT_DSN"])
+def test_backward_through_eval_batchnorm_raises(dev, kind):
+    """An eval-mode forward with grad enabled records a graph, but its BatchNorms used running statistics (folded into the conv GEMM
+    epilogues) and saved nothing to differentiate: backward raises instead of returning gradients of another function."""
+    from mdvit_b200.model import MDViT_DSN
+    m = build(dev) if kind == "MDViT" else MDViT_DSN(img_size=64, adapt_method="Sup", num_domains=4, decoder_name="MLPFM").to(dev)
+    m.eval()
+    img, _ = synth.synth_batch(1, 0, 2, 64, 64)
+    out, _ = m(img.to(dev), onehot(0, 2, dev), "0")
+    assert out.requires_grad
+    with pytest.raises(RuntimeError, match="backward through eval-mode BatchNorm is not supported"):
+        out.sum().backward()
+
+
 def _grads_of_step(dev, schedule, fuse_domains=True):
     from mdvit_b200.train_step import MKDTrainer
     m = build(dev).train()
